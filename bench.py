@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - decoded 20 ms frames/s of the batched IMBE/AMBE decode+synthesis path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|2|3|4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|2|3|4] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (frame bits -> ECC -> parameter decode -> synthesis -> int16 PCM) over one batch.
 Default workload = BASELINE.json configs[2], the configuration the metric is quoted on: IMBE 7200x4400 hard-decision ECC +
@@ -25,6 +25,12 @@ Numbers in the JSON line:
                same workload, the SAME counter-based input bits.
 `--impl reference` times only that CPU arm.  The CUDA library is mandatory for the default arm: there is no CPU fallback in
 the product, and nothing under oracle/ is on the measured GPU path.
+
+--dump-outputs DIR writes what the device-resident arm's last timed step returned, for a fixed seeded sample of rank 0's
+streams (at most DUMP_MAX_STREAMS per part, DUMP_BUDGET_BYTES in all), as DIR/<codec>_<input kind>_{streams,pcm,results}.npy:
+global stream ids (float64), int16 PCM as float32 [streams][frames][160] and the six mbe_b200_result words as float64
+[streams][frames][6].  Inputs and stream seeds depend only on the arguments, so two builds run with the same arguments can be
+compared output for output.
 """
 import argparse
 import json
@@ -49,6 +55,9 @@ STATE_BYTES = 7828  # 3 x mbe_parms + 16 B RNG words per stream
 RESULT_BYTES = 24
 HBM_FALLBACK_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md fallback
 INPUT_SEED = 0x4400
+DUMP_SEED = 0xD0D0
+DUMP_MAX_STREAMS = 512
+DUMP_BUDGET_BYTES = 64 << 20
 
 # BASELINE.json configs; a part = (codec, input kind).  Input kinds: "hard" iid random bits (counter-based, identical on the
 # CPU and the GPU arm), "tones" configs[3]-shaped frames, "softch" configs[4]-shaped soft-decision frames.
@@ -359,6 +368,26 @@ def run_cpu_reference(parts, n_frames, steps, warmup, streams_per_thread):
     return fps, info, total_sec
 
 
+def dump_outputs(out_dir, parts, bounds, first_global, n_frames, outs):
+    """Writes the --dump-outputs sample (see the module docstring) of the device outputs `outs` [(pcm, results)] per part."""
+    per_stream = n_frames * 160 * 4 + n_frames * 6 * 8 + 8
+    header = 4096                                     # bound on one .npy header (np.save pads it to 128 bytes here)
+    k_max = min(DUMP_MAX_STREAMS, (DUMP_BUDGET_BYTES - 3 * len(parts) * header) // (per_stream * len(parts)))
+    if k_max < 1:
+        raise SystemExit("bench.py: --dump-outputs: one stream of %d frames per part exceeds %d bytes" % (n_frames, DUMP_BUDGET_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for p, (codec, kind) in enumerate(parts):
+        n = bounds[p + 1] - bounds[p]
+        idx = np.sort(np.random.default_rng(DUMP_SEED + p).choice(n, size=min(n, k_max), replace=False))
+        pcm = outs[p][0][idx].cpu().numpy().astype(np.float32)
+        res = outs[p][1][idx].cpu().numpy().astype(np.int64)
+        res[..., 5] &= 0xffffffff                     # flags are uint32
+        name = os.path.join(out_dir, "%s_%s_" % (CODEC_NAMES[codec], kind))
+        np.save(name + "streams.npy", (idx + first_global + bounds[p]).astype(np.float64))
+        np.save(name + "pcm.npy", pcm)
+        np.save(name + "results.npy", res.astype(np.float64))
+
+
 def build_workload(args, world):
     """-> dict(parts=[(codec id, input kind)], total streams (None: per-GPU count), per_gpu, scaling, what)."""
     custom = args.codec is not None or args.soft or args.soft_channel or args.tones_unvoiced
@@ -397,7 +426,11 @@ def main():
                          "frames from parameter bits, valid channel frames (128 distinct streams tiled over the batch)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of the last timed step's PCM and results to DIR/*.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -540,6 +573,8 @@ def main():
         st_min = int(outs[p][1][:, :, 0].min().item())
         if (chk == 0 or st_min < 0) and not os.environ.get("MBE_B200_SKIP_KERNELS"):   # (timing experiments skip kernels)
             raise SystemExit("bench.py: device path produced silence or error statuses (part %d: max |pcm| %d, min status %d)" % (p, chk, st_min))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, parts, bounds, first_global, F, outs)
 
     # ---- end-to-end arm: host frames in, host PCM + results out, through the host-pointer C-ABI calls ----
     e2e = None

@@ -1,15 +1,15 @@
 #!/usr/bin/env python
 """Generates tests/golden/*.npz from the UNMODIFIED reference compiled by oracle/Makefile (oracle/_ref/libref_bench.so,
-Release flags = the parity build of SURVEY 8(c)).  Run in the build container (needs /root/reference mounted once, to build
-oracle/_ref):
+Release flags = the parity build of SURVEY 8(c)).  Needs the reference's sources once, to build
+oracle/_ref:
 
-    make -C oracle ref && python tests/golden/make_golden.py
+    MBELIB_NEO_SRC=<checkout of the reference> make -C oracle ref && python tests/golden/make_golden.py
 
 One file per codec and input kind: seeded inputs (random bits = repeats / mutes / re-initialisation; valid frames of held and
 changing parameters = stable pitch, interpolated harmonics; valid frames with flipped bits; AMBE tone / erasure signatures) and
 what the reference returns for them through mbe_process<Codec>[Soft]Framef + mbe_floattoshort, frame after frame:
-parameter bits, result counters and flags, float PCM (bit patterns), int16 PCM, the final mbe_parms triplets.  The GPU box
-has no /root/reference; tests/test_golden_fixtures.py compares the oracle port (CPU) and both GPU kernel paths with these."""
+parameter bits, result counters and flags, float PCM (bit patterns), int16 PCM, the final mbe_parms triplets.  The repository
+does not hold the reference; tests/test_golden_fixtures.py compares the oracle port (CPU) and both GPU kernel paths with these."""
 import os
 import sys
 
@@ -48,7 +48,7 @@ def frames_for(codec, S, F, seed):
 def main():
     ref = T.load_ref()
     if ref is None:
-        raise SystemExit("oracle/_ref/libref_bench.so is missing: run `make -C oracle ref` where /root/reference is mounted")
+        raise SystemExit("oracle/_ref/libref_bench.so is missing: run `MBELIB_NEO_SRC=<checkout of the reference> make -C oracle ref`")
     for codec in range(4):
         for soft in (0, 1):
             S, F = (8, 32) if not soft else (4, 12)

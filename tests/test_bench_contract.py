@@ -38,6 +38,11 @@ def test_other_configs_and_custom_workloads_parse():
         assert line["config"]["parts"] == [part] and line["scaling"] == "weak" and line["value"] > 0
 
 
+def test_zero_steps_are_refused():
+    r = _run(["--impl", "reference", "--steps", "0", "--warmup", "1"])
+    assert r.returncode != 0 and "--steps" in r.stderr
+
+
 def test_counter_based_input_is_the_same_on_both_arms():
     """the numpy generator (CPU arm) and the torch generator (GPU arm, run here on the CPU) give identical bits"""
     import importlib.util

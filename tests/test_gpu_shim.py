@@ -27,9 +27,39 @@ REFTESTS = ["test_golden_pcm", "test_noise_determinism", "test_floattoshort_pari
 def test_reference_test_program_passes_on_the_gpu_path(name):
     exe = os.path.join(ROOT, "oracle", "_ref", "shim_" + name)
     if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/shim_%s not built (needs /root/reference at build time: make -C oracle shimtests)" % name)
+        pytest.skip("oracle/_ref/shim_%s not built (needs the reference's sources at build time: MBELIB_NEO_SRC)" % name)
     r = subprocess.run([exe], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, "%s failed on the shim:\n%s\n%s" % (name, r.stdout[-2000:], r.stderr[-2000:])
+
+
+def test_golden_pcm_known_answer_through_the_shim():
+    """The known answer of the reference's tests/test_golden_pcm.c, stored here, on the shim's GPU path: its fixture frame
+    (fill_params) through mbe_synthesizeSpeechf with the thread RNG seeded 0xC0FFEE, then mbe_floattoshort; FNV-1a of the
+    float PCM 0x59741032, of the int16 PCM 0x4EDB8636 (the oracle's side is tests/test_oracle_kat.py)."""
+    shim = ctypes.CDLL(SHIM)
+    vp = ctypes.c_void_p
+    shim.mbe_setThreadRngSeed.argtypes = [ctypes.c_uint32]
+    shim.mbe_initMbeParms.argtypes = [vp, vp, vp]
+    shim.mbe_synthesizeSpeechf.argtypes = [vp, vp, vp]
+    shim.mbe_floattoshort.argtypes = [vp, vp]
+    cur, prev, enh = (np.zeros(T.PARMS_BYTES, np.uint8) for _ in range(3))
+    shim.mbe_initMbeParms(T._ptr(cur), T._ptr(prev), T._ptr(enh))
+    f, i = cur.view(np.float32), cur.view(np.int32)
+    f[0] = np.float32(0.105)
+    i[1] = 36
+    for l in range(1, 37):
+        i[3 + l] = 1 if l % 4 else 0
+        f[60 + l] = np.float32(0.035) + np.float32(0.0015) * np.float32(l)
+        f[174 + l] = np.float32(l) * np.float32(0.03)
+        f[231 + l] = np.float32(l) * np.float32(0.02)
+    prev[:] = cur
+    shim.mbe_setThreadRngSeed(0xC0FFEE)
+    out = np.zeros(160, np.float32)
+    pcm = np.zeros(160, np.int16)
+    shim.mbe_synthesizeSpeechf(T._ptr(out), T._ptr(cur), T._ptr(prev))
+    shim.mbe_floattoshort(T._ptr(out), T._ptr(pcm))
+    assert T.fnv1a32(out.tobytes()) == 0x59741032
+    assert T.fnv1a32(pcm.tobytes()) == 0x4EDB8636
 
 
 class Result(ctypes.Structure):

@@ -58,12 +58,12 @@ def test_shim_exports_every_declared_symbol(shim):
         assert hasattr(shim, name), "shim does not export %s" % name
 
 
-def test_struct_layouts():
+def test_struct_layouts(tmp_path):
     """mbe_parms is 2604 bytes with the reference's offsets (SURVEY 8(a) Y1)."""
     src = '#include <stdio.h>\n#include <stddef.h>\n#include "mbe_b200_compat.h"\nint main(void){printf("%zu %zu %zu %zu %zu %zu %zu\\n",' \
           'sizeof(mbe_parms),offsetof(mbe_parms,Ml),offsetof(mbe_parms,gamma),offsetof(mbe_parms,previousUw),' \
           'offsetof(mbe_parms,noiseSeed),sizeof(mbe_process_result),sizeof(mbe_soft_bit));return 0;}\n'
-    exe = "/tmp/mbe_compat_layout"
+    exe = str(tmp_path / "mbe_compat_layout")
     subprocess.run(["gcc", "-x", "c", "-", "-I" + os.path.join(ROOT, "include"), "-o", exe], input=src.encode(), check=True)
     out = subprocess.check_output([exe]).decode().split()
     assert out == ["2604", "240", "1152", "1192", "2216", "20", "2"]
