@@ -186,6 +186,42 @@ MBE_B200_API int mbe_b200_process_frames_packed(mbe_b200_ctx* ctx, int codec, in
                                                 int n_frames, const uint8_t* packed, int16_t* pcm, float* pcmf,
                                                 mbe_b200_result* results, uint8_t* bits);
 
+/* ---- indexed batches: any set of stream slots in one call -----------------------------------------------------
+ * A server that gives each call a state slot when the call starts and frees it when the call ends has, at every 20 ms tick,
+ * frames for a scattered subset of its slots.  An indexed call decodes that subset in one call: element i of the batch is
+ * stream slot slots[i] (any order), and frames / PCM / float PCM / results / bits are laid out [i][frame][...] exactly like
+ * stream i of a contiguous call; every element consumes n_frames frames with the semantics of the frame calls above.
+ * `input` says what `in` holds (MBE_B200_INPUT_*; PACKED uses the codec's channel map, mbe_b200_set_channel_map).
+ *   _dev    : d_slots and every buffer are device pointers, asynchronous on cuda_stream (as process_frames_dev).
+ *   host    : slots and every buffer are host pointers (as process_frames); submit_indexed is its asynchronous half,
+ *             completed by mbe_b200_wait (as submit_frames; the slot list must stay valid until then too).
+ * Rejection: an element whose slot is outside [0, max_streams), or repeats a slot an earlier element of the same list
+ * names, is rejected - all its frames read status MBE_STATUS_INVALID_ARGUMENT (-1) with every other result field zero,
+ * zero PCM / float PCM / bits, and no stream state is touched.  Every other element decodes normally, so the first
+ * occurrence of a repeated slot wins.  The check covers the whole list, on the device (_dev) as on the host calls.
+ * The state calls below validate on the host instead: an out-of-range or repeated slot fails the whole call with
+ * MBE_B200_E_ARG and nothing is touched.  n == 0 or n_frames == 0 returns 0 and launches nothing.
+ * Concurrent calls (on different CUDA streams) whose slot sets overlap are the caller's error, as overlapping stream ranges
+ * are for the contiguous calls.  Slot allocation stays with the caller. */
+#define MBE_B200_INPUT_HARD   0 /* one byte per bit, fr[R][C] order */
+#define MBE_B200_INPUT_SOFT   1 /* mbe_soft_bit pairs */
+#define MBE_B200_INPUT_PACKED 2 /* 8 hard bits per byte; the codec's channel map applies */
+MBE_B200_API int mbe_b200_process_indexed_dev(mbe_b200_ctx* ctx, int codec, int input, const int32_t* d_slots, int n,
+                                              int n_frames, const uint8_t* d_in, int16_t* d_pcm, float* d_pcmf,
+                                              mbe_b200_result* d_results, uint8_t* d_bits, void* cuda_stream);
+MBE_B200_API int mbe_b200_process_indexed(mbe_b200_ctx* ctx, int codec, int input, const int32_t* slots, int n,
+                                          int n_frames, const uint8_t* in, int16_t* pcm, float* pcmf,
+                                          mbe_b200_result* results, uint8_t* bits);
+MBE_B200_API int mbe_b200_submit_indexed(mbe_b200_ctx* ctx, int codec, int input, const int32_t* slots, int n, int n_frames,
+                                         const uint8_t* in, int16_t* pcm, float* pcmf, mbe_b200_result* results,
+                                         uint8_t* bits);
+/* init_streams / export / import of the listed slots (host slot list; element i <-> slots[i] of the dense buffers) */
+MBE_B200_API int mbe_b200_init_streams_indexed(mbe_b200_ctx* ctx, const int32_t* slots, int n, const uint32_t* seeds);
+MBE_B200_API int mbe_b200_export_state_indexed(mbe_b200_ctx* ctx, const int32_t* slots, int n, void* parms_triplets);
+MBE_B200_API int mbe_b200_import_state_indexed(mbe_b200_ctx* ctx, const int32_t* slots, int n, const void* parms_triplets);
+MBE_B200_API int mbe_b200_export_rng_indexed(mbe_b200_ctx* ctx, const int32_t* slots, int n, uint32_t* rng_words4);
+MBE_B200_API int mbe_b200_import_rng_indexed(mbe_b200_ctx* ctx, const int32_t* slots, int n, const uint32_t* rng_words4);
+
 /* ---- stage-split entry points ----------------------------------------------------------------
  * decode_frames: batched mbe_decode<Codec>[Soft]Frame (mbelib.h:315,323,395,403,471,479,545,553):
  *   ECC + PN de-scrambling only; stateless; n = number of frames; bits [n][param_bits] one byte per bit.
@@ -279,6 +315,14 @@ MBE_B200_API int mbe_b200_pool_import_state(mbe_b200_pool* pool, int first_strea
 MBE_B200_API int mbe_b200_pool_process_frames(mbe_b200_pool* pool, int codec, int soft, int first_stream, int n_streams,
                                               int n_frames, const uint8_t* frames, int16_t* pcm, float* pcmf,
                                               mbe_b200_result* results, uint8_t* bits);
+/* Indexed pool calls: slots are global pool slots in [0, max_streams), laid out as in mbe_b200_process_indexed /
+ * mbe_b200_init_streams_indexed.  Each shard gathers its elements (list order kept, so the first occurrence of a repeated
+ * slot still wins), runs the context's indexed call on its local slots and scatters the outputs back; an out-of-range
+ * element gets the rejected-element result of a context.  init_streams_indexed fails as a whole on a bad list. */
+MBE_B200_API int mbe_b200_pool_process_indexed(mbe_b200_pool* pool, int codec, int input, const int32_t* slots, int n,
+                                               int n_frames, const uint8_t* in, int16_t* pcm, float* pcmf,
+                                               mbe_b200_result* results, uint8_t* bits);
+MBE_B200_API int mbe_b200_pool_init_streams_indexed(mbe_b200_pool* pool, const int32_t* slots, int n, const uint32_t* seeds);
 MBE_B200_API int mbe_b200_pool_set_channel_map(mbe_b200_pool* pool, int codec, const uint16_t* map, int n_bits);
 MBE_B200_API int mbe_b200_pool_process_frames_packed(mbe_b200_pool* pool, int codec, int first_stream, int n_streams,
                                                      int n_frames, const uint8_t* packed, int16_t* pcm, float* pcmf,

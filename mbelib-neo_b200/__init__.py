@@ -42,7 +42,13 @@ _EXPORTS = ["mbe_b200_create", "mbe_b200_destroy", "mbe_b200_last_error", "mbe_b
             "mbe_b200_pool_import_state", "mbe_b200_pool_process_frames", "mbe_b200_pool_process_frames_packed",
             "mbe_b200_set_kernel_path", "mbe_b200_kernel_path", "mbe_b200_set_kernel_timing", "mbe_b200_kernel_timing",
             "mbe_b200_host_alloc", "mbe_b200_host_free", "mbe_b200_host_register", "mbe_b200_host_unregister",
-            "mbe_b200_single_frame"]
+            "mbe_b200_single_frame", "mbe_b200_process_indexed_dev", "mbe_b200_process_indexed", "mbe_b200_submit_indexed",
+            "mbe_b200_init_streams_indexed", "mbe_b200_export_state_indexed", "mbe_b200_import_state_indexed",
+            "mbe_b200_export_rng_indexed", "mbe_b200_import_rng_indexed", "mbe_b200_pool_process_indexed",
+            "mbe_b200_pool_init_streams_indexed"]
+
+# `input` of the indexed calls (MBE_B200_INPUT_* of include/mbe_b200.h)
+INPUT_HARD, INPUT_SOFT, INPUT_PACKED = 0, 1, 2
 
 _lib = None
 
@@ -127,6 +133,12 @@ def load_library():
         lib.mbe_b200_pool_import_state.argtypes = [vp, ci, ci, vp]
         lib.mbe_b200_pool_process_frames.argtypes = [vp, ci, ci, ci, ci, ci, vp, vp, vp, vp, vp]
         lib.mbe_b200_pool_process_frames_packed.argtypes = [vp, ci, ci, ci, ci, vp, vp, vp, vp, vp]
+        lib.mbe_b200_process_indexed_dev.argtypes = [vp, ci, ci, vp, ci, ci, vp, vp, vp, vp, vp, vp]
+        for n in ("process_indexed", "submit_indexed", "pool_process_indexed"):
+            getattr(lib, "mbe_b200_" + n).argtypes = [vp, ci, ci, vp, ci, ci, vp, vp, vp, vp, vp]
+        for n in ("init_streams_indexed", "export_state_indexed", "import_state_indexed", "export_rng_indexed",
+                  "import_rng_indexed", "pool_init_streams_indexed"):
+            getattr(lib, "mbe_b200_" + n).argtypes = [vp, vp, ci, vp]
         _lib = lib
     return _lib
 
@@ -141,6 +153,17 @@ def pack_frames(codec, frames):
     frames = np.ascontiguousarray(frames, dtype=np.uint8)
     assert frames.shape[-1] == FRAME_BITS[codec]
     return np.packbits(frames, axis=-1, bitorder="big")
+
+
+def _slots(slots):
+    return np.ascontiguousarray(slots, dtype=np.int32).reshape(-1)
+
+
+def _indexed_outputs(codec, n, F, want_float, want_bits=True, want_results=True):
+    return dict(pcm=np.zeros((n, F, SAMPLES), np.int16),
+                pcmf=np.zeros((n, F, SAMPLES), np.float32) if want_float else None,
+                results=np.zeros((n, F), RESULT_DTYPE) if want_results else None,
+                bits=np.zeros((n, F, PARAM_BITS[codec]), np.uint8) if want_bits else None)
 
 
 def _p(a):
@@ -253,6 +276,27 @@ class Pool:
         self._check(rc, "pool_process_frames")
         return dict(pcm=pcm, pcmf=pcmf, results=res, bits=bits)
 
+    def init_streams_indexed(self, slots, seeds=None):
+        """mbe_b200_pool_init_streams_indexed: init_streams of the listed global slots (seeds[i] for slots[i])."""
+        slots = _slots(slots)
+        if seeds is not None:
+            seeds = np.ascontiguousarray(seeds, dtype=np.uint32)
+            assert seeds.size == slots.size
+        self._check(self.lib.mbe_b200_pool_init_streams_indexed(self.h, _p(slots), slots.size, _p(seeds)),
+                    "pool_init_streams_indexed")
+
+    def process_indexed(self, codec, slots, frames, input=INPUT_HARD, want_float=False):
+        """mbe_b200_pool_process_indexed: element i of `frames` ([n][F][...]) is global slot slots[i]."""
+        slots = _slots(slots)
+        frames = np.ascontiguousarray(frames, dtype=np.uint8)
+        n, F = frames.shape[0], frames.shape[1]
+        assert n == slots.size
+        out = _indexed_outputs(codec, n, F, want_float)
+        self._check(self.lib.mbe_b200_pool_process_indexed(self.h, codec, int(input), _p(slots), n, F, _p(frames),
+                                                           _p(out["pcm"]), _p(out["pcmf"]), _p(out["results"]),
+                                                           _p(out["bits"])), "pool_process_indexed")
+        return out
+
 
 class Decoder:
     """One context = one GPU + a pool of `max_streams` device-resident voice-stream states."""
@@ -312,6 +356,68 @@ class Decoder:
     def import_rng(self, words, first=0):
         words = np.ascontiguousarray(words, dtype=np.uint32).reshape(-1, 4)
         self._check(self.lib.mbe_b200_import_rng(self.h, first, words.shape[0], _p(words)), "import_rng")
+
+    # ---- indexed state calls: host slot lists, element i <-> slots[i] ----
+    def init_streams_indexed(self, slots, seeds=None):
+        slots = _slots(slots)
+        if seeds is not None:
+            seeds = np.ascontiguousarray(seeds, dtype=np.uint32)
+            assert seeds.size == slots.size
+        self._check(self.lib.mbe_b200_init_streams_indexed(self.h, _p(slots), slots.size, _p(seeds)), "init_streams_indexed")
+
+    def export_state_indexed(self, slots):
+        slots = _slots(slots)
+        out = np.zeros((slots.size, 3, PARMS_BYTES), np.uint8)
+        self._check(self.lib.mbe_b200_export_state_indexed(self.h, _p(slots), slots.size, _p(out)), "export_state_indexed")
+        return out
+
+    def import_state_indexed(self, slots, blobs):
+        slots = _slots(slots)
+        blobs = np.ascontiguousarray(blobs, dtype=np.uint8).reshape(-1, 3, PARMS_BYTES)
+        assert blobs.shape[0] == slots.size
+        self._check(self.lib.mbe_b200_import_state_indexed(self.h, _p(slots), slots.size, _p(blobs)), "import_state_indexed")
+
+    def export_rng_indexed(self, slots):
+        slots = _slots(slots)
+        out = np.zeros((slots.size, 4), np.uint32)
+        self._check(self.lib.mbe_b200_export_rng_indexed(self.h, _p(slots), slots.size, _p(out)), "export_rng_indexed")
+        return out
+
+    def import_rng_indexed(self, slots, words):
+        slots = _slots(slots)
+        words = np.ascontiguousarray(words, dtype=np.uint32).reshape(-1, 4)
+        assert words.shape[0] == slots.size
+        self._check(self.lib.mbe_b200_import_rng_indexed(self.h, _p(slots), slots.size, _p(words)), "import_rng_indexed")
+
+    # ---- indexed batches: element i of frames / outputs is stream slot slots[i] ----
+    def process_indexed(self, codec, slots, frames, input=INPUT_HARD, want_float=False, want_bits=True, want_results=True):
+        """frames: uint8 [n][F][bits] (INPUT_HARD), [n][F][bits][2] (INPUT_SOFT) or [n][F][channel bytes] (INPUT_PACKED)."""
+        slots = _slots(slots)
+        frames = np.ascontiguousarray(frames, dtype=np.uint8)
+        n, F = frames.shape[0], frames.shape[1]
+        assert n == slots.size
+        out = _indexed_outputs(codec, n, F, want_float, want_bits, want_results)
+        self._check(self.lib.mbe_b200_process_indexed(self.h, codec, int(input), _p(slots), n, F, _p(frames), _p(out["pcm"]),
+                                                      _p(out["pcmf"]), _p(out["results"]), _p(out["bits"])),
+                    "process_indexed")
+        return out
+
+    def submit_indexed(self, codec, slots, frames, out, input=INPUT_HARD):
+        """Asynchronous process_indexed: `slots`, `frames` and the arrays of `out` (dict with pcm / pcmf / results / bits,
+        any may be missing) must stay alive and untouched until wait()."""
+        assert slots.dtype == np.int32 and slots.flags["C_CONTIGUOUS"]
+        n, F = frames.shape[0], frames.shape[1]
+        self._check(self.lib.mbe_b200_submit_indexed(self.h, codec, int(input), _p(slots), n, F, _p(frames),
+                                                     _p(out.get("pcm")), _p(out.get("pcmf")), _p(out.get("results")),
+                                                     _p(out.get("bits"))), "submit_indexed")
+
+    def process_indexed_dev(self, codec, input, d_slots, n, n_frames, d_in, d_pcm, d_pcmf=0, d_results=0, d_bits=0,
+                            cuda_stream=0):
+        """All pointers are raw device addresses (ints), d_slots int32 [n]; asynchronous on `cuda_stream`."""
+        self._check(self.lib.mbe_b200_process_indexed_dev(self.h, codec, int(input), _p(d_slots), n, n_frames, _p(d_in),
+                                                          _p(d_pcm or None), _p(d_pcmf or None), _p(d_results or None),
+                                                          _p(d_bits or None), _p(cuda_stream or None)),
+                    "process_indexed_dev")
 
     # ---- hot path, host buffers ----
     def process_frames(self, codec, frames, soft=False, first_stream=0, want_float=False, want_bits=True,

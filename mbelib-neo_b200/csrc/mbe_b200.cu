@@ -18,6 +18,7 @@
 
 #include <atomic>
 #include <mutex>
+#include <vector>
 
 #include "mbe_common.cuh"
 
@@ -559,7 +560,9 @@ struct StreamShape {
     static constexpr int MINB = SMALL ? P_MINB : MIN_BLOCKS_PER_SM;
 };
 
-template <int CODEC, int SOFT, int MODE, bool SPLIT>
+// INDEXED: channel frames of an indexed call (LaunchArgs::slots); a separate image, so that the contiguous launches keep
+// the register allocation they have without the slot list and the claim check
+template <int CODEC, int SOFT, int MODE, bool SPLIT, bool INDEXED = false>
 __global__ void __launch_bounds__(StreamShape<SOFT, SPLIT>::WARPS * 32, StreamShape<SOFT, SPLIT>::MINB)
 mbe_stream_kernel(const LaunchArgs A) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -585,9 +588,18 @@ mbe_stream_kernel(const LaunchArgs A) {
     const size_t fstride = (MODE == MODE_DATA) ? (size_t)pbits
                                                : (PACKED ? (size_t)A.packed_bytes : (size_t)fbits * (SOFT == 1 ? 2u : 1u));
 
-    uint32_t* gs = A.state + (size_t)(A.first_stream + (live ? s : 0)) * STATE_WORDS;
+    // an element of an indexed call whose slot is out of range or claimed by an earlier element is rejected: it touches no
+    // state, runs no decode, and its outputs are those of an invalid-argument frame (status -1, zeros)
+    int slot = A.first_stream + (live ? s : 0);   // slot_of(A, s) of a contiguous launch
+    bool own = live;
+    if (INDEXED && live) {
+        slot = slot_of(A, s);
+        own = (unsigned)slot < (unsigned)A.max_streams && A.claim[slot] == claim_tag(A.epoch, A.slot_base + A.io_base + s);
+        slot = own ? slot : 0;
+    }
+    uint32_t* gs = A.state + (size_t)slot * STATE_WORDS;
     const StreamHomeT<SPLIT> home = {gs, gs + PARMS_WORDS, gs + 2 * PARMS_WORDS, gs + SPILL_WORD};
-    if (live) {
+    if (own) {
         load_stream(ws, gs, lane);
     }
     if (lane == 0) {
@@ -620,7 +632,7 @@ mbe_stream_kernel(const LaunchArgs A) {
         rout.c0_errors = rout.protected_errors = rout.c4_errors = rout.total_errors = 0;
         rout.flags = 0;
 
-        if (live) {
+        if (own) {
             const uint8_t* fr = A.frames + idx * fstride;
             if (MODE == MODE_FRAMES) {
                 // soft decision: the parity cost table takes the whole union and the small tables, reliabilities and
@@ -797,7 +809,7 @@ mbe_stream_kernel(const LaunchArgs A) {
         }
         STAGE_T(6);
     }
-    if (live) {
+    if (own) {
         store_stream(ws, gs, lane);
     }
 #if MBE_STAGE_TIMING
@@ -1235,13 +1247,18 @@ __global__ void mbe_floattoshort_kernel(size_t n, const float* __restrict__ in, 
 }
 
 // per stream: mbe_setThreadRngSeed(seed) + mbe_initMbeParms (mbelib.c:173-181,367-410)
-__global__ void mbe_init_streams_kernel(uint32_t* state, int first, int count, const uint32_t* seeds, float w0, int L) {
+// (slots != nullptr: element i is stream slot slots[i] - an indexed call, validated on the host - instead of first + i)
+struct SlotList {
+    const int32_t* slots;
+    int first_stream, slot_base, io_base;
+};
+__global__ void mbe_init_streams_kernel(uint32_t* state, SlotList sl, int count, const uint32_t* seeds, float w0, int L) {
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (warp >= count) {
         return;
     }
-    uint32_t* gs = state + (size_t)(first + warp) * STATE_WORDS;
+    uint32_t* gs = state + (size_t)slot_of(sl, warp) * STATE_WORDS;
     Parms* p = reinterpret_cast<Parms*>(gs);
     for (int k = 0; k < 3; ++k) {
         fill_default(p + k, w0, L, 12, 0.0875f, lane);
@@ -1270,12 +1287,12 @@ __global__ void mbe_init_streams_kernel(uint32_t* state, int first, int count, c
 }
 
 // gather/scatter between the interleaved HBM state pool and dense [count][3][651] / [count][4] buffers
-__global__ void mbe_state_xfer_kernel(uint32_t* state, int first, int count, uint32_t* dense, int words, int offset,
+__global__ void mbe_state_xfer_kernel(uint32_t* state, SlotList sl, int count, uint32_t* dense, int words, int offset,
                                       int to_dense) {
     const size_t total = (size_t)count * words;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const size_t s = i / words, w = i % words;
-        uint32_t* g = state + (size_t)(first + s) * STATE_WORDS + offset + w;
+        uint32_t* g = state + (size_t)slot_of(sl, (int)s) * STATE_WORDS + offset + w;
         if (to_dense) {
             // exported mbe_parms images carry the reference's NaN pattern (the RNG words are integers: untouched)
             dense[i] = (words == 3 * PARMS_WORDS) ? ref_nan_parms_word((int)(w % PARMS_WORDS), *g) : *g;
@@ -1294,6 +1311,18 @@ __global__ void mbe_single_io_kernel(uint32_t* state, int stream, uint32_t* blob
             blob[i] = (i < 3 * PARMS_WORDS) ? ref_nan_parms_word(i % PARMS_WORDS, g[i]) : g[i];
         } else {
             g[i] = blob[i];
+        }
+    }
+}
+
+// indexed calls: every element whose slot is in range leaves its tag on the slot; the largest tag - the element of the call
+// that lists the slot first - is the one the frame kernels accept (one launch over the whole list, so a repeated slot is
+// caught wherever the host pipeline cuts the list into chunks)
+__global__ void mbe_claim_kernel(const int32_t* slots, int n, int max_streams, unsigned long long* claim, unsigned epoch) {
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const int slot = slots[i];
+        if ((unsigned)slot < (unsigned)max_streams) {
+            atomicMax(&claim[slot], claim_tag(epoch, i));
         }
     }
 }
@@ -1352,6 +1381,12 @@ struct mbe_b200_ctx {
     cudaEvent_t* kt_ev;               // [2 * KT_MAX]
     unsigned char* kt_kind;           // [KT_MAX]: 0 parameter (or fused) kernel, 1 bank kernel, 2 unvoiced kernel
     unsigned long long* d_cnt;        // [4] device counters of the bank kernel
+    // indexed calls: the claim tag of every slot (mbe_claim_kernel), the epoch of the latest call, and the device copy of a
+    // host slot list (reused like d_in: host-pointer calls are synchronous or pending until mbe_b200_wait)
+    unsigned long long* d_claim;      // [max_streams]
+    unsigned claim_epoch;
+    int32_t* d_slots;
+    size_t d_slots_cap;
     char err[256];
 };
 
@@ -1638,7 +1673,7 @@ typedef void (*StreamKernelFn)(const LaunchArgs);
 
 // one kernel image per (codec, soft) for channel frames; parameter-bit input (mbe_process<Codec>Data) has no
 // soft variant and IMBE 7100 shares the IMBE 4400 parameter layout
-template <bool SPLIT>
+template <bool SPLIT, bool INDEXED>
 static StreamKernelFn pick_stream_kernel_t(int codec, int soft, int mode) {
     if (mode == MODE_DATA) {
         switch (codec) {
@@ -1649,26 +1684,30 @@ static StreamKernelFn pick_stream_kernel_t(int codec, int soft, int mode) {
     }
     if (soft == 2) {  // packed hard bits
         switch (codec) {
-            case MBE_B200_IMBE7200X4400: return mbe_stream_kernel<MBE_B200_IMBE7200X4400, 2, MODE_FRAMES, SPLIT>;
-            case MBE_B200_IMBE7100X4400: return mbe_stream_kernel<MBE_B200_IMBE7100X4400, 2, MODE_FRAMES, SPLIT>;
-            case MBE_B200_AMBE3600X2400: return mbe_stream_kernel<MBE_B200_AMBE3600X2400, 2, MODE_FRAMES, SPLIT>;
-            default: return mbe_stream_kernel<MBE_B200_AMBE3600X2450, 2, MODE_FRAMES, SPLIT>;
+            case MBE_B200_IMBE7200X4400: return mbe_stream_kernel<MBE_B200_IMBE7200X4400, 2, MODE_FRAMES, SPLIT, INDEXED>;
+            case MBE_B200_IMBE7100X4400: return mbe_stream_kernel<MBE_B200_IMBE7100X4400, 2, MODE_FRAMES, SPLIT, INDEXED>;
+            case MBE_B200_AMBE3600X2400: return mbe_stream_kernel<MBE_B200_AMBE3600X2400, 2, MODE_FRAMES, SPLIT, INDEXED>;
+            default: return mbe_stream_kernel<MBE_B200_AMBE3600X2450, 2, MODE_FRAMES, SPLIT, INDEXED>;
         }
     }
     switch (codec * 2 + (soft ? 1 : 0)) {
-        case 0: return mbe_stream_kernel<MBE_B200_IMBE7200X4400, 0, MODE_FRAMES, SPLIT>;
-        case 1: return mbe_stream_kernel<MBE_B200_IMBE7200X4400, 1, MODE_FRAMES, SPLIT>;
-        case 2: return mbe_stream_kernel<MBE_B200_IMBE7100X4400, 0, MODE_FRAMES, SPLIT>;
-        case 3: return mbe_stream_kernel<MBE_B200_IMBE7100X4400, 1, MODE_FRAMES, SPLIT>;
-        case 4: return mbe_stream_kernel<MBE_B200_AMBE3600X2400, 0, MODE_FRAMES, SPLIT>;
-        case 5: return mbe_stream_kernel<MBE_B200_AMBE3600X2400, 1, MODE_FRAMES, SPLIT>;
-        case 6: return mbe_stream_kernel<MBE_B200_AMBE3600X2450, 0, MODE_FRAMES, SPLIT>;
-        default: return mbe_stream_kernel<MBE_B200_AMBE3600X2450, 1, MODE_FRAMES, SPLIT>;
+        case 0: return mbe_stream_kernel<MBE_B200_IMBE7200X4400, 0, MODE_FRAMES, SPLIT, INDEXED>;
+        case 1: return mbe_stream_kernel<MBE_B200_IMBE7200X4400, 1, MODE_FRAMES, SPLIT, INDEXED>;
+        case 2: return mbe_stream_kernel<MBE_B200_IMBE7100X4400, 0, MODE_FRAMES, SPLIT, INDEXED>;
+        case 3: return mbe_stream_kernel<MBE_B200_IMBE7100X4400, 1, MODE_FRAMES, SPLIT, INDEXED>;
+        case 4: return mbe_stream_kernel<MBE_B200_AMBE3600X2400, 0, MODE_FRAMES, SPLIT, INDEXED>;
+        case 5: return mbe_stream_kernel<MBE_B200_AMBE3600X2400, 1, MODE_FRAMES, SPLIT, INDEXED>;
+        case 6: return mbe_stream_kernel<MBE_B200_AMBE3600X2450, 0, MODE_FRAMES, SPLIT, INDEXED>;
+        default: return mbe_stream_kernel<MBE_B200_AMBE3600X2450, 1, MODE_FRAMES, SPLIT, INDEXED>;
     }
 }
 
-static StreamKernelFn pick_stream_kernel(int codec, int soft, int mode, bool split = false) {
-    return split ? pick_stream_kernel_t<true>(codec, soft, mode) : pick_stream_kernel_t<false>(codec, soft, mode);
+// (indexed: channel frames only - parameter-bit input has no indexed entry point)
+static StreamKernelFn pick_stream_kernel(int codec, int soft, int mode, bool split = false, bool indexed = false) {
+    if (indexed) {
+        return split ? pick_stream_kernel_t<true, true>(codec, soft, mode) : pick_stream_kernel_t<false, true>(codec, soft, mode);
+    }
+    return split ? pick_stream_kernel_t<true, false>(codec, soft, mode) : pick_stream_kernel_t<false, false>(codec, soft, mode);
 }
 
 static size_t bank_kernel_smem(void) { return BANK_TAB_FLOATS * sizeof(float) + (size_t)B_WARPS * sizeof(BankWS); }
@@ -1827,14 +1866,18 @@ int mbe_b200_create(mbe_b200_ctx** out, int device_ordinal, int max_streams) {
     CUC(cudaMalloc(&ctx->d_state, (size_t)max_streams * STATE_WORDS * sizeof(uint32_t)));
     CUC(cudaMalloc(&ctx->d_dbg, 16 * sizeof(unsigned long long)));
     CUC(cudaMemsetAsync(ctx->d_dbg, 0, 16 * sizeof(unsigned long long), ctx->stream));
+    CUC(cudaMalloc(&ctx->d_claim, (size_t)max_streams * sizeof(unsigned long long)));
+    CUC(cudaMemsetAsync(ctx->d_claim, 0, (size_t)max_streams * sizeof(unsigned long long), ctx->stream));
     CUC(cudaStreamSynchronize(ctx->stream));
     for (int codec = 0; codec < 4; ++codec) {
         for (int soft = 0; soft < 3; ++soft) {
             for (int mode = 0; mode < (soft == 2 ? 1 : 2); ++mode) {
-                CUC(cudaFuncSetAttribute(pick_stream_kernel(codec, soft, mode, false),
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)stream_kernel_smem()));
-                CUC(cudaFuncSetAttribute(pick_stream_kernel(codec, soft, mode, true),
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)parm_kernel_smem(soft)));
+                for (int indexed = 0; indexed < (mode == MODE_FRAMES ? 2 : 1); ++indexed) {
+                    CUC(cudaFuncSetAttribute(pick_stream_kernel(codec, soft, mode, false, indexed),
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)stream_kernel_smem()));
+                    CUC(cudaFuncSetAttribute(pick_stream_kernel(codec, soft, mode, true, indexed),
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)parm_kernel_smem(soft)));
+                }
             }
         }
     }
@@ -1928,6 +1971,8 @@ void mbe_b200_destroy(mbe_b200_ctx* ctx) {
     }
     cudaFree(ctx->d_one);
     cudaFree(ctx->d_state);
+    cudaFree(ctx->d_claim);
+    cudaFree(ctx->d_slots);
     cudaFree(ctx->d_dbg);
     cudaFree(ctx->d_tab);
     cudaFree(ctx->d_in);
@@ -1986,11 +2031,38 @@ static int check_range(mbe_b200_ctx* ctx, int first, int count) {
     return 0;
 }
 
-int mbe_b200_init_streams(mbe_b200_ctx* ctx, int first, int count, const uint32_t* seeds) {
-    int rc = check_range(ctx, first, count);
-    if (rc < 0 || count == 0) {
+// slot list of an indexed state call: every slot in [0, max_streams) and none listed twice, or the whole call fails
+static int check_slots(mbe_b200_ctx* ctx, const int32_t* slots, int n) {
+    if (!ctx) {
+        return MBE_B200_E_ARG;
+    }
+    if (n < 0 || (n > 0 && !slots)) {
+        return fail(ctx, MBE_B200_E_ARG, "slot list: bad argument", cudaSuccess);
+    }
+    std::vector<unsigned char> seen(n > 0 ? (size_t)ctx->max_streams : 0, 0);
+    for (int i = 0; i < n; ++i) {
+        const int32_t slot = slots[i];
+        if (slot < 0 || slot >= ctx->max_streams || seen[slot]) {
+            return fail(ctx, MBE_B200_E_ARG, "slot list: a slot is outside the context's pool or listed twice", cudaSuccess);
+        }
+        seen[slot] = 1;
+    }
+    return 0;
+}
+
+// a host slot list into the context's device copy, ordered on `st`
+static int upload_slots(mbe_b200_ctx* ctx, const int32_t* slots, int n, cudaStream_t st) {
+    int rc = ensure(ctx, (void**)&ctx->d_slots, &ctx->d_slots_cap, (size_t)n * sizeof(int32_t));
+    if (rc < 0) {
         return rc;
     }
+    CU(cudaMemcpyAsync(ctx->d_slots, slots, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    return 0;
+}
+
+// slots == nullptr: streams first .. first + count - 1; otherwise the (validated) host slot list
+static int init_streams_impl(mbe_b200_ctx* ctx, int first, int count, const uint32_t* seeds, const int32_t* slots) {
+    int rc;
     if (check_idle(ctx, "init_streams") < 0) {
         return MBE_B200_E_ARG;
     }
@@ -2004,8 +2076,12 @@ int mbe_b200_init_streams(mbe_b200_ctx* ctx, int first, int count, const uint32_
         d_seeds = (uint32_t*)ctx->d_in;
         CU(cudaMemcpyAsync(d_seeds, seeds, (size_t)count * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
     }
+    if (slots && (rc = upload_slots(ctx, slots, count, ctx->stream)) < 0) {
+        return rc;
+    }
+    const SlotList sl = {slots ? ctx->d_slots : nullptr, first, 0, 0};
     const int threads = 256, wpb = threads / 32;
-    mbe_init_streams_kernel<<<(count + wpb - 1) / wpb, threads, 0, ctx->stream>>>(ctx->d_state, first, count, d_seeds,
+    mbe_init_streams_kernel<<<(count + wpb - 1) / wpb, threads, 0, ctx->stream>>>(ctx->d_state, sl, count, d_seeds,
                                                                                     ctx->imbe_default_w0,
                                                                                     ctx->imbe_default_L);
     ctx->launches++;
@@ -2014,8 +2090,25 @@ int mbe_b200_init_streams(mbe_b200_ctx* ctx, int first, int count, const uint32_
     return 0;
 }
 
-static int state_xfer(mbe_b200_ctx* ctx, int first, int count, void* host, int words, int offset, int to_host) {
-    int rc = check_range(ctx, first, count);
+int mbe_b200_init_streams(mbe_b200_ctx* ctx, int first, int count, const uint32_t* seeds) {
+    const int rc = check_range(ctx, first, count);
+    if (rc < 0 || count == 0) {
+        return rc;
+    }
+    return init_streams_impl(ctx, first, count, seeds, nullptr);
+}
+
+int mbe_b200_init_streams_indexed(mbe_b200_ctx* ctx, const int32_t* slots, int n, const uint32_t* seeds) {
+    const int rc = check_slots(ctx, slots, n);
+    if (rc < 0 || n == 0) {
+        return rc;
+    }
+    return init_streams_impl(ctx, 0, n, seeds, slots);
+}
+
+static int state_xfer(mbe_b200_ctx* ctx, int first, int count, void* host, int words, int offset, int to_host,
+                      const int32_t* slots = nullptr) {
+    int rc = slots ? check_slots(ctx, slots, count) : check_range(ctx, first, count);
     if (rc < 0 || count == 0) {
         return rc;
     }
@@ -2036,9 +2129,13 @@ static int state_xfer(mbe_b200_ctx* ctx, int first, int count, void* host, int w
     if (!to_host) {
         CU(cudaMemcpyAsync(dense, host, bytes, cudaMemcpyHostToDevice, ctx->stream));
     }
+    if (slots && (rc = upload_slots(ctx, slots, count, ctx->stream)) < 0) {
+        return rc;
+    }
+    const SlotList sl = {slots ? ctx->d_slots : nullptr, first, 0, 0};
     const size_t n_words = (size_t)count * words;
     const int blocks = (int)((n_words + 255) / 256 < 1024 ? (n_words + 255) / 256 : 1024);
-    mbe_state_xfer_kernel<<<blocks, 256, 0, ctx->stream>>>(ctx->d_state, first, count, dense, words, offset, to_host);
+    mbe_state_xfer_kernel<<<blocks, 256, 0, ctx->stream>>>(ctx->d_state, sl, count, dense, words, offset, to_host);
     ctx->launches++;
     CU(cudaGetLastError());
     if (to_host) {
@@ -2056,6 +2153,18 @@ int mbe_b200_import_state(mbe_b200_ctx* ctx, int first, int count, const void* p
 }
 int mbe_b200_export_rng(mbe_b200_ctx* ctx, int first, int count, uint32_t* rng_words4) {
     return state_xfer(ctx, first, count, rng_words4, RNG_WORDS, 3 * PARMS_WORDS, 1);
+}
+int mbe_b200_export_state_indexed(mbe_b200_ctx* ctx, const int32_t* slots, int n, void* parms_triplets) {
+    return state_xfer(ctx, 0, n, parms_triplets, 3 * PARMS_WORDS, 0, 1, slots);
+}
+int mbe_b200_import_state_indexed(mbe_b200_ctx* ctx, const int32_t* slots, int n, const void* parms_triplets) {
+    return state_xfer(ctx, 0, n, const_cast<void*>(parms_triplets), 3 * PARMS_WORDS, 0, 0, slots);
+}
+int mbe_b200_export_rng_indexed(mbe_b200_ctx* ctx, const int32_t* slots, int n, uint32_t* rng_words4) {
+    return state_xfer(ctx, 0, n, rng_words4, RNG_WORDS, 3 * PARMS_WORDS, 1, slots);
+}
+int mbe_b200_import_rng_indexed(mbe_b200_ctx* ctx, const int32_t* slots, int n, const uint32_t* rng_words4) {
+    return state_xfer(ctx, 0, n, const_cast<uint32_t*>(rng_words4), RNG_WORDS, 3 * PARMS_WORDS, 0, slots);
 }
 int mbe_b200_import_rng(mbe_b200_ctx* ctx, int first, int count, const uint32_t* rng_words4) {
     return state_xfer(ctx, first, count, const_cast<uint32_t*>(rng_words4), RNG_WORDS, 3 * PARMS_WORDS, 0);
@@ -2110,7 +2219,8 @@ static int launch_stream_kernel(mbe_b200_ctx* ctx, const LaunchArgs& a_in, cudaS
         const int blocks = (a.n_streams + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
         {
             KernelTimer kt(ctx, 0, st);
-            pick_stream_kernel(a.codec, a.soft, a.mode)<<<blocks, WARPS_PER_BLOCK * 32, stream_kernel_smem(), st>>>(a);
+            pick_stream_kernel(a.codec, a.soft, a.mode, false, a.slots != nullptr)<<<blocks, WARPS_PER_BLOCK * 32,
+                                                                                      stream_kernel_smem(), st>>>(a);
         }
         ctx->launches++;
         CU(cudaGetLastError());
@@ -2153,7 +2263,7 @@ static int launch_stream_kernel(mbe_b200_ctx* ctx, const LaunchArgs& a_in, cudaS
             CU(cudaStreamWaitEvent(ctx->s_aux[i], ctx->ev_fork, 0));
         }
     }
-    StreamKernelFn pk = pick_stream_kernel(a.codec, a.soft, a.mode, true);
+    StreamKernelFn pk = pick_stream_kernel(a.codec, a.soft, a.mode, true, a.slots != nullptr);
     const int n_total = a.n_streams, first0 = a.first_stream;
     for (int i = 0, o = 0; o < n_total; o += sub, ++i) {
         const int slot = fork ? MAX_KSTREAMS + (i % n_aux) : kslot;
@@ -2186,6 +2296,8 @@ static int launch_stream_kernel(mbe_b200_ctx* ctx, const LaunchArgs& a_in, cudaS
         sa.state = a.state;
         sa.tab = a.tab;
         sa.counters = ctx->kt_on ? ctx->d_cnt : nullptr;
+        sa.slots = a.slots;
+        sa.slot_base = a.slot_base;
         const long long groups = ((long long)ns * a.n_frames + BG - 1) / BG;
         long long bank_blocks = (groups + B_WARPS - 1) / B_WARPS;
         const long long resident = (long long)g_sm_count.load() * B_MINB;   // grid-stride warps: one resident wave is enough
@@ -2283,9 +2395,12 @@ int mbe_b200_kernel_timing(mbe_b200_ctx* ctx, double ms[3], long long launches[3
 }
 
 // input kinds of the frame entry points: 0 = one byte per hard bit, 1 = mbe_soft_bit pairs, 2 = hard bits packed
+// (MBE_B200_INPUT_*).  d_slots != nullptr: an indexed launch, elements slot_base .. slot_base + n_streams - 1 of the call's
+// device slot list, claimed under `epoch` (first_stream is ignored)
 static int frames_dev_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_stream, int n_streams, int n_frames,
                            const uint8_t* d_frames, int16_t* d_pcm, float* d_pcmf, mbe_b200_result* d_results,
-                           uint8_t* d_bits, void* cuda_stream);
+                           uint8_t* d_bits, void* cuda_stream, const int32_t* d_slots = nullptr, int slot_base = 0,
+                           unsigned epoch = 0);
 
 int mbe_b200_process_frames_dev(mbe_b200_ctx* ctx, int codec, int soft, int first_stream, int n_streams, int n_frames,
                                 const uint8_t* d_frames, int16_t* d_pcm, float* d_pcmf, mbe_b200_result* d_results,
@@ -2359,9 +2474,9 @@ int mbe_b200_packed_frame_bytes(int codec) {
 
 static int frames_dev_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_stream, int n_streams, int n_frames,
                            const uint8_t* d_frames, int16_t* d_pcm, float* d_pcmf, mbe_b200_result* d_results,
-                           uint8_t* d_bits, void* cuda_stream) {
+                           uint8_t* d_bits, void* cuda_stream, const int32_t* d_slots, int slot_base, unsigned epoch) {
     const int soft = kind;
-    int rc = check_range(ctx, first_stream, n_streams);
+    int rc = d_slots ? (ctx ? 0 : MBE_B200_E_ARG) : check_range(ctx, first_stream, n_streams);
     if (rc < 0) {
         return rc;
     }
@@ -2388,6 +2503,11 @@ static int frames_dev_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_str
     a.state = ctx->d_state;
     a.tab = ctx->d_tab;
     a.dbg = ctx->d_dbg;
+    a.slots = d_slots;
+    a.claim = ctx->d_claim;
+    a.epoch = epoch;
+    a.slot_base = slot_base;
+    a.max_streams = ctx->max_streams;
     return launch_stream_kernel(ctx, a, cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream);
 }
 
@@ -2654,7 +2774,80 @@ int mbe_b200_pipeline_plan(int n_streams, int* sizes, int cap) {
 
 static int frames_host_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_stream, int n_streams, int n_frames,
                             const uint8_t* frames, int16_t* pcm, float* pcmf, mbe_b200_result* results, uint8_t* bits,
-                            bool wait = true);
+                            bool wait = true, const int32_t* slots = nullptr);
+
+// A new claim epoch for an indexed call and the claim launch over its whole device slot list on `st`.  After 2^32 - 1
+// calls the epochs start over from a cleared claim table (nothing of the device may still read it).
+static int claim_slots(mbe_b200_ctx* ctx, const int32_t* d_slots, int n, cudaStream_t st, unsigned* epoch) {
+    if (++ctx->claim_epoch == 0u) {
+        CU(cudaDeviceSynchronize());
+        CU(cudaMemsetAsync(ctx->d_claim, 0, (size_t)ctx->max_streams * sizeof(unsigned long long), st));
+        ctx->claim_epoch = 1u;
+    }
+    *epoch = ctx->claim_epoch;
+    const int threads = 256;
+    const int blocks = (n + threads - 1) / threads < 4096 ? (n + threads - 1) / threads : 4096;
+    mbe_claim_kernel<<<blocks, threads, 0, st>>>(d_slots, n, ctx->max_streams, ctx->d_claim, *epoch);
+    ctx->launches++;
+    CU(cudaGetLastError());
+    return 0;
+}
+
+static int check_indexed(mbe_b200_ctx* ctx, const char* what, int codec, int input, const int32_t* slots, int n, int n_frames,
+                         const uint8_t* in) {
+    if (!ctx) {
+        return MBE_B200_E_ARG;
+    }
+    if (codec < 0 || codec > 3 || input < MBE_B200_INPUT_HARD || input > MBE_B200_INPUT_PACKED || n < 0 || n_frames < 0 ||
+        (n > 0 && !slots) || !in) {
+        char msg[96];
+        snprintf(msg, sizeof(msg), "%s: bad argument", what);
+        return fail(ctx, MBE_B200_E_ARG, msg, cudaSuccess);
+    }
+    return 0;
+}
+
+int mbe_b200_process_indexed_dev(mbe_b200_ctx* ctx, int codec, int input, const int32_t* d_slots, int n, int n_frames,
+                                 const uint8_t* d_in, int16_t* d_pcm, float* d_pcmf, mbe_b200_result* d_results,
+                                 uint8_t* d_bits, void* cuda_stream) {
+    int rc = check_indexed(ctx, "process_indexed_dev", codec, input, d_slots, n, n_frames, d_in);
+    if (rc < 0 || n == 0 || n_frames == 0) {
+        return rc;
+    }
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
+    unsigned epoch = 0;
+    if ((rc = claim_slots(ctx, d_slots, n, st, &epoch)) < 0) {
+        return rc;
+    }
+    return frames_dev_impl(ctx, codec, input, 0, n, n_frames, d_in, d_pcm, d_pcmf, d_results, d_bits, st, d_slots, 0, epoch);
+}
+
+int mbe_b200_process_indexed(mbe_b200_ctx* ctx, int codec, int input, const int32_t* slots, int n, int n_frames,
+                             const uint8_t* in, int16_t* pcm, float* pcmf, mbe_b200_result* results, uint8_t* bits) {
+    const int rc = check_indexed(ctx, "process_indexed", codec, input, slots, n, n_frames, in);
+    if (rc < 0) {
+        return rc;
+    }
+    return frames_host_impl(ctx, codec, input, 0, n, n_frames, in, pcm, pcmf, results, bits, true, slots);
+}
+
+int mbe_b200_submit_indexed(mbe_b200_ctx* ctx, int codec, int input, const int32_t* slots, int n, int n_frames,
+                            const uint8_t* in, int16_t* pcm, float* pcmf, mbe_b200_result* results, uint8_t* bits) {
+    int rc = check_indexed(ctx, "submit_indexed", codec, input, slots, n, n_frames, in);
+    if (rc < 0) {
+        return rc;
+    }
+    if (ctx->pending) {
+        return fail(ctx, MBE_B200_E_ARG, "submit_indexed: a submission is still pending (call mbe_b200_wait first)",
+                    cudaSuccess);
+    }
+    rc = frames_host_impl(ctx, codec, input, 0, n, n_frames, in, pcm, pcmf, results, bits, false, slots);
+    if (rc == 0) {
+        ctx->pending = 1;
+    }
+    return rc;
+}
 
 int mbe_b200_wait(mbe_b200_ctx* ctx) {
     if (!ctx) {
@@ -2695,8 +2888,8 @@ int mbe_b200_process_frames_packed(mbe_b200_ctx* ctx, int codec, int first_strea
 
 static int frames_host_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_stream, int n_streams, int n_frames,
                             const uint8_t* frames, int16_t* pcm, float* pcmf, mbe_b200_result* results, uint8_t* bits,
-                            bool wait) {
-    int rc = check_range(ctx, first_stream, n_streams);
+                            bool wait, const int32_t* slots) {
+    int rc = slots ? 0 : check_range(ctx, first_stream, n_streams);   // (indexed: checked by check_indexed)
     if (rc == 0 && ctx->pending) {
         return fail(ctx, MBE_B200_E_ARG, "process_frames: a submission is still pending (call mbe_b200_wait first)", cudaSuccess);
     }
@@ -2761,6 +2954,18 @@ static int frames_host_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_st
         for (int i = 0; i < MAX_KSTREAMS; ++i) {
             CU(cudaStreamWaitEvent(ctx->s_k[i], ctx->ev_start, 0));
         }
+        // indexed: the slot list goes up once and is claimed as a whole ahead of the first chunk's frames (every chunk's
+        // kernel waits for its copy-in, which s_in orders after the claim)
+        unsigned epoch = 0;
+        if (slots) {
+            int rs = upload_slots(ctx, slots, n_streams, ctx->s_in);
+            if (rs == 0) {
+                rs = claim_slots(ctx, ctx->d_slots, n_streams, ctx->s_in, &epoch);
+            }
+            if (rs < 0) {
+                return rs;
+            }
+        }
         int s0 = 0;
         for (int c = 0; c < n_chunks; s0 += sizes[c], ++c) {
             const int ns = sizes[c];
@@ -2775,7 +2980,8 @@ static int frames_host_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_st
             mbe_b200_result* const o_res = results ? (mbe_b200_result*)ctx->d_out[2] + f0 : nullptr;
             uint8_t* const o_bits = bits ? (uint8_t*)ctx->d_out[3] + f0 * pb : nullptr;
             const uint8_t* const i_fr = (const uint8_t*)ctx->d_in + f0 * in_per_frame;
-            const int rk = frames_dev_impl(ctx, codec, kind, first_stream + s0, ns, n_frames, i_fr, o_pcm, o_pcmf, o_res, o_bits, sk);
+            const int rk = frames_dev_impl(ctx, codec, kind, first_stream + s0, ns, n_frames, i_fr, o_pcm, o_pcmf, o_res, o_bits, sk,
+                                           slots ? ctx->d_slots : nullptr, s0, epoch);
             if (rk < 0) {
                 return rk;
             }

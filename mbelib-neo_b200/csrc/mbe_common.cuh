@@ -235,7 +235,25 @@ struct LaunchArgs {
     float pcmf_scale;           // float PCM is multiplied by this on store: 1 (reference scale) or 7/32768 (normalised)
     uint32_t* desc;             // split path: frame descriptors [n_streams][n_frames][DESC_WORDS] (mbe_split.cuh)
     int io_base;                // stream s of the launch is element io_base + s of the caller's frame / PCM / result arrays
+    // indexed calls (mbe_b200_process_indexed*): element e = slot_base + io_base + s of the call decodes stream slot
+    // slots[e] (slots == nullptr: the contiguous range first_stream + s).  The element owns its slot only when the slot is in
+    // [0, max_streams) and claim[slot] holds its own tag (claim_tag: the first occurrence of a repeated slot wins).
+    const int32_t* slots;
+    const unsigned long long* claim;
+    unsigned epoch;
+    int slot_base, max_streams;
 };
+
+// the claim an element of an indexed call leaves on its slot: later calls have larger epochs, earlier elements larger tags
+__host__ __device__ __forceinline__ unsigned long long claim_tag(unsigned epoch, int e) {
+    return ((unsigned long long)epoch << 32) | (0xffffffffu - (unsigned)e);
+}
+
+// state slot of stream s of a launch (LaunchArgs, SynthArgs): the contiguous range, or the slot an indexed call lists
+template <class Args>
+__device__ __forceinline__ int slot_of(const Args& A, int s) {
+    return A.slots ? A.slots[A.slot_base + A.io_base + s] : A.first_stream + s;
+}
 
 
 // Tables every warp of a block reads with lane-varying indices on the synthesis path, staged into

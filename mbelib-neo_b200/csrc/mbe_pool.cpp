@@ -16,6 +16,9 @@ struct mbe_b200_pool {
     std::vector<mbe_b200_ctx*> ctx;
     std::vector<int> first;   // global id of the first stream of each shard (+ one past the end)
     int max_streams;
+    // indexed calls: per shard, a pinned staging buffer (mbe_b200_host_alloc, grown on demand) its elements are gathered into
+    std::vector<void*> stage;
+    std::vector<size_t> stage_cap;
     char err[320];
 };
 
@@ -60,6 +63,8 @@ int mbe_b200_pool_create(mbe_b200_pool** out, int n_devices, const int* device_o
         p->ctx.push_back(c);
     }
     p->first.push_back(max_streams);
+    p->stage.assign(p->ctx.size(), nullptr);
+    p->stage_cap.assign(p->ctx.size(), 0);
     *out = p;
     return 0;
 }
@@ -70,6 +75,11 @@ void mbe_b200_pool_destroy(mbe_b200_pool* p) {
     }
     for (mbe_b200_ctx* c : p->ctx) {
         mbe_b200_destroy(c);
+    }
+    for (void* b : p->stage) {
+        if (b) {
+            mbe_b200_host_free(b);
+        }
     }
     delete p;
 }
@@ -204,6 +214,177 @@ int mbe_b200_pool_process_frames_packed(mbe_b200_pool* p, int codec, int first_s
                                         uint8_t* bits) {
     return pool_process(p, "pool_process_frames_packed", codec, 0, 1, first_stream, n_streams, n_frames, packed, pcm, pcmf,
                         results, bits);
+}
+
+}  // extern "C"
+
+// ---- indexed calls -----------------------------------------------------------------------------------------------------
+// shard owning global slot `slot` (in range)
+static int shard_of(const mbe_b200_pool* p, int slot) {
+    return (int)(std::upper_bound(p->first.begin(), p->first.end(), slot) - p->first.begin()) - 1;
+}
+
+// run fn(shard, ctx, element positions of that shard) on every shard that owns an element, one host thread per shard
+template <class F>
+static int for_each_part(mbe_b200_pool* p, const char* what, const std::vector<std::vector<int>>& part, F fn) {
+    const int n = (int)p->ctx.size();
+    std::vector<int> rc(n, 0);
+    std::vector<std::thread> th;
+    for (int i = 0; i < n; ++i) {
+        if (!part[i].empty()) {
+            th.emplace_back([&, i]() { rc[i] = fn(i, p->ctx[i], part[i]); });
+        }
+    }
+    for (std::thread& t : th) {
+        t.join();
+    }
+    for (int i = 0; i < n; ++i) {
+        if (rc[i] != 0) {
+            snprintf(p->err, sizeof(p->err), "%s: shard %d: %s", what, i, mbe_b200_last_error(p->ctx[i]));
+            return rc[i];
+        }
+    }
+    return 0;
+}
+
+static int grow_stage(mbe_b200_pool* p, int shard, size_t bytes) {
+    if (bytes <= p->stage_cap[shard]) {
+        return 0;
+    }
+    if (p->stage[shard]) {
+        mbe_b200_host_free(p->stage[shard]);
+        p->stage[shard] = nullptr;
+        p->stage_cap[shard] = 0;
+    }
+    const int rc = mbe_b200_host_alloc(&p->stage[shard], bytes);
+    if (rc == 0) {
+        p->stage_cap[shard] = bytes;
+    }
+    return rc;
+}
+
+static size_t align64(size_t x) { return (x + 63) & ~(size_t)63; }
+
+extern "C" {
+
+int mbe_b200_pool_process_indexed(mbe_b200_pool* p, int codec, int input, const int32_t* slots, int n, int n_frames,
+                                  const uint8_t* in, int16_t* pcm, float* pcmf, mbe_b200_result* results, uint8_t* bits) {
+    if (!p) {
+        return MBE_B200_E_ARG;
+    }
+    int fbits = 0, pbits = 0;
+    if (mbe_b200_geometry(codec, &fbits, &pbits) != 0 || input < MBE_B200_INPUT_HARD || input > MBE_B200_INPUT_PACKED ||
+        n < 0 || n_frames < 0 || (n > 0 && !slots) || !in) {
+        snprintf(p->err, sizeof(p->err), "pool_process_indexed: bad argument");
+        return MBE_B200_E_ARG;
+    }
+    if (n == 0 || n_frames == 0) {
+        return 0;
+    }
+    const size_t F = (size_t)n_frames, NS = MBE_B200_SAMPLES_PER_FRAME;
+    const size_t fbytes = input == MBE_B200_INPUT_PACKED ? (size_t)mbe_b200_channel_frame_bytes(p->ctx[0], codec)
+                                                         : (size_t)fbits * (input == MBE_B200_INPUT_SOFT ? 2u : 1u);
+    // stable partition of the element positions by owning shard: a slot always maps to one shard, so the context's
+    // first-occurrence rule holds for the whole list; out-of-range elements are rejected here, like a context does
+    std::vector<std::vector<int>> part(p->ctx.size());
+    for (int i = 0; i < n; ++i) {
+        const int slot = slots[i];
+        if (slot >= 0 && slot < p->max_streams) {
+            part[shard_of(p, slot)].push_back(i);
+            continue;
+        }
+        if (pcm) {
+            memset(pcm + (size_t)i * F * NS, 0, F * NS * sizeof(int16_t));
+        }
+        if (pcmf) {
+            memset(pcmf + (size_t)i * F * NS, 0, F * NS * sizeof(float));
+        }
+        if (bits) {
+            memset(bits + (size_t)i * F * pbits, 0, F * (size_t)pbits);
+        }
+        if (results) {
+            for (size_t f = 0; f < F; ++f) {
+                mbe_b200_result& r = results[(size_t)i * F + f];
+                memset(&r, 0, sizeof(r));
+                r.status = -1;   // MBE_STATUS_INVALID_ARGUMENT
+            }
+        }
+    }
+    return for_each_part(p, "pool_process_indexed", part, [&](int shard, mbe_b200_ctx* c, const std::vector<int>& el) {
+        const size_t m = el.size();
+        // staging layout: local slots | frames | pcm | pcmf | results | bits
+        const size_t b_slots = align64(m * sizeof(int32_t)), b_in = align64(m * F * fbytes);
+        const size_t b_pcm = pcm ? align64(m * F * NS * sizeof(int16_t)) : 0, b_pcmf = pcmf ? align64(m * F * NS * sizeof(float)) : 0;
+        const size_t b_res = results ? align64(m * F * sizeof(mbe_b200_result)) : 0, b_bits = bits ? align64(m * F * pbits) : 0;
+        int rc = grow_stage(p, shard, b_slots + b_in + b_pcm + b_pcmf + b_res + b_bits);
+        if (rc != 0) {
+            return rc;
+        }
+        uint8_t* base = (uint8_t*)p->stage[shard];
+        int32_t* l_slots = (int32_t*)base;
+        uint8_t* l_in = base + b_slots;
+        int16_t* l_pcm = pcm ? (int16_t*)(l_in + b_in) : nullptr;
+        float* l_pcmf = pcmf ? (float*)(l_in + b_in + b_pcm) : nullptr;
+        mbe_b200_result* l_res = results ? (mbe_b200_result*)(l_in + b_in + b_pcm + b_pcmf) : nullptr;
+        uint8_t* l_bits = bits ? l_in + b_in + b_pcm + b_pcmf + b_res : nullptr;
+        const int lo = p->first[shard];
+        for (size_t k = 0; k < m; ++k) {
+            l_slots[k] = slots[el[k]] - lo;
+            memcpy(l_in + k * F * fbytes, in + (size_t)el[k] * F * fbytes, F * fbytes);
+        }
+        rc = mbe_b200_process_indexed(c, codec, input, l_slots, (int)m, n_frames, l_in, l_pcm, l_pcmf, l_res, l_bits);
+        if (rc != 0) {
+            return rc;
+        }
+        for (size_t k = 0; k < m; ++k) {
+            const size_t g = (size_t)el[k];
+            if (pcm) {
+                memcpy(pcm + g * F * NS, l_pcm + k * F * NS, F * NS * sizeof(int16_t));
+            }
+            if (pcmf) {
+                memcpy(pcmf + g * F * NS, l_pcmf + k * F * NS, F * NS * sizeof(float));
+            }
+            if (results) {
+                memcpy(results + g * F, l_res + k * F, F * sizeof(mbe_b200_result));
+            }
+            if (bits) {
+                memcpy(bits + g * F * pbits, l_bits + k * F * pbits, F * (size_t)pbits);
+            }
+        }
+        return 0;
+    });
+}
+
+int mbe_b200_pool_init_streams_indexed(mbe_b200_pool* p, const int32_t* slots, int n, const uint32_t* seeds) {
+    if (!p) {
+        return MBE_B200_E_ARG;
+    }
+    if (n < 0 || (n > 0 && !slots)) {
+        snprintf(p->err, sizeof(p->err), "pool_init_streams_indexed: bad argument");
+        return MBE_B200_E_ARG;
+    }
+    std::vector<unsigned char> seen(n > 0 ? (size_t)p->max_streams : 0, 0);
+    std::vector<std::vector<int>> part(p->ctx.size());
+    for (int i = 0; i < n; ++i) {
+        const int slot = slots[i];
+        if (slot < 0 || slot >= p->max_streams || seen[slot]) {
+            snprintf(p->err, sizeof(p->err), "pool_init_streams_indexed: a slot is outside the pool or listed twice");
+            return MBE_B200_E_ARG;
+        }
+        seen[slot] = 1;
+        part[shard_of(p, slot)].push_back(i);
+    }
+    return for_each_part(p, "pool_init_streams_indexed", part, [&](int shard, mbe_b200_ctx* c, const std::vector<int>& el) {
+        std::vector<int32_t> l_slots(el.size());
+        std::vector<uint32_t> l_seeds(seeds ? el.size() : 0);
+        for (size_t k = 0; k < el.size(); ++k) {
+            l_slots[k] = slots[el[k]] - p->first[shard];
+            if (seeds) {
+                l_seeds[k] = seeds[el[k]];
+            }
+        }
+        return mbe_b200_init_streams_indexed(c, l_slots.data(), (int)el.size(), seeds ? l_seeds.data() : nullptr);
+    });
 }
 
 }  // extern "C"

@@ -236,6 +236,8 @@ struct SynthArgs {
     const DevTables* tab;
     unsigned long long* counters;   // profiling (may be null): [0] oscillator slots run, [1] of them interpolated harmonics,
                                     // [2] frames synthesised
+    const int32_t* slots;   // indexed calls: as LaunchArgs (slot_of)
+    int slot_base;
 };
 
 // Oscillator tile of the bank kernel: 32 samples x 32 slots, rows padded to 36 words: phase A (lane = slot, one row per
@@ -561,7 +563,8 @@ __global__ void __launch_bounds__(U_WARPS * 32, U_MINB) mbe_split_unvoiced_kerne
     UnvWS& ws = wsa[warp];
     const int s = blockIdx.x * U_WARPS + warp;
     const bool live = s < A.n_streams;
-    uint32_t* gs = A.state + (size_t)(A.first_stream + (live ? s : 0)) * STATE_WORDS;
+    // (an element an indexed call rejected left descriptors without ops: its slot, possibly out of range, is never used)
+    uint32_t* gs = A.state + (size_t)(live ? slot_of(A, s) : A.first_stream) * STATE_WORDS;
     uint32_t* h_cur = gs;
     uint32_t* h_prev = gs + PARMS_WORDS;
     uint32_t* h_enh = gs + 2 * PARMS_WORDS;
