@@ -4,8 +4,10 @@ compiled reference (oracle/_ref/*.so, optional) and seeded input generators.
 TEST INFRASTRUCTURE ONLY - nothing here is on the product path.
 """
 import ctypes
+import json
 import os
 import subprocess
+import sys
 
 import numpy as np
 
@@ -296,6 +298,90 @@ def oracle_ecc_blocks(code, words, soft, fast=True, n_threads=8):
     o.mbo_ecc_blocks(int(code), int(bool(soft)), int(bool(fast)), int(n), _ptr(np.ascontiguousarray(words)), _ptr(out), _ptr(st),
                      int(n_threads))
     return out, st
+
+
+def mixed_frames(codec, S, F, seed):
+    """random bits (repeats, mutes, re-initialisation), valid voice held for several frames (stable pitch: interpolated
+    harmonics), valid frames with flipped bits, and for the AMBE codecs tone / erasure frames."""
+    rng = np.random.default_rng(seed)
+    fb = FRAME_BITS[codec]
+    enc = {0: encode_imbe7200_frame, 1: encode_imbe7100_frame}.get(codec, encode_ambe_frame)
+    frames = rng.integers(0, 2, size=(S, F, fb), dtype=np.uint8)
+    for s in range(0, S, 2):
+        f = 0
+        while f < F:
+            n = int(min(F - f, rng.integers(2, 9)))
+            p = rng.integers(0, 2, size=PARAM_BITS[codec], dtype=np.uint8)
+            if codec <= 1:
+                p[codec] = 0
+            elif rng.random() < 0.15:
+                p[0:6] = 1                       # AMBE tone / erasure signatures
+                if rng.random() < 0.5:
+                    p[45:49] = 0
+            fr = enc(p).reshape(-1)
+            frames[s, f:f + n] = fr
+            if rng.random() < 0.4:
+                frames[s, f:f + n] ^= (rng.random((n, fb)) < 0.04).astype(np.uint8)
+            f += n
+    return frames
+
+
+def oracle_rng_words(codec, soft, frames, seeds, n_threads=8):
+    """Final RNG words [S][4] (export_rng layout) of each stream after the oracle decodes its frames from a fresh
+    init_streams: the part of the end state that mbo_run does not return.  Replays the streams frame by frame
+    (mbo_process_frame); ctypes releases the GIL, so threads over disjoint streams run in parallel."""
+    from concurrent.futures import ThreadPoolExecutor
+    o = load_oracle()
+    frames = np.ascontiguousarray(frames, dtype=np.uint8)
+    S, F = frames.shape[0], frames.shape[1]
+    stride = frames[0, 0].nbytes
+    out = np.zeros((S, 4), np.uint32)
+
+    def work(lo_hi):
+        bufs = dict(cur=np.zeros(PARMS_BYTES, np.uint8), prev=np.zeros(PARMS_BYTES, np.uint8),
+                    enh=np.zeros(PARMS_BYTES, np.uint8), rng=np.zeros(16, np.uint8), pf=np.zeros(160, np.float32),
+                    res=np.zeros(5, np.int32), d=np.zeros(88, np.uint8))
+        p = {k: _ptr(v) for k, v in bufs.items()}
+        for s in range(*lo_hi):
+            o.mbo_rng_default(p["rng"])
+            o.mbo_rng_seed(p["rng"], ctypes.c_uint32(int(seeds[s])))
+            o.mbo_init_parms(p["cur"], p["prev"], p["enh"])
+            for f in range(F):
+                fr = ctypes.c_void_p(frames.ctypes.data + (s * F + f) * stride)
+                o.mbo_process_frame(codec, int(bool(soft)), p["pf"], p["res"], fr, p["d"], p["cur"], p["prev"], p["enh"],
+                                    p["rng"])
+            out[s] = bufs["rng"].view(np.uint32)
+
+    step = (S + n_threads - 1) // n_threads
+    with ThreadPoolExecutor(n_threads) as ex:
+        list(ex.map(work, [(lo, min(S, lo + step)) for lo in range(0, S, step)]))
+    return out
+
+
+# Tuning knobs of libmbe_b200 read from the environment once per process (knobs() in mbe_b200.cu); a test that varies
+# them runs the library in a child process (tests/helpers/knob_child.py)
+KNOBS = ("MBE_B200_PAD_SMEM", "MBE_B200_CHUNKS", "MBE_B200_TAPER", "MBE_B200_KSTREAMS", "MBE_B200_AUX", "MBE_B200_SPLIT",
+         "MBE_B200_SKIP_KERNELS", "MBE_B200_DESC_MB")
+KNOB_CHILD = os.path.join(ROOT, "tests", "helpers", "knob_child.py")
+
+
+def run_knob_child(args, knobs, timeout):
+    """Run tests/helpers/knob_child.py with `args` under exactly the knob settings `knobs` ({name: value}; every other
+    knob is removed from the environment).  Returns its stdout; raises AssertionError with its output if it fails.  On a
+    timeout subprocess.run kills the child, so nothing outlives the call."""
+    env = {k: v for k, v in os.environ.items() if k not in KNOBS}
+    env.update({k: str(v) for k, v in knobs.items()})
+    cmd = [sys.executable] + (["-s"] if sys.flags.no_user_site else []) + [KNOB_CHILD] + [str(a) for a in args]
+    p = subprocess.run(cmd, env=env, timeout=timeout, capture_output=True, text=True)
+    if p.returncode != 0:
+        raise AssertionError("knob child %s failed (%d) under %s:\n%s\n%s" % (args[0], p.returncode, knobs, p.stdout[-4000:],
+                                                                            p.stderr[-4000:]))
+    return p.stdout
+
+
+def pipeline_plans(ns, knobs):
+    """{n: mbe_b200_pipeline_plan(n)} under `knobs`, from a child process (no device needed)."""
+    return {int(k): v for k, v in json.loads(run_knob_child(["plan"] + list(ns), knobs, timeout=120)).items()}
 
 
 def soften(frames_hard, rng, flip_p=0.0, rel_ok=255, rel_bad_max=64):

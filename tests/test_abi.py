@@ -88,6 +88,11 @@ def test_pool_has_no_cpu_fallback(pkg):
     assert "-3" in str(e.value)
 
 
+HALF_WAVE = 148 * 14
+PLAN_SIZES = (1, 13, 14, 15, 2072, 4 * HALF_WAVE, 4 * HALF_WAVE + 1, 20000, 65536, 66000, 131072, 262144, 1048576, 1048577,
+              4000000)
+
+
 def test_pipeline_plan_covers_every_stream_once(pkg):
     """Host logic of the host-pointer call (DESIGN 4.4): the chunk plan of a batch covers [0, n_streams) exactly once in
     order, small batches stay one chunk, large ones are tapered at both ends, and the plan never exceeds the event pool."""
@@ -97,9 +102,8 @@ def test_pipeline_plan_covers_every_stream_once(pkg):
     assert lib.mbe_b200_pipeline_plan(0, buf, 64) == 0
     assert lib.mbe_b200_pipeline_plan(-1, buf, 64) < 0
     assert lib.mbe_b200_pipeline_plan(10, None, 64) < 0
-    half_wave = 148 * 14
-    for n in (1, 13, 14, 15, 2072, 4 * half_wave, 4 * half_wave + 1, 20000, 65536, 66000, 131072, 262144, 1048576, 1048577,
-              4000000):
+    half_wave = HALF_WAVE
+    for n in PLAN_SIZES:
         k = lib.mbe_b200_pipeline_plan(n, buf, 64)
         assert 1 <= k <= 64, (n, k)
         sizes = list(buf[:k])
@@ -113,3 +117,35 @@ def test_pipeline_plan_covers_every_stream_once(pkg):
     assert sizes[0] == sizes[-1] == 18 * 14 and sizes[1] == sizes[-2] == 36 * 14
     assert max(sizes) == half_wave and sizes[:4] == sorted(sizes[:4]) and sizes[-4:] == sorted(sizes[-4:], reverse=True)
     assert all(s % 14 == 0 for s in sizes[:-5])
+
+
+def test_pipeline_plan_under_knobs(pkg):
+    """MBE_B200_CHUNKS / MBE_B200_TAPER (read once per process, so each setting runs in a child process) change how a
+    host call is cut, never what it covers: every plan covers [0, n_streams) within the event pool; an out-of-range value
+    is ignored; one chunk means one chunk; without a taper every chunk but the last has the same size; with one, a call
+    of at least four chunks starts with pieces of TAPER x 14 x 2^i streams (below a chunk, eight at most) and ends with
+    the same pieces mirrored, and the chunks between are whole."""
+    import mbe_testlib as T
+    chunks, tapers = (None, 1, 5, 64, 65), (None, 0, 1, 148, 149)
+    knobs = lambda c, t: {k: v for k, v in (("MBE_B200_CHUNKS", c), ("MBE_B200_TAPER", t)) if v is not None}
+    plans = {(c, t): T.pipeline_plans(PLAN_SIZES, knobs(c, t)) for c in chunks for t in tapers}
+    for (c, t), by_n in plans.items():
+        taper = 18 if t is None or t > 148 else t
+        for n, sizes in by_n.items():
+            where = (c, t, n, sizes)
+            assert 1 <= len(sizes) <= 64 and all(s > 0 for s in sizes) and sum(sizes) == n, where
+            if c == 65:
+                assert sizes == plans[None, t][n], where
+            if t == 149:
+                assert sizes == plans[c, None][n], where
+            if c == 1:
+                assert len(sizes) == 1, where
+            chunk = plans[c, 0][n][0]             # the taper does not change the chunk size: the untapered plan shows it
+            head = [taper * 14 << i for i in range(8) if taper * 14 << i < chunk] if taper and n >= 4 * chunk else []
+            assert sizes[:len(head)] == head and sizes[len(sizes) - len(head):] == head[::-1], where
+            body = sizes[len(head):len(sizes) - len(head)]
+            assert body and all(s == chunk for s in body[:-1]), where
+            if not taper:
+                assert body[-1] <= chunk, where
+    assert plans[64, 0][1048576] == [16576] * 63 + [4288]
+    assert plans[5, 1][1048576][:8] == [14 << i for i in range(8)]

@@ -1,8 +1,10 @@
 """GPU parity tests proper: the CUDA path (through the C-ABI, libmbe_b200.so) against the CPU oracle on the
-same seeded inputs.  Bars (BASELINE.json north_star):
+same seeded inputs.  Bars against the oracle (check_batch and the long-stream test):
   - ECC error counts, result flags and decoded parameter bits: bit-exact;
-  - int16 PCM: max |delta| <= 2 LSB and >= 99.99 % of samples exact (tolerance stated here);
-  - final mbe_parms triplets: integer fields exact, float fields compared bitwise and reported."""
+  - int16 PCM and float PCM: bit-exact;
+  - final mbe_parms triplets (previousUw / noiseOverlap / PHIl included): byte for byte.
+Against the compiled reference (oracle/_ref, when present) - a build of the reference, not the oracle - int16 PCM keeps the
+tolerance max |delta| <= 2 LSB with >= 99.99 % of samples exact; float PCM and state are reported."""
 import numpy as np
 import pytest
 
@@ -31,7 +33,25 @@ def dec(pkg, request):
     d.close()
 
 
-def check_batch(dec, codec, soft, frames, seeds, strict_state=True):
+def assert_pcm_exact(pcm, pcmf, want):
+    """int16 and float PCM bit for bit against the oracle; the message locates the first difference."""
+    for name, g, w in (("int16 PCM", pcm, want["pcm"]), ("float PCM", pcmf.view(np.uint32), want["pcmf"].view(np.uint32))):
+        ne = g != w
+        assert not ne.any(), "%s: %d of %d samples differ from the oracle, the first at (stream, frame, sample) %s" % (
+            name, int(ne.sum()), ne.size, tuple(int(i) for i in np.argwhere(ne)[0]))
+
+
+def assert_state_exact(st, want_state):
+    """Final mbe_parms triplets byte for byte against the oracle; the message names the first differing field."""
+    ne = st != want_state
+    if ne.any():
+        s, k, byte = (int(i) for i in np.argwhere(ne)[0])
+        field = max((off, name) for name, off in T.OFF.items() if off <= byte)[1]
+        raise AssertionError("final state differs from the oracle in %d streams, the first: stream %d, %s parms, field %s "
+                             "(byte %d)" % (int(ne.any(axis=(1, 2)).sum()), s, ("cur", "prev", "enh")[k], field, byte))
+
+
+def check_batch(dec, codec, soft, frames, seeds):
     S = frames.shape[0]
     dec.init_streams(0, S, seeds)
     got = dec.process_frames(codec, frames, soft=soft, want_float=True)
@@ -44,24 +64,13 @@ def check_batch(dec, codec, soft, frames, seeds, strict_state=True):
     assert np.array_equal(res["c4_errors"], want["results"][..., 3])
     assert np.array_equal(res["total_errors"], want["results"][..., 4])
     assert np.array_equal(res["flags"].astype(np.int64), want["results"][..., 5].astype(np.int64) & 0xffffffff)
-    d = np.abs(got["pcm"].astype(np.int32) - want["pcm"].astype(np.int32))
-    exact = float((d == 0).mean())
-    assert d.max() <= PCM_MAX_LSB, "max |delta| = %d LSB" % d.max()
-    assert exact >= PCM_EXACT_FRACTION, "only %.6f of samples exact" % exact
+    assert_pcm_exact(got["pcm"], got["pcmf"], want)
     st = dec.export_state(0, S)
-    state_equal = np.array_equal(st, want["state"])
-    if strict_state:
-        # integer fields of the final state must match exactly
-        for k in range(3):
-            for s in range(0, S, max(1, S // 16)):
-                a, b = T.parms_view(st[s, k]), T.parms_view(want["state"][s, k])
-                for name in ("L", "K", "repeatCount", "errorCountTotal", "errorCount4", "amplitudeThreshold", "swn"):
-                    assert a[name] == b[name], (name, s, k)
-                assert np.array_equal(a["Vl"], b["Vl"])
-    fexact = float((got["pcmf"].view(np.uint32) == want["pcmf"].view(np.uint32)).mean())
-    out = dict(exact=exact, maxd=int(d.max()), float_exact=fexact, state_equal=state_equal)
+    assert_state_exact(st, want["state"])
+    out = dict(frames=int(res.size))
     # Second checker, one hop closer: the UNMODIFIED reference compiled by oracle/Makefile (Release flags, the parity
-    # build of SURVEY 8(c)), when oracle/_ref travelled with the tree.  Same bars as against the port.
+    # build of SURVEY 8(c)), when oracle/_ref travelled with the tree.  Bit-exact ECC and parameters, int16 PCM within the
+    # tolerance of BASELINE.json: a build of the reference is not held to the oracle's bit-exact PCM bar.
     if T.ref_available(fast=False):
         ref = T.run_cpu(T.load_ref(fast=False).ref_bench_run, codec, soft, frames, seeds, n_threads=8)
         assert np.array_equal(res["status"], ref["results"][..., 0]), "status differs from the compiled reference"
@@ -517,8 +526,8 @@ def test_long_streams_stay_exact(dec, codec):
     """24 s of channel per stream (1200 frames x 48 streams), decoded in launches of 1 to 300 frames, against the oracle run
     in one go: steady voice (the same parameters held for several frames, so the pitch is stable and the low harmonics go
     through the phase-interpolated path), clean and noisy valid frames, random-bit bursts long enough to repeat, mute and
-    re-initialise, then recovery.  Nothing may drift: parameter bits and results exact over the whole run, PCM inside the
-    bar, final state integer fields exact."""
+    re-initialise, then recovery.  Nothing may drift: parameter bits, results, int16 and float PCM exact over the whole
+    run, final state byte for byte."""
     rng = np.random.default_rng(0x10C0 + codec)
     S, F, P = 48, 1200, 160
     fb = T.FRAME_BITS[codec]
@@ -553,24 +562,14 @@ def test_long_streams_stay_exact(dec, codec):
         cuts.append((f, min(F, f + n)))
         f = min(F, f + n)
     assert f == F
-    parts = [dec.process_frames(codec, np.ascontiguousarray(frames[:, a:b]), want_float=False) for a, b in cuts if b > a]
+    parts = [dec.process_frames(codec, np.ascontiguousarray(frames[:, a:b]), want_float=True) for a, b in cuts if b > a]
     pcm = np.concatenate([p["pcm"] for p in parts], axis=1)
+    pcmf = np.concatenate([p["pcmf"] for p in parts], axis=1)
     bits = np.concatenate([p["bits"] for p in parts], axis=1)
     res = np.concatenate([p["results"] for p in parts], axis=1)
     assert np.array_equal(bits, want["bits"])
     assert np.array_equal(res["status"], want["results"][..., 0])
     assert np.array_equal(res["total_errors"], want["results"][..., 4])
     assert np.array_equal(res["flags"].astype(np.int64), want["results"][..., 5].astype(np.int64) & 0xffffffff)
-    d = np.abs(pcm.astype(np.int32) - want["pcm"].astype(np.int32))
-    assert d.max() <= PCM_MAX_LSB, "max |delta| = %d LSB at frame %d" % (d.max(), int(np.argwhere(d == d.max())[0][1]))
-    assert float((d == 0).mean()) >= PCM_EXACT_FRACTION
-    # the last quarter of the run is as exact as the first: no drift
-    q = F // 4
-    assert float((d[:, -q:] == 0).mean()) >= PCM_EXACT_FRACTION
-    st = dec.export_state(0, S)
-    for s in range(S):
-        for k in range(3):
-            a, b = T.parms_view(st[s, k]), T.parms_view(want["state"][s, k])
-            for name in ("L", "K", "repeatCount", "errorCountTotal", "errorCount4", "amplitudeThreshold", "swn"):
-                assert a[name] == b[name], (name, s, k)
-    print(T.CODEC_NAMES[codec], "exact", float((d == 0).mean()), "state bytes equal", np.array_equal(st, want["state"]))
+    assert_pcm_exact(pcm, pcmf, want)
+    assert_state_exact(dec.export_state(0, S), want["state"])

@@ -16,37 +16,11 @@ def pkg():
     return load_package()
 
 
-def _mixed_frames(codec, S, F, seed):
-    """random bits (repeats, mutes, re-initialisation), valid voice held for several frames (stable pitch: interpolated
-    harmonics), valid frames with flipped bits, and for the AMBE codecs tone / erasure frames."""
-    rng = np.random.default_rng(seed)
-    fb = T.FRAME_BITS[codec]
-    enc = {0: T.encode_imbe7200_frame, 1: T.encode_imbe7100_frame}.get(codec, T.encode_ambe_frame)
-    frames = rng.integers(0, 2, size=(S, F, fb), dtype=np.uint8)
-    for s in range(0, S, 2):
-        f = 0
-        while f < F:
-            n = int(min(F - f, rng.integers(2, 9)))
-            p = rng.integers(0, 2, size=T.PARAM_BITS[codec], dtype=np.uint8)
-            if codec <= 1:
-                p[codec] = 0
-            elif rng.random() < 0.15:
-                p[0:6] = 1                       # AMBE tone / erasure signatures
-                if rng.random() < 0.5:
-                    p[45:49] = 0
-            fr = enc(p).reshape(-1)
-            frames[s, f:f + n] = fr
-            if rng.random() < 0.4:
-                frames[s, f:f + n] ^= (rng.random((n, fb)) < 0.04).astype(np.uint8)
-            f += n
-    return frames
-
-
 @pytest.mark.parametrize("codec", [0, 1, 2, 3])
 @pytest.mark.parametrize("soft", [0, 1])
 def test_split_equals_fused(pkg, codec, soft):
     S, F = (300, 40) if not soft else (60, 12)
-    frames = _mixed_frames(codec, S, F, 0x5917 + 10 * codec + soft)
+    frames = T.mixed_frames(codec, S, F, 0x5917 + 10 * codec + soft)
     if soft:
         rng = np.random.default_rng(codec)
         frames = T.soften(frames, rng, flip_p=0.05)
@@ -74,7 +48,8 @@ def test_split_equals_fused(pkg, codec, soft):
 def test_split_descriptor_buffer_ranges(pkg, monkeypatch):
     """A batch whose descriptors exceed the buffer budget is cut into stream ranges inside the call (MBE_B200_DESC_MB is read
     once per process, so this test only checks a batch much larger than one block through both paths: ragged last block,
-    stream window in the middle of the pool)."""
+    stream window in the middle of the pool; tests/test_gpu_knobs.py cuts real ranges under a 1 MiB budget in child
+    processes)."""
     codec, S, F = 3, 1000, 9
     frames = T.random_hard_frames(codec, S, F, 0xD5C)
     seeds = T.stream_seeds(S + 50, 7)
