@@ -107,7 +107,8 @@ MBE_B200_API int mbe_b200_kernel_path(const mbe_b200_ctx* ctx);
  * stream it runs on.  kernel_timing() synchronises and returns, per kernel kind (0 parameter or fused kernel, 1 bank
  * kernel, 2 unvoiced kernel), the summed device time in ms and the launch count since timing was enabled, plus the bank
  * kernel's work counters: [0] oscillator slots run (160 samples each), [1] of them phase-interpolated harmonics,
- * [2] frames synthesised. */
+ * [2] frames synthesised, [3] 32-slot passes the bank kernel ran (slots / (32 x passes) = its lane fill).  The fused
+ * kernel counts nothing. */
 MBE_B200_API int mbe_b200_set_kernel_timing(mbe_b200_ctx* ctx, int enable);
 MBE_B200_API int mbe_b200_kernel_timing(mbe_b200_ctx* ctx, double ms[3], long long launches[3], unsigned long long counters[4]);
 

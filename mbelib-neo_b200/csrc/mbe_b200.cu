@@ -2298,8 +2298,7 @@ static int launch_stream_kernel(mbe_b200_ctx* ctx, const LaunchArgs& a_in, cudaS
         sa.counters = ctx->kt_on ? ctx->d_cnt : nullptr;
         sa.slots = a.slots;
         sa.slot_base = a.slot_base;
-        const long long groups = ((long long)ns * a.n_frames + BG - 1) / BG;
-        long long bank_blocks = (groups + B_WARPS - 1) / B_WARPS;
+        long long bank_blocks = ((long long)ns * a.n_frames + B_WARPS - 1) / B_WARPS;   // at least one frame per warp
         const long long resident = (long long)g_sm_count.load() * B_MINB;   // grid-stride warps: one resident wave is enough
         if (bank_blocks > resident) {
             bank_blocks = resident;

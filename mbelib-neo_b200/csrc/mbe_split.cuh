@@ -8,9 +8,10 @@
 //                      warps on the same code share their instruction fetches).
 //   bank kernel        mbe_split_bank_kernel: the voiced oscillator bank (mbelib.c:953-1040) and nothing else - a loop of a
 //                      few hundred instructions that stays in the instruction cache, so its warps need no lockstep: a warp
-//                      pools the components of BG consecutive frames into 32-slot passes over its private 32 x 32 tile
-//                      (phase A: lane = slot runs the reference's unfused rotation recurrence; phase B: lane = sample adds
-//                      each frame's slots in the reference's order).  One warp's latency-bound ordered sums overlap another
+//                      lays the components of the frames it visits end to end and runs them in 32-slot passes over its
+//                      private 32 x 32 tile, a pass crossing frame boundaries freely (phase A: lane = slot runs the
+//                      reference's unfused rotation recurrence; phase B: lane = sample adds each frame's slots in the
+//                      reference's order).  One warp's latency-bound ordered sums overlap another
 //                      warp's FP32-dense recurrences, and a frame with many harmonics delays nobody else.
 //   unvoiced kernel    mbe_split_unvoiced_kernel: 256-point FFT / IFFT unvoiced synthesis with weighted overlap-add
 //                      (mbe_unvoiced_fft.c:714-761), soft clip, float -> int16.  It owns the previousUw arrays of the
@@ -46,9 +47,6 @@ constexpr int D_VOICED = D_G;  // the bank kernel leaves the frame's 160 voiced 
 constexpr int DESC_WORDS = 768;
 static_assert(D_SD + 112 <= DESC_WORDS && D_VOICED + NS <= D_S, "descriptor layout");
 
-#ifndef MBE_BG
-#define MBE_BG 3
-#endif
 #ifndef MBE_BWARPS
 #define MBE_BWARPS 8
 #endif
@@ -64,7 +62,6 @@ static_assert(D_SD + 112 <= DESC_WORDS && D_VOICED + NS <= D_S, "descriptor layo
 #ifndef MBE_U_LOCKSTEP
 #define MBE_U_LOCKSTEP 0
 #endif
-constexpr int BG = MBE_BG;            // frames pooled per warp of the bank kernel
 constexpr int B_WARPS = MBE_BWARPS;   // warps per block of the bank kernel
 constexpr int B_MINB = MBE_BMINB;
 constexpr int U_WARPS = MBE_UWARPS;   // warps (= streams) per block of the unvoiced kernel
@@ -235,7 +232,7 @@ struct SynthArgs {
     uint32_t* state;        // [max_streams][STATE_WORDS]: only the previousUw words are touched
     const DevTables* tab;
     unsigned long long* counters;   // profiling (may be null): [0] oscillator slots run, [1] of them interpolated harmonics,
-                                    // [2] frames synthesised
+                                    // [2] frames synthesised, [3] 32-slot passes of the bank kernel
     const int32_t* slots;   // indexed calls: as LaunchArgs (slot_of)
     int slot_base;
 };
@@ -250,7 +247,7 @@ constexpr int BT_STRIDE = 36;
 constexpr int BANK_STEPS = MBE_BANK_STEPS;   // oscillator steps per loop body of phase A (8 / 16 / 32)
 struct __align__(16) BankWS {
     float tile[32 * BT_STRIDE];
-    float out[BG][NS];      // voiced samples of the group's frames (lane i owns i, 32 + i, ...)
+    float carry[NS];        // running sums of the frame a pass left open (lane i owns i, 32 + i, ...); 0 while none is
 };
 
 // smem: voiced window halves (BlockTables::voiced_win layout, 336 floats) | n / 160 for n = 0..159 | per-warp workspaces
@@ -272,177 +269,197 @@ __global__ void __launch_bounds__(B_WARPS * 32, B_MINB) mbe_split_bank_kernel(co
     const int lane = threadIdx.x & 31;
     BankWS& ws = wsa[warp];
     float* tile = ws.tile;
-    const long long n_items = (long long)A.n_streams * A.n_frames;
-    const long long n_groups = (n_items + BG - 1) / BG;
-    const long long warps_total = (long long)gridDim.x * B_WARPS;
-    // the grid is resident (a few blocks per SM); every warp walks groups of BG consecutive frames with a grid stride
-#pragma unroll 1
-    for (long long grp = (long long)blockIdx.x * B_WARPS + warp; grp < n_groups; grp += warps_total) {
-        const long long i0 = grp * BG;
-        const int n_live = (int)min((long long)BG, n_items - i0);
-        uint32_t* const d0 = A.desc + (size_t)i0 * DESC_WORDS;
-
-        int off[BG + 1], cnt[BG];
-        int total = 0;
-        unsigned go_mask = 0;   // frames of the group that run the synthesis (bit q)
 #pragma unroll
-        for (int q = 0; q < BG; ++q) {
-            off[q] = total;
-            cnt[q] = 0;
-            if (q < n_live) {
-                const unsigned info = d0[(size_t)q * DESC_WORDS + D_INFO];
-                if (info & 1u) {
-                    go_mask |= 1u << q;
-                    cnt[q] = (int)((info >> 16) & 255u);
-                    total += (cnt[q] + 3) & ~3;
-                }
+    for (int c = 0; c < 5; ++c) {
+        ws.carry[32 * c + lane] = 0.0f;
+    }
+    // The grid is resident (a few blocks per SM); warp gw visits frames gw, gw + W, gw + 2 W, ... (W warps in the grid).  The
+    // oscillator slots of the frames it visits form one queue in visit order, each frame's list padded to a multiple of four
+    // (a four-slot group of the tile never straddles frames), and every pass takes the next 32 slots of that queue: only the
+    // warp's last pass runs part empty.  Frame sums are independent, so a pass may hold the tail of one frame, whole frames and
+    // the head of another; what a frame has summed when a pass ends inside it waits in ws.carry.
+    const long long n_items = (long long)A.n_streams * A.n_frames;
+    const long long gw = (long long)blockIdx.x * B_WARPS + warp;
+    const long long warps_total = (long long)gridDim.x * B_WARPS;
+    auto frame_desc = [&](int v) { return A.desc + (size_t)(gw + (long long)v * warps_total) * DESC_WORDS; };
+
+    // The window: frames v0 .. v0 + 31 of the walk, lane j holding frame v0 + j.  Queue positions count from the window's
+    // first slot; pos is where the next pass starts.
+    int v0 = 0, pos = 0;
+    int v_seen = 0;            // frames of the walk before this one were counted and, when they have no slots, zeroed already
+    unsigned win = 0u;         // lane j: end of frame j's padded slots in the queue | its slot count << 16 (0 without synthesis)
+    int total = 0, n_live = 0; // end of the window's queue; frames of the window that exist
+    int n_slots = 0;           // profiling counters (this lane's share of [0]; [1], [2] and [3] are warp-uniform)
+    int n_k2 = 0, n_go = 0, n_pass = 0;
+    auto load_window = [&]() {
+        const long long it = gw + (long long)(v0 + lane) * warps_total;
+        const bool live = it < n_items;
+        unsigned info = 0u;
+        if (live) {
+            info = A.desc[(size_t)it * DESC_WORDS + D_INFO];
+        }
+        const int cnt = (info & 1u) ? (int)((info >> 16) & 255u) : 0;
+        int e = (cnt + 3) & ~3;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const int t = __shfl_up_sync(FULL, e, d);
+            if (lane >= d) {
+                e += t;
             }
         }
-        off[BG] = total;
-        if (go_mask == 0u) {
-            continue;   // (no frame of the group runs the synthesis: nothing to leave behind)
-        }
-#pragma unroll
-        for (int q = 0; q < BG; ++q) {
+        win = (unsigned)e | ((unsigned)cnt << 16);
+        total = __shfl_sync(FULL, e, 31);
+        n_live = __popc(__ballot_sync(FULL, live));
+        const bool fresh = (info & 1u) && v0 + lane >= v_seen;
+        n_go += __popc(__ballot_sync(FULL, fresh));
+        n_slots += fresh ? cnt : 0;
+        // a frame that runs the synthesis without a slot still gets its 160 zero samples
+        for (unsigned zm = __ballot_sync(FULL, fresh && cnt == 0); zm; zm &= zm - 1u) {
+            uint32_t* d = frame_desc(v0 + __ffs(zm) - 1);
 #pragma unroll
             for (int c = 0; c < 5; ++c) {
-                ws.out[q][32 * c + lane] = 0.0f;
+                d[D_VOICED + 32 * c + lane] = 0u;
             }
         }
-
-        int n_k2 = 0;   // interpolated harmonics of the group (profiling counter)
+        v_seen = v0 + 32;
+    };
+    load_window();
 #pragma unroll 1
-        for (int base = 0; base < total; base += 32) {
-            const int k = base + lane;
-            int q = 0;
+    while (true) {
+        // frames of the window wholly before pos (the next one holds pos); once fewer than 32 slots are left, the window moves
+        // on to start at that frame so that the pass can be filled
+        const int j0 = __popc(__ballot_sync(FULL, (int)(win & 0xffffu) <= pos));
+        if (j0 == 32 && n_live < 32) {
+            break;
+        }
+        if (n_live == 32 && total - pos < 32 && j0 > 0) {
+            const int start = __shfl_sync(FULL, (int)(win & 0xffffu), j0 - 1);
+            pos = (j0 == 32) ? 0 : pos - start;
+            v0 += j0;
+            load_window();
+            continue;
+        }
+        ++n_pass;
+        // the window frame j that owns queue position pos + lane: the first whose end lies beyond it (31 past the queue's end,
+        // where nothing is used)
+        const int p = pos + lane;
+        int j = 0;
 #pragma unroll
-            for (int t = 1; t < BG; ++t) {
-                q += (off[t] <= k) ? 1 : 0;
-            }
-            int ofs_q = off[0], cnt_q = cnt[0];
-#pragma unroll
-            for (int t = 1; t < BG; ++t) {
-                if (q == t) {
-                    ofs_q = off[t];
-                    cnt_q = cnt[t];
-                }
-            }
-            const int pos = k - ofs_q;
-            const bool used = pos < cnt_q;
-            float g = 0.f, c = 0.f, s = 0.f, cd = 0.f, sd = 0.f, dw0 = 0.f;
-            int kind = 0, l = 0;
-            if (used) {
-                const uint32_t* d = d0 + (size_t)q * DESC_WORDS;
-                const unsigned id = reinterpret_cast<const unsigned char*>(d + D_KIND)[pos];
-                kind = (int)(id & 3u);
-                l = (int)(id >> 2);
-                g = __uint_as_float(d[D_G + pos]);
-                c = __uint_as_float(d[D_C + pos]);
-                s = __uint_as_float(d[D_S + pos]);
-                cd = __uint_as_float(d[D_CD + pos]);
-                sd = __uint_as_float(d[D_SD + pos]);
-                dw0 = __uint_as_float(d[D_DW0]);
-            }
-            const bool k2lane = (kind == 2);
-            const unsigned k2mask = __ballot_sync(FULL, k2lane);
-            n_k2 += __popc(k2mask);
-            const float* Wb = vwin + ((kind == 0) ? WIN_PREV : 0);
-            const float gg = k2lane ? 0.0f : g;   // interpolated slots are written by whoever renders them
-            const float rec_c = c, rec_s = s;     // (the recurrence below rotates c and s on every lane)
-            // phase B's map of the pass: which frame owns each four-slot group of the tile (a frame's slots start at a multiple
-            // of four, so a group never straddles frames): bit 4g of (fq0, fq1) = frame of group g, fchg = groups where it changes
-            static_assert(BG <= 8, "three bits per group");
-            const unsigned fq0 = __ballot_sync(FULL, (q & 1) != 0), fq1 = __ballot_sync(FULL, (q & 2) != 0);
-            const unsigned fq2 = (BG > 4) ? __ballot_sync(FULL, (q & 4) != 0) : 0u;
-            const unsigned fchg = (fq0 ^ (fq0 << 4)) | (fq1 ^ (fq1 << 4)) | (fq2 ^ (fq2 << 4));
-            const int ng = min(8, (total - base) >> 2);   // groups of this pass that hold slots
-#pragma unroll 1
-            for (int ch = 0; ch < 5; ++ch) {
-                // phase A: 32 oscillator steps, sixteen per loop body (the body stays in the L0 instruction cache)
-                const float4* W4 = reinterpret_cast<const float4*>(Wb) + 8 * ch;
-                float* tp = tile + lane;
-#pragma unroll 1
-                for (int h = 0; h < 32 / BANK_STEPS; ++h) {
-#pragma unroll
-                    for (int n4 = 0; n4 < BANK_STEPS / 4; ++n4) {
-                        const float4 w4 = W4[(BANK_STEPS / 4) * h + n4];
-                        const float wv[4] = {w4.x, w4.y, w4.z, w4.w};
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            if (!k2lane) {
-                                tp[(4 * n4 + i) * BT_STRIDE] = (gg * wv[i]) * c;   // row n = BANK_STEPS h + 4 n4 + i
-                            }
-                            const float cn = (c * cd) - (s * sd);
-                            const float sn = (s * cd) + (c * sd);
-                            c = cn;
-                            s = sn;
-                        }
-                    }
-                    tp += BANK_STEPS * BT_STRIDE;
-                }
-                // phase-interpolated harmonics of this pass: lane = sample (mbelib.c:953-968); the slot's lane holds its record
-                if (k2mask) {
-                    const int n = 32 * ch + lane;
-                    const float fn = (float)n, fr = nfrac[n];
-                    const int nn = n * n;
-                    for (unsigned m = k2mask; m; m &= m - 1u) {
-                        const int sl = __ffs(m) - 1;
-                        const float a1 = __shfl_sync(FULL, g, sl), phi = __shfl_sync(FULL, rec_c, sl),
-                                    pM = __shfl_sync(FULL, rec_s, sl), cM = __shfl_sync(FULL, cd, sl),
-                                    dw = __shfl_sync(FULL, dw0, sl);
-                        const int ll = __shfl_sync(FULL, l, sl);
-                        const float th = phi + (a1 * fn) + ((dw * (float)(ll * nn)) / (float)(2 * NS));
-                        const float am = pM + (fr * (cM - pM));
-                        tile[lane * BT_STRIDE + sl] = 2.0f * am * dev_cosf(th);
-                    }
-                }
-                __syncwarp();
-                // phase B: lane = sample; the tile's groups in order, each added to the running sum of the frame that owns it
-                // (list order = the reference's summation order); the sum moves to the next frame's row where the owner changes
-                {
-                    const float4* row = reinterpret_cast<const float4*>(tile + lane * BT_STRIDE);
-                    float* op = &ws.out[(fq0 & 1u) | ((fq1 & 1u) << 1) | ((fq2 & 1u) << 2)][32 * ch + lane];
-                    float a = *op;
-#pragma unroll
-                    for (int gi = 0; gi < 8; ++gi) {
-                        if (gi < ng) {
-                            if (gi > 0 && ((fchg >> (4 * gi)) & 1u)) {
-                                *op = a;
-                                op = &ws.out[((fq0 >> (4 * gi)) & 1u) | (((fq1 >> (4 * gi)) & 1u) << 1) |
-                                             (((fq2 >> (4 * gi)) & 1u) << 2)][32 * ch + lane];
-                                a = *op;
-                            }
-                            const float4 v = row[gi];
-                            a += v.x;
-                            a += v.y;
-                            a += v.z;
-                            a += v.w;
-                        }
-                    }
-                    *op = a;
-                }
-                __syncwarp();
+        for (int st = 16; st; st >>= 1) {
+            if ((int)(__shfl_sync(FULL, win, j + st - 1) & 0xffffu) <= p) {
+                j += st;
             }
         }
-        if (A.counters && lane == 0) {
-            int slots = 0;
+        const unsigned wj = __shfl_sync(FULL, win, j);
+        const int end_j = (int)(wj & 0xffffu), cnt_j = (int)(wj >> 16);
+        const int at = p - (end_j - ((cnt_j + 3) & ~3));   // position in frame j's list
+        const bool used = at < cnt_j;
+        float g = 0.f, c = 0.f, s = 0.f, cd = 0.f, sd = 0.f, dw0 = 0.f;
+        int kind = 0, l = 0;
+        if (used) {
+            const uint32_t* d = frame_desc(v0 + j);
+            const unsigned id = reinterpret_cast<const unsigned char*>(d + D_KIND)[at];
+            kind = (int)(id & 3u);
+            l = (int)(id >> 2);
+            g = __uint_as_float(d[D_G + at]);
+            c = __uint_as_float(d[D_C + at]);
+            s = __uint_as_float(d[D_S + at]);
+            cd = __uint_as_float(d[D_CD + at]);
+            sd = __uint_as_float(d[D_SD + at]);
+            dw0 = __uint_as_float(d[D_DW0]);
+        }
+        const bool k2lane = (kind == 2);
+        const unsigned k2mask = __ballot_sync(FULL, k2lane);
+        n_k2 += __popc(k2mask);
+        const float* Wb = vwin + ((kind == 0) ? WIN_PREV : 0);
+        const float gg = k2lane ? 0.0f : g;   // interpolated slots are written by whoever renders them
+        const float rec_c = c, rec_s = s;     // (the recurrence below rotates c and s on every lane)
+        // phase B's map of the pass: bit 4g of fchg = the frame changes at four-slot group g; ng groups hold slots; last_open =
+        // the frame of the last group has slots beyond this pass.  Every frame but the last one ends inside the pass: all its
+        // slots are in registers by now, so its samples may overwrite its slot records
+        const int j_up = __shfl_up_sync(FULL, j, 4);
+        const unsigned fchg = __ballot_sync(FULL, (lane & 3) == 0 && j != j_up);
+        const int ng = min(8, (total - pos) >> 2);
+        const bool last_open = ((__ballot_sync(FULL, end_j > pos + 32) >> (4 * (ng - 1))) & 1u) != 0u;
+        pos += 32;
+#pragma unroll 1
+        for (int ch = 0; ch < 5; ++ch) {
+            // phase A: 32 oscillator steps, sixteen per loop body (the body stays in the L0 instruction cache)
+            const float4* W4 = reinterpret_cast<const float4*>(Wb) + 8 * ch;
+            float* tp = tile + lane;
+#pragma unroll 1
+            for (int h = 0; h < 32 / BANK_STEPS; ++h) {
 #pragma unroll
-            for (int q = 0; q < BG; ++q) {
-                slots += cnt[q];
+                for (int n4 = 0; n4 < BANK_STEPS / 4; ++n4) {
+                    const float4 w4 = W4[(BANK_STEPS / 4) * h + n4];
+                    const float wv[4] = {w4.x, w4.y, w4.z, w4.w};
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) {
+                        if (!k2lane) {
+                            tp[(4 * n4 + i) * BT_STRIDE] = (gg * wv[i]) * c;   // row n = BANK_STEPS h + 4 n4 + i
+                        }
+                        const float cn = (c * cd) - (s * sd);
+                        const float sn = (s * cd) + (c * sd);
+                        c = cn;
+                        s = sn;
+                    }
+                }
+                tp += BANK_STEPS * BT_STRIDE;
             }
-            atomicAdd(&A.counters[0], (unsigned long long)slots);
+            // phase-interpolated harmonics of this pass: lane = sample (mbelib.c:953-968); the slot's lane holds its record
+            if (k2mask) {
+                const int n = 32 * ch + lane;
+                const float fn = (float)n, fr = nfrac[n];
+                const int nn = n * n;
+                for (unsigned m = k2mask; m; m &= m - 1u) {
+                    const int sl = __ffs(m) - 1;
+                    const float a1 = __shfl_sync(FULL, g, sl), phi = __shfl_sync(FULL, rec_c, sl),
+                                pM = __shfl_sync(FULL, rec_s, sl), cM = __shfl_sync(FULL, cd, sl),
+                                dw = __shfl_sync(FULL, dw0, sl);
+                    const int ll = __shfl_sync(FULL, l, sl);
+                    const float th = phi + (a1 * fn) + ((dw * (float)(ll * nn)) / (float)(2 * NS));
+                    const float am = pM + (fr * (cM - pM));
+                    tile[lane * BT_STRIDE + sl] = 2.0f * am * dev_cosf(th);
+                }
+            }
+            __syncwarp();
+            // phase B: lane = sample; the tile's groups in order, each added to the running sum of the frame that owns it
+            // (list order = the reference's summation order).  Every sum starts from 0 (pad slots add +0, which is exactly
+            // neutral); where the frame changes, the finished frame's samples go straight to its descriptor
+            {
+                const float4* row = reinterpret_cast<const float4*>(tile + lane * BT_STRIDE);
+                float* cr = ws.carry + 32 * ch + lane;
+                float a = *cr;
+#pragma unroll
+                for (int gi = 0; gi < 8; ++gi) {
+                    if (gi < ng) {
+                        if (gi > 0 && ((fchg >> (4 * gi)) & 1u)) {
+                            frame_desc(v0 + __shfl_sync(FULL, j, 4 * gi - 4))[D_VOICED + 32 * ch + lane] = __float_as_uint(a);
+                            a = 0.0f;
+                        }
+                        const float4 v = row[gi];
+                        a += v.x;
+                        a += v.y;
+                        a += v.z;
+                        a += v.w;
+                    }
+                }
+                if (!last_open) {
+                    frame_desc(v0 + __shfl_sync(FULL, j, 4 * ng - 4))[D_VOICED + 32 * ch + lane] = __float_as_uint(a);
+                    a = 0.0f;
+                }
+                *cr = a;
+            }
+            __syncwarp();
+        }
+    }
+    if (A.counters) {
+        n_slots = __reduce_add_sync(FULL, (unsigned)n_slots);
+        if (lane == 0) {
+            atomicAdd(&A.counters[0], (unsigned long long)n_slots);
             atomicAdd(&A.counters[1], (unsigned long long)n_k2);
-            atomicAdd(&A.counters[2], (unsigned long long)__popc(go_mask));
-        }
-        // the frames' voiced samples replace their (now dead) slot records
-#pragma unroll
-        for (int q = 0; q < BG; ++q) {
-            if ((go_mask >> q) & 1u) {
-#pragma unroll
-                for (int c = 0; c < 5; ++c) {
-                    d0[(size_t)q * DESC_WORDS + D_VOICED + 32 * c + lane] = __float_as_uint(ws.out[q][32 * c + lane]);
-                }
-            }
+            atomicAdd(&A.counters[2], (unsigned long long)n_go);
+            atomicAdd(&A.counters[3], (unsigned long long)n_pass);
         }
     }
 }
