@@ -198,7 +198,8 @@ MBE_B200_API int mbe_b200_process_frames_packed(mbe_b200_ctx* ctx, int codec, in
  *             completed by mbe_b200_wait (as submit_frames; the slot list must stay valid until then too).
  * Rejection: an element whose slot is outside [0, max_streams), or repeats a slot an earlier element of the same list
  * names, is rejected - all its frames read status MBE_STATUS_INVALID_ARGUMENT (-1) with every other result field zero,
- * zero PCM / float PCM / bits, and no stream state is touched.  Every other element decodes normally, so the first
+ * zero PCM / float PCM / bits, and no stream state is touched (the indexed parameter-bit calls, whose results are
+ * IN/OUT, echo the caller's result instead: mbe_b200_process_data_indexed).  Every other element decodes normally, so the first
  * occurrence of a repeated slot wins.  The check covers the whole list, on the device (_dev) as on the host calls.
  * The state calls below validate on the host instead: an out-of-range or repeated slot fails the whole call with
  * MBE_B200_E_ARG and nothing is touched.  n == 0 or n_frames == 0 returns 0 and launches nothing.
@@ -251,6 +252,35 @@ MBE_B200_API int mbe_b200_process_data_dev(mbe_b200_ctx* ctx, int codec, int fir
                                            float* d_pcmf, void* cuda_stream);
 MBE_B200_API int mbe_b200_process_data(mbe_b200_ctx* ctx, int codec, int first_stream, int n_streams, int n_frames,
                                        const uint8_t* bits, mbe_b200_result* results_inout, int16_t* pcm, float* pcmf);
+/* Indexed parameter-bit batches: process_data for any set of stream slots, the indexed calls above applied to
+ * mbe_process<Codec>Data.  For a server whose frames arrive with the FEC already removed (P25 DFSI / ISSI carry IMBE as 88
+ * information bits in 11 bytes), or that runs decode_frames itself before synthesis.
+ *   - Element i is stream slot slots[i]: bits / results_inout / pcm / pcmf are laid out [i][frame][...] exactly like
+ *     stream i of process_data, and every element consumes n_frames frames with the process_data rules above
+ *     (results_inout IN/OUT, NULL = no decode context; IMBE 7100 takes the IMBE 4400 layout).
+ *   - packed = 0: one byte per bit, as process_data; a byte other than 0 / 1 gives MBE_STATUS_INVALID_BITS (-2).
+ *   - packed = 1: mbe_b200_packed_param_bytes(codec) = 11 / 11 / 7 / 7 bytes per frame, parameter bit k is bit
+ *     7 - (k & 7) of byte k >> 3 (MSB first, as the packed channel frames); the pad bits of the last byte are ignored and
+ *     MBE_STATUS_INVALID_BITS cannot occur.  A feed with another bit order is repacked by the caller.
+ *   - Rejection: the rules of the indexed frame calls (out-of-range slot, or a repeat of a slot an earlier element names;
+ *     the first occurrence wins; the whole list is checked, on the device for _dev).  A rejected element follows the rule
+ *     of every negative status on this path, NOT the frame calls' zeroed result: each of its results is the caller's
+ *     input element with only .status replaced by MBE_STATUS_INVALID_ARGUMENT (-1) (nothing is written when results_inout
+ *     is NULL); its PCM and float PCM are zero and no stream state is touched.
+ *   - n == 0 or n_frames == 0 returns 0 and launches nothing.  _dev / host / submit (completed by mbe_b200_wait) as for
+ *     process_indexed[_dev] / submit_indexed: host calls refuse while a submission is pending, one submission may be
+ *     pending per context, and concurrent calls whose slot sets overlap are the caller's error.
+ * A contiguous caller that wants packed input passes the identity list first_stream .. first_stream + n - 1. */
+MBE_B200_API int mbe_b200_packed_param_bytes(int codec);
+MBE_B200_API int mbe_b200_process_data_indexed_dev(mbe_b200_ctx* ctx, int codec, int packed, const int32_t* d_slots, int n,
+                                                   int n_frames, const uint8_t* d_bits, mbe_b200_result* d_results_inout,
+                                                   int16_t* d_pcm, float* d_pcmf, void* cuda_stream);
+MBE_B200_API int mbe_b200_process_data_indexed(mbe_b200_ctx* ctx, int codec, int packed, const int32_t* slots, int n,
+                                               int n_frames, const uint8_t* bits, mbe_b200_result* results_inout,
+                                               int16_t* pcm, float* pcmf);
+MBE_B200_API int mbe_b200_submit_data_indexed(mbe_b200_ctx* ctx, int codec, int packed, const int32_t* slots, int n,
+                                              int n_frames, const uint8_t* bits, mbe_b200_result* results_inout,
+                                              int16_t* pcm, float* pcmf);
 
 /* ---- single stages on caller-held parameter sets -------------------------------------------------------
  * Batched forms of the reference's per-stage helpers, one element = one call, host `mbe_parms` blobs updated in place:
@@ -323,6 +353,12 @@ MBE_B200_API int mbe_b200_pool_process_frames(mbe_b200_pool* pool, int codec, in
 MBE_B200_API int mbe_b200_pool_process_indexed(mbe_b200_pool* pool, int codec, int input, const int32_t* slots, int n,
                                                int n_frames, const uint8_t* in, int16_t* pcm, float* pcmf,
                                                mbe_b200_result* results, uint8_t* bits);
+/* mbe_b200_process_data_indexed over global pool slots, gathered and scattered the same way (the IN/OUT results travel
+ * both ways); an out-of-range element gets the rejected-element result of the context call: the caller's result with
+ * status -1, zero PCM. */
+MBE_B200_API int mbe_b200_pool_process_data_indexed(mbe_b200_pool* pool, int codec, int packed, const int32_t* slots, int n,
+                                                    int n_frames, const uint8_t* bits, mbe_b200_result* results_inout,
+                                                    int16_t* pcm, float* pcmf);
 MBE_B200_API int mbe_b200_pool_init_streams_indexed(mbe_b200_pool* pool, const int32_t* slots, int n, const uint32_t* seeds);
 MBE_B200_API int mbe_b200_pool_set_channel_map(mbe_b200_pool* pool, int codec, const uint16_t* map, int n_bits);
 MBE_B200_API int mbe_b200_pool_process_frames_packed(mbe_b200_pool* pool, int codec, int first_stream, int n_streams,

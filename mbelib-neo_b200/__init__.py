@@ -45,7 +45,8 @@ _EXPORTS = ["mbe_b200_create", "mbe_b200_destroy", "mbe_b200_last_error", "mbe_b
             "mbe_b200_single_frame", "mbe_b200_process_indexed_dev", "mbe_b200_process_indexed", "mbe_b200_submit_indexed",
             "mbe_b200_init_streams_indexed", "mbe_b200_export_state_indexed", "mbe_b200_import_state_indexed",
             "mbe_b200_export_rng_indexed", "mbe_b200_import_rng_indexed", "mbe_b200_pool_process_indexed",
-            "mbe_b200_pool_init_streams_indexed"]
+            "mbe_b200_pool_init_streams_indexed", "mbe_b200_packed_param_bytes", "mbe_b200_process_data_indexed_dev",
+            "mbe_b200_process_data_indexed", "mbe_b200_submit_data_indexed", "mbe_b200_pool_process_data_indexed"]
 
 # `input` of the indexed calls (MBE_B200_INPUT_* of include/mbe_b200.h)
 INPUT_HARD, INPUT_SOFT, INPUT_PACKED = 0, 1, 2
@@ -136,6 +137,10 @@ def load_library():
         lib.mbe_b200_process_indexed_dev.argtypes = [vp, ci, ci, vp, ci, ci, vp, vp, vp, vp, vp, vp]
         for n in ("process_indexed", "submit_indexed", "pool_process_indexed"):
             getattr(lib, "mbe_b200_" + n).argtypes = [vp, ci, ci, vp, ci, ci, vp, vp, vp, vp, vp]
+        lib.mbe_b200_packed_param_bytes.argtypes = [ci]
+        lib.mbe_b200_process_data_indexed_dev.argtypes = [vp, ci, ci, vp, ci, ci, vp, vp, vp, vp, vp]
+        for n in ("process_data_indexed", "submit_data_indexed", "pool_process_data_indexed"):
+            getattr(lib, "mbe_b200_" + n).argtypes = [vp, ci, ci, vp, ci, ci, vp, vp, vp, vp]
         for n in ("init_streams_indexed", "export_state_indexed", "import_state_indexed", "export_rng_indexed",
                   "import_rng_indexed", "pool_init_streams_indexed"):
             getattr(lib, "mbe_b200_" + n).argtypes = [vp, vp, ci, vp]
@@ -145,6 +150,30 @@ def load_library():
 
 def packed_frame_bytes(codec):
     return (FRAME_BITS[codec] + 7) // 8
+
+
+def packed_param_bytes(codec):
+    """bytes of one packed parameter frame: 11 / 11 / 7 / 7"""
+    return (PARAM_BITS[codec] + 7) // 8
+
+
+def pack_params(codec, bits):
+    """uint8 [..., param_bits] of 0/1 -> uint8 [..., packed_param_bytes(codec)], MSB first, the pad bits of the last byte
+    zero (host-side data preparation for the packed parameter-bit calls)."""
+    bits = np.ascontiguousarray(bits, dtype=np.uint8)
+    assert bits.shape[-1] == PARAM_BITS[codec]
+    return np.packbits(bits, axis=-1, bitorder="big")
+
+
+def _data_indexed_args(codec, slots, bits, results, packed):
+    """(slots, bits, IN/OUT results copy or None) of an indexed parameter-bit call"""
+    slots = _slots(slots)
+    bits = np.ascontiguousarray(bits, dtype=np.uint8)
+    n, F = bits.shape[0], bits.shape[1]
+    assert n == slots.size and bits.shape[2] == (packed_param_bytes(codec) if packed else PARAM_BITS[codec])
+    if results is not None:
+        results = np.ascontiguousarray(results, dtype=RESULT_DTYPE).reshape(n, F).copy()
+    return slots, bits, results
 
 
 def pack_frames(codec, frames):
@@ -297,6 +326,17 @@ class Pool:
                                                            _p(out["bits"])), "pool_process_indexed")
         return out
 
+    def process_data_indexed(self, codec, slots, bits, results=None, packed=False, want_float=False):
+        """mbe_b200_pool_process_data_indexed: element i of `bits` ([n][F][88|49], or [n][F][11|7] packed) and of
+        `results` (IN/OUT decode context, None = none) is global slot slots[i].  Returns the dict process_data returns."""
+        slots, bits, results = _data_indexed_args(codec, slots, bits, results, packed)
+        n, F = bits.shape[0], bits.shape[1]
+        pcm = np.zeros((n, F, SAMPLES), np.int16)
+        pcmf = np.zeros((n, F, SAMPLES), np.float32) if want_float else None
+        self._check(self.lib.mbe_b200_pool_process_data_indexed(self.h, codec, int(bool(packed)), _p(slots), n, F, _p(bits),
+                                                                _p(results), _p(pcm), _p(pcmf)), "pool_process_data_indexed")
+        return dict(pcm=pcm, pcmf=pcmf, results=results)
+
 
 class Decoder:
     """One context = one GPU + a pool of `max_streams` device-resident voice-stream states."""
@@ -418,6 +458,36 @@ class Decoder:
                                                           _p(d_pcm or None), _p(d_pcmf or None), _p(d_results or None),
                                                           _p(d_bits or None), _p(cuda_stream or None)),
                     "process_indexed_dev")
+
+    # ---- indexed parameter-bit batches (mbe_process<Codec>Data): element i of bits / results / outputs is slot slots[i] ----
+    def process_data_indexed(self, codec, slots, bits, results=None, packed=False, want_float=False):
+        """bits: uint8 [n][F][88|49] one byte per bit, or [n][F][packed_param_bytes(codec)] with packed=True (see
+        pack_params); results: the IN/OUT decode context [n][F] (None = none).  Returns the dict process_data returns."""
+        slots, bits, results = _data_indexed_args(codec, slots, bits, results, packed)
+        n, F = bits.shape[0], bits.shape[1]
+        pcm = np.zeros((n, F, SAMPLES), np.int16)
+        pcmf = np.zeros((n, F, SAMPLES), np.float32) if want_float else None
+        self._check(self.lib.mbe_b200_process_data_indexed(self.h, codec, int(bool(packed)), _p(slots), n, F, _p(bits),
+                                                           _p(results), _p(pcm), _p(pcmf)), "process_data_indexed")
+        return dict(pcm=pcm, pcmf=pcmf, results=results)
+
+    def submit_data_indexed(self, codec, slots, bits, out, packed=False):
+        """Asynchronous process_data_indexed: `slots`, `bits` and the arrays of `out` (dict with pcm / pcmf / results, any
+        may be missing; results holds the decode context in and the results out) must stay alive and untouched until
+        wait()."""
+        assert slots.dtype == np.int32 and slots.flags["C_CONTIGUOUS"]
+        n, F = bits.shape[0], bits.shape[1]
+        self._check(self.lib.mbe_b200_submit_data_indexed(self.h, codec, int(bool(packed)), _p(slots), n, F, _p(bits),
+                                                          _p(out.get("results")), _p(out.get("pcm")), _p(out.get("pcmf"))),
+                    "submit_data_indexed")
+
+    def process_data_indexed_dev(self, codec, packed, d_slots, n, n_frames, d_bits, d_results_inout, d_pcm, d_pcmf=0,
+                                 cuda_stream=0):
+        """All pointers are raw device addresses (ints, 0 = NULL), d_slots int32 [n]; asynchronous on `cuda_stream`."""
+        self._check(self.lib.mbe_b200_process_data_indexed_dev(self.h, codec, int(bool(packed)), _p(d_slots), n, n_frames,
+                                                               _p(d_bits), _p(d_results_inout or None), _p(d_pcm or None),
+                                                               _p(d_pcmf or None), _p(cuda_stream or None)),
+                    "process_data_indexed_dev")
 
     # ---- hot path, host buffers ----
     def process_frames(self, codec, frames, soft=False, first_stream=0, want_float=False, want_bits=True,

@@ -560,8 +560,9 @@ struct StreamShape {
     static constexpr int MINB = SMALL ? P_MINB : MIN_BLOCKS_PER_SM;
 };
 
-// INDEXED: channel frames of an indexed call (LaunchArgs::slots); a separate image, so that the contiguous launches keep
-// the register allocation they have without the slot list and the claim check
+// INDEXED: an indexed call (LaunchArgs::slots); a separate image, so that the contiguous launches keep the register
+// allocation they have without the slot list and the claim check.  Indexed MODE_DATA launches also take packed parameter
+// bits (LaunchArgs::packed_bytes != 0), a warp-uniform run-time choice rather than another image.
 template <int CODEC, int SOFT, int MODE, bool SPLIT, bool INDEXED = false>
 __global__ void __launch_bounds__(StreamShape<SOFT, SPLIT>::WARPS * 32, StreamShape<SOFT, SPLIT>::MINB)
 mbe_stream_kernel(const LaunchArgs A) {
@@ -585,7 +586,8 @@ mbe_stream_kernel(const LaunchArgs A) {
     constexpr int fbits = (CODEC == MBE_B200_IMBE7200X4400) ? 184 : (CODEC == MBE_B200_IMBE7100X4400 ? 168 : 96);
     constexpr int pbits = AMBE ? 49 : 88;
     constexpr bool PACKED = (SOFT == 2);
-    const size_t fstride = (MODE == MODE_DATA) ? (size_t)pbits
+    const bool data_packed = INDEXED && MODE == MODE_DATA && A.packed_bytes != 0;
+    const size_t fstride = (MODE == MODE_DATA) ? (data_packed ? (size_t)A.packed_bytes : (size_t)pbits)
                                                : (PACKED ? (size_t)A.packed_bytes : (size_t)fbits * (SOFT == 1 ? 2u : 1u));
 
     // an element of an indexed call whose slot is out of range or claimed by an earlier element is rejected: it touches no
@@ -664,7 +666,8 @@ mbe_stream_kernel(const LaunchArgs A) {
                     const int i = 32 * w + lane;
                     unsigned b = 0;
                     if (i < pbits) {
-                        const unsigned v = fr[i];
+                        // packed: bit i is bit 7 - (i & 7) of byte i >> 3 (MSB first), so it can only be 0 or 1
+                        const unsigned v = data_packed ? (fr[i >> 3] >> (7 - (i & 7))) & 1u : fr[i];
                         bad |= (v > 1u);
                         b = v & 1u;
                     }
@@ -693,6 +696,10 @@ mbe_stream_kernel(const LaunchArgs A) {
                 fc.c4 = fc.c4v ? c4 : 0;
                 fc.total = total;
             }
+        } else if (INDEXED && MODE == MODE_DATA && live && A.results) {
+            // a rejected element echoes the caller's decode context with only .status replaced, the rule of every
+            // negative status on this path (the location is the caller's I/O element, not stream state)
+            rout = A.results[idx];
         }
         // ECC front-end | parameter decode: soft-decision kernels re-join here, because their front-end runs a data-dependent
         // number of coset walks per stream and the block would otherwise walk the parameter decode out of step (instruction
@@ -1677,9 +1684,9 @@ template <bool SPLIT, bool INDEXED>
 static StreamKernelFn pick_stream_kernel_t(int codec, int soft, int mode) {
     if (mode == MODE_DATA) {
         switch (codec) {
-            case MBE_B200_AMBE3600X2400: return mbe_stream_kernel<MBE_B200_AMBE3600X2400, 0, MODE_DATA, SPLIT>;
-            case MBE_B200_AMBE3600X2450: return mbe_stream_kernel<MBE_B200_AMBE3600X2450, 0, MODE_DATA, SPLIT>;
-            default: return mbe_stream_kernel<MBE_B200_IMBE7200X4400, 0, MODE_DATA, SPLIT>;
+            case MBE_B200_AMBE3600X2400: return mbe_stream_kernel<MBE_B200_AMBE3600X2400, 0, MODE_DATA, SPLIT, INDEXED>;
+            case MBE_B200_AMBE3600X2450: return mbe_stream_kernel<MBE_B200_AMBE3600X2450, 0, MODE_DATA, SPLIT, INDEXED>;
+            default: return mbe_stream_kernel<MBE_B200_IMBE7200X4400, 0, MODE_DATA, SPLIT, INDEXED>;
         }
     }
     if (soft == 2) {  // packed hard bits
@@ -1702,7 +1709,6 @@ static StreamKernelFn pick_stream_kernel_t(int codec, int soft, int mode) {
     }
 }
 
-// (indexed: channel frames only - parameter-bit input has no indexed entry point)
 static StreamKernelFn pick_stream_kernel(int codec, int soft, int mode, bool split = false, bool indexed = false) {
     if (indexed) {
         return split ? pick_stream_kernel_t<true, true>(codec, soft, mode) : pick_stream_kernel_t<false, true>(codec, soft, mode);
@@ -1872,7 +1878,7 @@ int mbe_b200_create(mbe_b200_ctx** out, int device_ordinal, int max_streams) {
     for (int codec = 0; codec < 4; ++codec) {
         for (int soft = 0; soft < 3; ++soft) {
             for (int mode = 0; mode < (soft == 2 ? 1 : 2); ++mode) {
-                for (int indexed = 0; indexed < (mode == MODE_FRAMES ? 2 : 1); ++indexed) {
+                for (int indexed = 0; indexed < 2; ++indexed) {
                     CUC(cudaFuncSetAttribute(pick_stream_kernel(codec, soft, mode, false, indexed),
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)stream_kernel_smem()));
                     CUC(cudaFuncSetAttribute(pick_stream_kernel(codec, soft, mode, true, indexed),
@@ -2207,7 +2213,9 @@ static size_t split_cap_streams(int n_frames, int soft) {
 static int launch_stream_kernel(mbe_b200_ctx* ctx, const LaunchArgs& a_in, cudaStream_t st) {
     LaunchArgs a = a_in;
     a.pcmf_scale = ctx->normalized_float ? (7.0f / 32768.0f) : 1.0f;
-    a.packed_bytes = (a.mode == MODE_FRAMES && a.soft == 2) ? (ctx->chan_bits[a.codec] + 7) / 8 : 0;
+    a.packed_bytes = a.soft != 2                ? 0
+                     : a.mode == MODE_FRAMES    ? (ctx->chan_bits[a.codec] + 7) / 8
+                                                : mbe_b200_packed_param_bytes(a.codec);   // packed parameter bits
     if (a.mode == MODE_SYNTH) {
         const int blocks = (a.n_streams + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
         mbe_synth_kernel<<<blocks, WARPS_PER_BLOCK * 32, stream_kernel_smem(), st>>>(a);
@@ -2395,11 +2403,12 @@ int mbe_b200_kernel_timing(mbe_b200_ctx* ctx, double ms[3], long long launches[3
 
 // input kinds of the frame entry points: 0 = one byte per hard bit, 1 = mbe_soft_bit pairs, 2 = hard bits packed
 // (MBE_B200_INPUT_*).  d_slots != nullptr: an indexed launch, elements slot_base .. slot_base + n_streams - 1 of the call's
-// device slot list, claimed under `epoch` (first_stream is ignored)
+// device slot list, claimed under `epoch` (first_stream is ignored).  mode MODE_DATA: parameter bits (kind 0 one byte per
+// bit, 2 packed, indexed launches only), d_results is the IN/OUT decode context and d_bits is not used.
 static int frames_dev_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_stream, int n_streams, int n_frames,
                            const uint8_t* d_frames, int16_t* d_pcm, float* d_pcmf, mbe_b200_result* d_results,
                            uint8_t* d_bits, void* cuda_stream, const int32_t* d_slots = nullptr, int slot_base = 0,
-                           unsigned epoch = 0);
+                           unsigned epoch = 0, int mode = MODE_FRAMES);
 
 int mbe_b200_process_frames_dev(mbe_b200_ctx* ctx, int codec, int soft, int first_stream, int n_streams, int n_frames,
                                 const uint8_t* d_frames, int16_t* d_pcm, float* d_pcmf, mbe_b200_result* d_results,
@@ -2471,16 +2480,26 @@ int mbe_b200_packed_frame_bytes(int codec) {
     return (fb + 7) / 8;
 }
 
+int mbe_b200_packed_param_bytes(int codec) {
+    int fb, pb;
+    if (mbe_b200_geometry(codec, &fb, &pb) != 0) {
+        return MBE_B200_E_ARG;
+    }
+    return (pb + 7) / 8;
+}
+
 static int frames_dev_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_stream, int n_streams, int n_frames,
                            const uint8_t* d_frames, int16_t* d_pcm, float* d_pcmf, mbe_b200_result* d_results,
-                           uint8_t* d_bits, void* cuda_stream, const int32_t* d_slots, int slot_base, unsigned epoch) {
+                           uint8_t* d_bits, void* cuda_stream, const int32_t* d_slots, int slot_base, unsigned epoch,
+                           int mode) {
     const int soft = kind;
     int rc = d_slots ? (ctx ? 0 : MBE_B200_E_ARG) : check_range(ctx, first_stream, n_streams);
     if (rc < 0) {
         return rc;
     }
     if (codec < 0 || codec > 3 || n_frames < 0 || !d_frames) {
-        return fail(ctx, MBE_B200_E_ARG, "process_frames: bad argument", cudaSuccess);
+        return fail(ctx, MBE_B200_E_ARG, mode == MODE_DATA ? "process_data: bad argument" : "process_frames: bad argument",
+                    cudaSuccess);
     }
     if (n_streams == 0 || n_frames == 0) {
         return 0;
@@ -2490,7 +2509,7 @@ static int frames_dev_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_str
     memset(&a, 0, sizeof(a));
     a.codec = codec;
     a.soft = soft;
-    a.mode = MODE_FRAMES;
+    a.mode = mode;
     a.first_stream = first_stream;
     a.n_streams = n_streams;
     a.n_frames = n_frames;
@@ -2498,7 +2517,7 @@ static int frames_dev_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_str
     a.pcm = d_pcm;
     a.pcmf = d_pcmf;
     a.results = d_results;
-    a.bits = d_bits;
+    a.bits = mode == MODE_FRAMES ? d_bits : nullptr;
     a.state = ctx->d_state;
     a.tab = ctx->d_tab;
     a.dbg = ctx->d_dbg;
@@ -2513,31 +2532,8 @@ static int frames_dev_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_str
 int mbe_b200_process_data_dev(mbe_b200_ctx* ctx, int codec, int first_stream, int n_streams, int n_frames,
                               const uint8_t* d_bits, mbe_b200_result* d_results_inout, int16_t* d_pcm, float* d_pcmf,
                               void* cuda_stream) {
-    int rc = check_range(ctx, first_stream, n_streams);
-    if (rc < 0) {
-        return rc;
-    }
-    if (codec < 0 || codec > 3 || n_frames < 0 || !d_bits) {
-        return fail(ctx, MBE_B200_E_ARG, "process_data: bad argument", cudaSuccess);
-    }
-    if (n_streams == 0 || n_frames == 0) {
-        return 0;
-    }
-    CU(cudaSetDevice(ctx->device));
-    LaunchArgs a;
-    memset(&a, 0, sizeof(a));
-    a.codec = codec;
-    a.mode = MODE_DATA;
-    a.first_stream = first_stream;
-    a.n_streams = n_streams;
-    a.n_frames = n_frames;
-    a.frames = d_bits;
-    a.pcm = d_pcm;
-    a.pcmf = d_pcmf;
-    a.results = d_results_inout;
-    a.state = ctx->d_state;
-    a.tab = ctx->d_tab;
-    return launch_stream_kernel(ctx, a, cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream);
+    return frames_dev_impl(ctx, codec, 0, first_stream, n_streams, n_frames, d_bits, d_pcm, d_pcmf, d_results_inout, nullptr,
+                           cuda_stream, nullptr, 0, 0, MODE_DATA);
 }
 
 // ---- one stream, one frame, caller-owned state: what the single-stream shim needs, as ONE upload, three kernels, ONE
@@ -2773,7 +2769,7 @@ int mbe_b200_pipeline_plan(int n_streams, int* sizes, int cap) {
 
 static int frames_host_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_stream, int n_streams, int n_frames,
                             const uint8_t* frames, int16_t* pcm, float* pcmf, mbe_b200_result* results, uint8_t* bits,
-                            bool wait = true, const int32_t* slots = nullptr);
+                            bool wait = true, const int32_t* slots = nullptr, int mode = MODE_FRAMES);
 
 // A new claim epoch for an indexed call and the claim launch over its whole device slot list on `st`.  After 2^32 - 1
 // calls the epochs start over from a cleared claim table (nothing of the device may still read it).
@@ -2806,10 +2802,12 @@ static int check_indexed(mbe_b200_ctx* ctx, const char* what, int codec, int inp
     return 0;
 }
 
-int mbe_b200_process_indexed_dev(mbe_b200_ctx* ctx, int codec, int input, const int32_t* d_slots, int n, int n_frames,
-                                 const uint8_t* d_in, int16_t* d_pcm, float* d_pcmf, mbe_b200_result* d_results,
-                                 uint8_t* d_bits, void* cuda_stream) {
-    int rc = check_indexed(ctx, "process_indexed_dev", codec, input, d_slots, n, n_frames, d_in);
+// the indexed calls of both modes: MODE_FRAMES (channel frames, `input` MBE_B200_INPUT_*) and MODE_DATA (parameter bits,
+// `input` HARD = one byte per bit or PACKED, `results` the IN/OUT decode context, no `bits` output)
+static int indexed_dev_impl(mbe_b200_ctx* ctx, const char* what, int mode, int codec, int input, const int32_t* d_slots, int n,
+                            int n_frames, const uint8_t* d_in, int16_t* d_pcm, float* d_pcmf, mbe_b200_result* d_results,
+                            uint8_t* d_bits, void* cuda_stream) {
+    int rc = check_indexed(ctx, what, codec, input, d_slots, n, n_frames, d_in);
     if (rc < 0 || n == 0 || n_frames == 0) {
         return rc;
     }
@@ -2819,33 +2817,70 @@ int mbe_b200_process_indexed_dev(mbe_b200_ctx* ctx, int codec, int input, const 
     if ((rc = claim_slots(ctx, d_slots, n, st, &epoch)) < 0) {
         return rc;
     }
-    return frames_dev_impl(ctx, codec, input, 0, n, n_frames, d_in, d_pcm, d_pcmf, d_results, d_bits, st, d_slots, 0, epoch);
+    return frames_dev_impl(ctx, codec, input, 0, n, n_frames, d_in, d_pcm, d_pcmf, d_results, d_bits, st, d_slots, 0, epoch,
+                           mode);
 }
 
-int mbe_b200_process_indexed(mbe_b200_ctx* ctx, int codec, int input, const int32_t* slots, int n, int n_frames,
-                             const uint8_t* in, int16_t* pcm, float* pcmf, mbe_b200_result* results, uint8_t* bits) {
-    const int rc = check_indexed(ctx, "process_indexed", codec, input, slots, n, n_frames, in);
-    if (rc < 0) {
-        return rc;
-    }
-    return frames_host_impl(ctx, codec, input, 0, n, n_frames, in, pcm, pcmf, results, bits, true, slots);
-}
-
-int mbe_b200_submit_indexed(mbe_b200_ctx* ctx, int codec, int input, const int32_t* slots, int n, int n_frames,
-                            const uint8_t* in, int16_t* pcm, float* pcmf, mbe_b200_result* results, uint8_t* bits) {
-    int rc = check_indexed(ctx, "submit_indexed", codec, input, slots, n, n_frames, in);
+// wait == false: the asynchronous half (submit_*), completed by mbe_b200_wait
+static int indexed_host_impl(mbe_b200_ctx* ctx, const char* what, int mode, int codec, int input, const int32_t* slots, int n,
+                             int n_frames, const uint8_t* in, int16_t* pcm, float* pcmf, mbe_b200_result* results,
+                             uint8_t* bits, bool wait) {
+    int rc = check_indexed(ctx, what, codec, input, slots, n, n_frames, in);
     if (rc < 0) {
         return rc;
     }
     if (ctx->pending) {
-        return fail(ctx, MBE_B200_E_ARG, "submit_indexed: a submission is still pending (call mbe_b200_wait first)",
-                    cudaSuccess);
+        char msg[128];
+        snprintf(msg, sizeof(msg), "%s: a submission is still pending (call mbe_b200_wait first)", what);
+        return fail(ctx, MBE_B200_E_ARG, msg, cudaSuccess);
     }
-    rc = frames_host_impl(ctx, codec, input, 0, n, n_frames, in, pcm, pcmf, results, bits, false, slots);
-    if (rc == 0) {
+    rc = frames_host_impl(ctx, codec, input, 0, n, n_frames, in, pcm, pcmf, results, bits, wait, slots, mode);
+    if (rc == 0 && !wait) {
         ctx->pending = 1;
     }
     return rc;
+}
+
+int mbe_b200_process_indexed_dev(mbe_b200_ctx* ctx, int codec, int input, const int32_t* d_slots, int n, int n_frames,
+                                 const uint8_t* d_in, int16_t* d_pcm, float* d_pcmf, mbe_b200_result* d_results,
+                                 uint8_t* d_bits, void* cuda_stream) {
+    return indexed_dev_impl(ctx, "process_indexed_dev", MODE_FRAMES, codec, input, d_slots, n, n_frames, d_in, d_pcm, d_pcmf,
+                            d_results, d_bits, cuda_stream);
+}
+
+int mbe_b200_process_indexed(mbe_b200_ctx* ctx, int codec, int input, const int32_t* slots, int n, int n_frames,
+                             const uint8_t* in, int16_t* pcm, float* pcmf, mbe_b200_result* results, uint8_t* bits) {
+    return indexed_host_impl(ctx, "process_indexed", MODE_FRAMES, codec, input, slots, n, n_frames, in, pcm, pcmf, results, bits,
+                             true);
+}
+
+int mbe_b200_submit_indexed(mbe_b200_ctx* ctx, int codec, int input, const int32_t* slots, int n, int n_frames,
+                            const uint8_t* in, int16_t* pcm, float* pcmf, mbe_b200_result* results, uint8_t* bits) {
+    return indexed_host_impl(ctx, "submit_indexed", MODE_FRAMES, codec, input, slots, n, n_frames, in, pcm, pcmf, results, bits,
+                             false);
+}
+
+// parameter-bit input of the indexed data calls: packed 0 = one byte per bit, 1 = eight bits per byte (anything else fails
+// check_indexed)
+static int data_input(int packed) { return packed == 0 ? MBE_B200_INPUT_HARD : packed == 1 ? MBE_B200_INPUT_PACKED : -1; }
+
+int mbe_b200_process_data_indexed_dev(mbe_b200_ctx* ctx, int codec, int packed, const int32_t* d_slots, int n, int n_frames,
+                                      const uint8_t* d_bits, mbe_b200_result* d_results_inout, int16_t* d_pcm, float* d_pcmf,
+                                      void* cuda_stream) {
+    return indexed_dev_impl(ctx, "process_data_indexed_dev", MODE_DATA, codec, data_input(packed), d_slots, n, n_frames, d_bits,
+                            d_pcm, d_pcmf, d_results_inout, nullptr, cuda_stream);
+}
+
+int mbe_b200_process_data_indexed(mbe_b200_ctx* ctx, int codec, int packed, const int32_t* slots, int n, int n_frames,
+                                  const uint8_t* bits, mbe_b200_result* results_inout, int16_t* pcm, float* pcmf) {
+    return indexed_host_impl(ctx, "process_data_indexed", MODE_DATA, codec, data_input(packed), slots, n, n_frames, bits, pcm,
+                             pcmf, results_inout, nullptr, true);
+}
+
+int mbe_b200_submit_data_indexed(mbe_b200_ctx* ctx, int codec, int packed, const int32_t* slots, int n, int n_frames,
+                                 const uint8_t* bits, mbe_b200_result* results_inout, int16_t* pcm, float* pcmf) {
+    return indexed_host_impl(ctx, "submit_data_indexed", MODE_DATA, codec, data_input(packed), slots, n, n_frames, bits, pcm,
+                             pcmf, results_inout, nullptr, false);
 }
 
 int mbe_b200_wait(mbe_b200_ctx* ctx) {
@@ -2885,9 +2920,12 @@ int mbe_b200_process_frames_packed(mbe_b200_ctx* ctx, int codec, int first_strea
     return frames_host_impl(ctx, codec, 2, first_stream, n_streams, n_frames, packed, pcm, pcmf, results, bits);
 }
 
+// The pipelined host call of both modes.  MODE_DATA (indexed parameter-bit calls): `frames` holds parameter bits (kind 0
+// one byte per bit, 2 packed), `results` is IN/OUT - each chunk's decode context goes up on s_in ahead of its kernel - and
+// `bits` is unused.
 static int frames_host_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_stream, int n_streams, int n_frames,
                             const uint8_t* frames, int16_t* pcm, float* pcmf, mbe_b200_result* results, uint8_t* bits,
-                            bool wait, const int32_t* slots) {
+                            bool wait, const int32_t* slots, int mode) {
     int rc = slots ? 0 : check_range(ctx, first_stream, n_streams);   // (indexed: checked by check_indexed)
     if (rc == 0 && ctx->pending) {
         return fail(ctx, MBE_B200_E_ARG, "process_frames: a submission is still pending (call mbe_b200_wait first)", cudaSuccess);
@@ -2905,9 +2943,10 @@ static int frames_host_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_st
     CU(cudaSetDevice(ctx->device));
     int fb, pb;
     mbe_b200_geometry(codec, &fb, &pb);
-    const size_t in_per_frame = (kind == 2) ? (size_t)((ctx->chan_bits[codec] + 7) / 8) : (size_t)fb * (kind == 1 ? 2 : 1);
+    const size_t in_per_frame = (mode == MODE_DATA) ? (size_t)(kind == 2 ? (pb + 7) / 8 : pb)
+                                : (kind == 2) ? (size_t)((ctx->chan_bits[codec] + 7) / 8) : (size_t)fb * (kind == 1 ? 2 : 1);
     const size_t per_frame[4] = {pcm ? NS * sizeof(int16_t) : 0, pcmf ? NS * sizeof(float) : 0,
-                                 results ? sizeof(mbe_b200_result) : 0, bits ? (size_t)pb : 0};
+                                 results ? sizeof(mbe_b200_result) : 0, (bits && mode == MODE_FRAMES) ? (size_t)pb : 0};
     if ((rc = ensure(ctx, &ctx->d_in, &ctx->d_in_cap, nf * in_per_frame)) < 0) {
         return rc;
     }
@@ -2972,6 +3011,10 @@ static int frames_host_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_st
             cudaStream_t sk = ctx->s_k[c % n_k];
             CU(cudaMemcpyAsync((uint8_t*)ctx->d_in + f0 * in_per_frame, frames + f0 * in_per_frame, fn * in_per_frame,
                                cudaMemcpyHostToDevice, ctx->s_in));
+            if (mode == MODE_DATA && results) {
+                CU(cudaMemcpyAsync((mbe_b200_result*)ctx->d_out[2] + f0, results + f0, fn * sizeof(mbe_b200_result),
+                                   cudaMemcpyHostToDevice, ctx->s_in));
+            }
             CU(cudaEventRecord(ctx->ev_in[c], ctx->s_in));
             CU(cudaStreamWaitEvent(sk, ctx->ev_in[c], 0));
             int16_t* const o_pcm = pcm ? (int16_t*)ctx->d_out[0] + f0 * NS : nullptr;
@@ -2980,7 +3023,7 @@ static int frames_host_impl(mbe_b200_ctx* ctx, int codec, int kind, int first_st
             uint8_t* const o_bits = bits ? (uint8_t*)ctx->d_out[3] + f0 * pb : nullptr;
             const uint8_t* const i_fr = (const uint8_t*)ctx->d_in + f0 * in_per_frame;
             const int rk = frames_dev_impl(ctx, codec, kind, first_stream + s0, ns, n_frames, i_fr, o_pcm, o_pcmf, o_res, o_bits, sk,
-                                           slots ? ctx->d_slots : nullptr, s0, epoch);
+                                           slots ? ctx->d_slots : nullptr, s0, epoch, mode);
             if (rk < 0) {
                 return rk;
             }

@@ -265,6 +265,82 @@ static int grow_stage(mbe_b200_pool* p, int shard, size_t bytes) {
 
 static size_t align64(size_t x) { return (x + 63) & ~(size_t)63; }
 
+// One per-element array of an indexed pool call, `bytes` per element (all its frames): `in` arrays are gathered into the
+// shard's staging buffer before the context call, `out` arrays scattered back after it (results_inout is both).
+// host == nullptr: the array is not used and the context call gets nullptr.
+struct IndexedArray {
+    uint8_t* host;
+    size_t bytes;
+    bool in, out;
+};
+
+// The shared body of the indexed pool calls.  A stable partition of the element positions by owning shard: a slot always
+// maps to one shard, so the context's first-occurrence rule holds for the whole list.  An out-of-range element is rejected
+// here as a context rejects it: its output-only arrays are zeroed and the status of each of its `results` frames is set to
+// -1 (a frame call's results are output-only and so read zero otherwise, a data call's IN/OUT results keep the caller's
+// input).  Every shard then gathers its elements in list order into its pinned staging buffer (local slots first), runs
+// call(ctx, local slots, count, local arrays) and scatters the outputs back.
+template <class Call>
+static int pool_indexed(mbe_b200_pool* p, const char* what, const int32_t* slots, int n, size_t n_frames,
+                        mbe_b200_result* results, std::vector<IndexedArray> arr, Call call) {
+    std::vector<std::vector<int>> part(p->ctx.size());
+    for (int i = 0; i < n; ++i) {
+        const int slot = slots[i];
+        if (slot >= 0 && slot < p->max_streams) {
+            part[shard_of(p, slot)].push_back(i);
+            continue;
+        }
+        for (const IndexedArray& a : arr) {
+            if (a.host && !a.in) {
+                memset(a.host + (size_t)i * a.bytes, 0, a.bytes);
+            }
+        }
+        for (size_t f = 0; results && f < n_frames; ++f) {
+            results[(size_t)i * n_frames + f].status = -1;   // MBE_STATUS_INVALID_ARGUMENT
+        }
+    }
+    return for_each_part(p, what, part, [&](int shard, mbe_b200_ctx* c, const std::vector<int>& el) {
+        const size_t m = el.size();
+        std::vector<size_t> off(arr.size());
+        size_t total = align64(m * sizeof(int32_t));
+        for (size_t j = 0; j < arr.size(); ++j) {
+            off[j] = total;
+            total += arr[j].host ? align64(m * arr[j].bytes) : 0;
+        }
+        int rc = grow_stage(p, shard, total);
+        if (rc != 0) {
+            return rc;
+        }
+        uint8_t* base = (uint8_t*)p->stage[shard];
+        int32_t* l_slots = (int32_t*)base;
+        std::vector<uint8_t*> local(arr.size());
+        for (size_t j = 0; j < arr.size(); ++j) {
+            local[j] = arr[j].host ? base + off[j] : nullptr;
+        }
+        const int lo = p->first[shard];
+        for (size_t k = 0; k < m; ++k) {
+            l_slots[k] = slots[el[k]] - lo;
+            for (size_t j = 0; j < arr.size(); ++j) {
+                if (local[j] && arr[j].in) {
+                    memcpy(local[j] + k * arr[j].bytes, arr[j].host + (size_t)el[k] * arr[j].bytes, arr[j].bytes);
+                }
+            }
+        }
+        rc = call(c, l_slots, (int)m, local.data());
+        if (rc != 0) {
+            return rc;
+        }
+        for (size_t k = 0; k < m; ++k) {
+            for (size_t j = 0; j < arr.size(); ++j) {
+                if (local[j] && arr[j].out) {
+                    memcpy(arr[j].host + (size_t)el[k] * arr[j].bytes, local[j] + k * arr[j].bytes, arr[j].bytes);
+                }
+            }
+        }
+        return 0;
+    });
+}
+
 extern "C" {
 
 int mbe_b200_pool_process_indexed(mbe_b200_pool* p, int codec, int input, const int32_t* slots, int n, int n_frames,
@@ -284,75 +360,43 @@ int mbe_b200_pool_process_indexed(mbe_b200_pool* p, int codec, int input, const 
     const size_t F = (size_t)n_frames, NS = MBE_B200_SAMPLES_PER_FRAME;
     const size_t fbytes = input == MBE_B200_INPUT_PACKED ? (size_t)mbe_b200_channel_frame_bytes(p->ctx[0], codec)
                                                          : (size_t)fbits * (input == MBE_B200_INPUT_SOFT ? 2u : 1u);
-    // stable partition of the element positions by owning shard: a slot always maps to one shard, so the context's
-    // first-occurrence rule holds for the whole list; out-of-range elements are rejected here, like a context does
-    std::vector<std::vector<int>> part(p->ctx.size());
-    for (int i = 0; i < n; ++i) {
-        const int slot = slots[i];
-        if (slot >= 0 && slot < p->max_streams) {
-            part[shard_of(p, slot)].push_back(i);
-            continue;
-        }
-        if (pcm) {
-            memset(pcm + (size_t)i * F * NS, 0, F * NS * sizeof(int16_t));
-        }
-        if (pcmf) {
-            memset(pcmf + (size_t)i * F * NS, 0, F * NS * sizeof(float));
-        }
-        if (bits) {
-            memset(bits + (size_t)i * F * pbits, 0, F * (size_t)pbits);
-        }
-        if (results) {
-            for (size_t f = 0; f < F; ++f) {
-                mbe_b200_result& r = results[(size_t)i * F + f];
-                memset(&r, 0, sizeof(r));
-                r.status = -1;   // MBE_STATUS_INVALID_ARGUMENT
-            }
-        }
+    return pool_indexed(p, "pool_process_indexed", slots, n, F, results,
+                        {{(uint8_t*)in, F * fbytes, true, false},
+                         {(uint8_t*)pcm, F * NS * sizeof(int16_t), false, true},
+                         {(uint8_t*)pcmf, F * NS * sizeof(float), false, true},
+                         {(uint8_t*)results, F * sizeof(mbe_b200_result), false, true},
+                         {bits, F * (size_t)pbits, false, true}},
+                        [&](mbe_b200_ctx* c, const int32_t* l_slots, int m, uint8_t* const* l) {
+                            return mbe_b200_process_indexed(c, codec, input, l_slots, m, n_frames, l[0], (int16_t*)l[1],
+                                                            (float*)l[2], (mbe_b200_result*)l[3], l[4]);
+                        });
+}
+
+int mbe_b200_pool_process_data_indexed(mbe_b200_pool* p, int codec, int packed, const int32_t* slots, int n, int n_frames,
+                                       const uint8_t* bits, mbe_b200_result* results_inout, int16_t* pcm, float* pcmf) {
+    if (!p) {
+        return MBE_B200_E_ARG;
     }
-    return for_each_part(p, "pool_process_indexed", part, [&](int shard, mbe_b200_ctx* c, const std::vector<int>& el) {
-        const size_t m = el.size();
-        // staging layout: local slots | frames | pcm | pcmf | results | bits
-        const size_t b_slots = align64(m * sizeof(int32_t)), b_in = align64(m * F * fbytes);
-        const size_t b_pcm = pcm ? align64(m * F * NS * sizeof(int16_t)) : 0, b_pcmf = pcmf ? align64(m * F * NS * sizeof(float)) : 0;
-        const size_t b_res = results ? align64(m * F * sizeof(mbe_b200_result)) : 0, b_bits = bits ? align64(m * F * pbits) : 0;
-        int rc = grow_stage(p, shard, b_slots + b_in + b_pcm + b_pcmf + b_res + b_bits);
-        if (rc != 0) {
-            return rc;
-        }
-        uint8_t* base = (uint8_t*)p->stage[shard];
-        int32_t* l_slots = (int32_t*)base;
-        uint8_t* l_in = base + b_slots;
-        int16_t* l_pcm = pcm ? (int16_t*)(l_in + b_in) : nullptr;
-        float* l_pcmf = pcmf ? (float*)(l_in + b_in + b_pcm) : nullptr;
-        mbe_b200_result* l_res = results ? (mbe_b200_result*)(l_in + b_in + b_pcm + b_pcmf) : nullptr;
-        uint8_t* l_bits = bits ? l_in + b_in + b_pcm + b_pcmf + b_res : nullptr;
-        const int lo = p->first[shard];
-        for (size_t k = 0; k < m; ++k) {
-            l_slots[k] = slots[el[k]] - lo;
-            memcpy(l_in + k * F * fbytes, in + (size_t)el[k] * F * fbytes, F * fbytes);
-        }
-        rc = mbe_b200_process_indexed(c, codec, input, l_slots, (int)m, n_frames, l_in, l_pcm, l_pcmf, l_res, l_bits);
-        if (rc != 0) {
-            return rc;
-        }
-        for (size_t k = 0; k < m; ++k) {
-            const size_t g = (size_t)el[k];
-            if (pcm) {
-                memcpy(pcm + g * F * NS, l_pcm + k * F * NS, F * NS * sizeof(int16_t));
-            }
-            if (pcmf) {
-                memcpy(pcmf + g * F * NS, l_pcmf + k * F * NS, F * NS * sizeof(float));
-            }
-            if (results) {
-                memcpy(results + g * F, l_res + k * F, F * sizeof(mbe_b200_result));
-            }
-            if (bits) {
-                memcpy(bits + g * F * pbits, l_bits + k * F * pbits, F * (size_t)pbits);
-            }
-        }
+    int fbits = 0, pbits = 0;
+    if (mbe_b200_geometry(codec, &fbits, &pbits) != 0 || packed < 0 || packed > 1 || n < 0 || n_frames < 0 ||
+        (n > 0 && !slots) || !bits) {
+        snprintf(p->err, sizeof(p->err), "pool_process_data_indexed: bad argument");
+        return MBE_B200_E_ARG;
+    }
+    if (n == 0 || n_frames == 0) {
         return 0;
-    });
+    }
+    const size_t F = (size_t)n_frames, NS = MBE_B200_SAMPLES_PER_FRAME;
+    const size_t bbytes = packed ? (size_t)mbe_b200_packed_param_bytes(codec) : (size_t)pbits;
+    return pool_indexed(p, "pool_process_data_indexed", slots, n, F, results_inout,
+                        {{(uint8_t*)bits, F * bbytes, true, false},
+                         {(uint8_t*)results_inout, F * sizeof(mbe_b200_result), true, true},
+                         {(uint8_t*)pcm, F * NS * sizeof(int16_t), false, true},
+                         {(uint8_t*)pcmf, F * NS * sizeof(float), false, true}},
+                        [&](mbe_b200_ctx* c, const int32_t* l_slots, int m, uint8_t* const* l) {
+                            return mbe_b200_process_data_indexed(c, codec, packed, l_slots, m, n_frames, l[0],
+                                                                 (mbe_b200_result*)l[1], (int16_t*)l[2], (float*)l[3]);
+                        });
 }
 
 int mbe_b200_pool_init_streams_indexed(mbe_b200_pool* p, const int32_t* slots, int n, const uint32_t* seeds) {
