@@ -307,7 +307,9 @@ struct __align__(16) WarpWS {
     int ncomp;                            // oscillator components of this frame (0: no voiced synthesis)
     unsigned k2mask;                      // list positions (< 32) of phase-interpolated harmonics
     unsigned short off[WARPS_PER_BLOCK + 3];  // this warp's copy of the block's slot offsets (prefix of padded counts)
-    unsigned short interp_item[8];        // interpolated harmonics of the block this warp renders in this round: owner << 8 | position
+    // interpolated harmonics of the block this warp renders in this round (indices into the block's list): up to 3 as a warp
+    // without an oscillator pass plus up to 7 dealt round-robin (7 per stream at most, W streams over W warps), so 10
+    unsigned short interp_item[10];
     unsigned char comp[112];              // component descriptor: harmonic << 2 | kind
     // LAST member: the parameter kernel of the multi-kernel path with hard-decision input only needs the decode scratch
     // (WS_STRIDE_SMALL), so its per-warp stride stops short of the tile

@@ -1664,6 +1664,9 @@ unvoiced_synthesis(float* out, mbo_parms* cur, const mbo_parms* prev, const floa
 #define TWO_PI_F (2.0f * (float)M_PI)
 #define CLIP_F   ((32767.0f * 0.95f) / 7.0f)
 
+/* mbo_run_work: where the frame being decoded by this thread reports its oscillator-bank work (null: nowhere) */
+static __thread int32_t* g_work;
+
 static void
 voiced_windowed(float* out, const float* W, float gain, float phase0, float step) {
     float sd, cd, s, c;
@@ -1723,6 +1726,7 @@ mbo_synthesize_speech(float* out, mbo_parms* cur, mbo_parms* prev, int has_rm0, 
         }
     }
 
+    int n_slots = 0, n_interp = 0;   /* the frame's work on the device's oscillator bank (mbo_run_work) */
     const float cw0 = cur->w0, pw0 = prev->w0;
     for (int l = 1; l <= 56; ++l) {
         float wrapped = fmodf(prev->PSIl[l], TWO_PI_F);
@@ -1747,6 +1751,8 @@ mbo_synthesize_speech(float* out, mbo_parms* cur, mbo_parms* prev, int has_rm0, 
             continue;
         }
         if ((l < 8) && cv && pv && (fabsf(cw0 - pw0) < (0.1f * cw0))) {
+            n_slots++;
+            n_interp++;
             /* phase/amplitude interpolation for stable low harmonics */
             float dphi = cur->PHIl[l] - prev->PHIl[l] - (((pw0 + cw0) * (float)(l * N)) / 2.0f);
             float dw = (1.0f / (float)N)
@@ -1758,6 +1764,10 @@ mbo_synthesize_speech(float* out, mbo_parms* cur, mbo_parms* prev, int has_rm0, 
                 out[n] += 2.0f * a * cosf(th);
             }
         } else {
+            /* a windowed component of gain exactly 0 adds +-0 and gets no slot, unless its phase is not finite (its
+             * product is NaN then) */
+            n_slots += (pv && ((2.0f * prev->Ml[l]) != 0.0f || !isfinite(prev->PHIl[l])))
+                       + (cv && ((2.0f * cur->Ml[l]) != 0.0f || !isfinite(cur->PHIl[l])));
             /* the reference adds prev then cur per sample; the two contributions go to the same
              * accumulator in that order, which is what two sequential passes would NOT give when
              * both are present - so interleave them explicitly */
@@ -1786,6 +1796,11 @@ mbo_synthesize_speech(float* out, mbo_parms* cur, mbo_parms* prev, int has_rm0, 
                 voiced_windowed(out, t_win_voiced, 2.0f * cur->Ml[l], cur->PHIl[l] - (cw0l * (float)N), cw0l);
             }
         }
+    }
+    if (g_work) {
+        g_work[0] = n_slots;
+        g_work[1] = n_interp;
+        g_work[2] = 1;
     }
 
     unvoiced_synthesis(out, cur, prev, noise);
@@ -2293,6 +2308,7 @@ typedef struct {
     int32_t* results;
     uint8_t* bits;
     mbo_parms* state;
+    int32_t* work;
 } run_t;
 
 static void*
@@ -2316,7 +2332,12 @@ run_worker(void* arg) {
             mbo_result res;
             memset(d, 0, sizeof(d));
             memset(&res, 0, sizeof(res));
+            if (j->work) {
+                g_work = j->work + idx * 3;
+                memset(g_work, 0, 3 * sizeof(int32_t));
+            }
             int ret = mbo_process_frame(j->codec, j->soft, pf, &res, fr, d, &cur, &prev, &enh, &rng);
+            g_work = NULL;
             if (ret < 0) {
                 memset(pf, 0, sizeof(pf));
                 memset(ps, 0, sizeof(ps));
@@ -2354,6 +2375,12 @@ run_worker(void* arg) {
 double
 mbo_run(int codec, int soft, int n_streams, int n_frames, const uint8_t* frames, const uint32_t* seeds, int16_t* pcm,
         float* pcmf, int32_t* results, uint8_t* bits, void* state, int n_threads) {
+    return mbo_run_work(codec, soft, n_streams, n_frames, frames, seeds, pcm, pcmf, results, bits, state, NULL, n_threads);
+}
+
+double
+mbo_run_work(int codec, int soft, int n_streams, int n_frames, const uint8_t* frames, const uint32_t* seeds, int16_t* pcm,
+             float* pcmf, int32_t* results, uint8_t* bits, void* state, int32_t* work, int n_threads) {
     if (n_threads < 1) {
         n_threads = 1;
     }
@@ -2368,7 +2395,7 @@ mbo_run(int codec, int soft, int n_streams, int n_frames, const uint8_t* frames,
     clock_gettime(CLOCK_MONOTONIC, &t0);
     for (int t = 0; t < n_threads; ++t) {
         run_t j = {codec, soft, n_streams, n_frames, 0, n_threads, t, frames, seeds, pcm, pcmf, results, bits,
-                   (mbo_parms*)state};
+                   (mbo_parms*)state, work};
         jobs[t] = j;
         if (n_threads > 1) {
             pthread_create(&th[t], NULL, run_worker, &jobs[t]);

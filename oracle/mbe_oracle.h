@@ -131,6 +131,17 @@ int mbo_process_frame(int codec, int soft, float* out, mbo_result* result, const
 double mbo_run(int codec, int soft, int n_streams, int n_frames, const uint8_t* frames, const uint32_t* seeds,
                int16_t* pcm, float* pcmf, int32_t* results, uint8_t* bits, void* state, int n_threads);
 
+/* mbo_run that also reports every frame's oscillator-bank work, work[stream][frame][3] (may be null):
+ *   [0] oscillator slots: one per interpolated harmonic (l < 8, voiced in both frames, |cur w0 - prev w0| < 0.1 cur w0),
+ *       one per other windowed component of the previous and of the current frame whose gain 2 Ml is not exactly 0 or
+ *       whose phase is not finite (the device's build_components rule);
+ *   [1] of them interpolated harmonics;
+ *   [2] 1 when the frame runs the speech synthesis (0 for tone, silence, comfort-noise and rejected frames).
+ * Everything else it returns is what mbo_run returns. */
+double mbo_run_work(int codec, int soft, int n_streams, int n_frames, const uint8_t* frames, const uint32_t* seeds,
+                    int16_t* pcm, float* pcmf, int32_t* results, uint8_t* bits, void* state, int32_t* work,
+                    int n_threads);
+
 #ifdef __cplusplus
 }
 #endif

@@ -411,3 +411,224 @@ def parms_view(state_bytes):
                 amplitudeThreshold=i[292], errorRate=f[293], errorCountTotal=i[294], errorCount4=i[295],
                 repeatCount=i[296], mutingThreshold=f[297], previousUw=f[298:554], noiseSeed=f[554],
                 noiseOverlap=f[555:651])
+
+
+def counters(dec):
+    """The kernel-timing record of `dec` since set_kernel_timing(True), through the C-ABI: (counters, launches).
+    counters: the bank kernel's [slots, interpolated harmonics, synthesised frames, 32-slot passes] (all 0 on the fused
+    path); launches: [parameter or fused, bank, unvoiced] kernel launches."""
+    ms = (ctypes.c_double * 3)()
+    n = (ctypes.c_longlong * 3)()
+    cnt = (ctypes.c_ulonglong * 4)()
+    assert dec.lib.mbe_b200_kernel_timing(dec.h, ms, n, cnt) == 0
+    return list(cnt), list(n)
+
+
+def oracle_work(codec, soft, frames, seeds, n_threads=8, want_float=True, want_state=True):
+    """run_cpu on the oracle's mbo_run_work: mbo_run's outputs plus "work", int32 [S][F][3] = per frame the oscillator
+    slots the bank kernel runs, how many of them are interpolated harmonics, and 1 when the frame runs the speech
+    synthesis."""
+    frames = np.ascontiguousarray(frames, dtype=np.uint8)
+    work = np.zeros(frames.shape[:2] + (3,), np.int32)
+    o = load_oracle()
+    out = run_cpu(lambda *a: o.mbo_run_work(*(a[:-1] + (_ptr(work), a[-1]))), codec, soft, frames, seeds, n_threads,
+                  want_float, want_state)
+    out["work"] = work
+    return out
+
+
+# ----------------------------------------------------------------------------------------------
+# Shaped workloads for the bank kernel's frame queue (mbe_split_bank_kernel, DESIGN 4.5).  Each warp of the resident bank
+# grid visits frames item = gw + v * W of a launch (item = stream * n_frames + frame, W warps in the grid) and streams their
+# oscillator slots through 32-slot passes, keeping a 32-frame window of slot counts.  The builders pick parameter vectors
+# by what the oracle decodes from them (pitch, number of bands, voicing) and encode them into valid channel frames, so
+# that a launch of SHAPED_STREAMS x SHAPED_FRAMES puts every warp in a chosen regime.
+# ----------------------------------------------------------------------------------------------
+SHAPED_CODECS = (IMBE7200, AMBE2450)
+SHAPED_MIXES = ("heavy", "boundaries", "empty", "interp", "quiet")
+SHAPED_STREAMS, SHAPED_FRAMES = 6000, 64
+BANK_WARPS_PER_SM = 4 * 8          # B_MINB resident blocks of B_WARPS warps (mbe_split.cuh)
+DESC_BYTES = 768 * 4               # one frame descriptor (DESC_WORDS)
+BOUNDARY_COUNTS = (32, 64, 96, 33, 65, 97)
+
+_B0_BITS = {IMBE7200: (0, 1, 2, 3, 4, 5, 85, 86), AMBE2450: (0, 1, 2, 3, 37, 38, 39)}
+_A2450_VUV_BITS = (4, 5, 6, 7, 35)
+_A2450_TONE_ID_BITS = tuple(range(12, 20))
+_pitch = {}
+
+
+def _set_field(p, idx, value):
+    n = len(idx)
+    for i, ix in enumerate(idx):
+        p[ix] = (value >> (n - 1 - i)) & 1
+
+
+def pitch_table(codec):
+    """{b0: (w0, L)} for every pitch index the oracle decodes as voice (mbo_decode_*_parms on a fresh state)."""
+    if codec not in _pitch:
+        o = load_oracle()
+        tab = {}
+        for b0 in range(208 if codec == IMBE7200 else 120):
+            p = np.zeros(PARAM_BITS[codec], np.uint8)
+            _set_field(p, _B0_BITS[codec], b0)
+            cur, prev, enh = (np.zeros(PARMS_BYTES, np.uint8) for _ in range(3))
+            o.mbo_init_parms(_ptr(cur), _ptr(prev), _ptr(enh))
+            if codec == IMBE7200:
+                rc = o.mbo_decode_imbe4400_parms(_ptr(p), _ptr(cur), _ptr(prev))
+            else:
+                rc = o.mbo_decode_ambe2450_parms(_ptr(p), _ptr(cur), _ptr(prev), 0)
+            v = parms_view(cur)
+            if rc == 0:
+                tab[b0] = (float(v["w0"]), int(v["L"]))
+        _pitch[codec] = tab
+    return _pitch[codec]
+
+
+def _unstable(wa, wb, margin=1.05):
+    """Both orders fail the interpolation's pitch test |cur w0 - prev w0| < 0.1 cur w0, with a margin."""
+    return abs(wa - wb) >= 0.1 * margin * max(wa, wb)
+
+
+def voice_params(codec, b0, voiced, rng):
+    """Parameter bits of a voice frame with pitch index b0, every band voiced (or every band unvoiced), other fields
+    (gains, spectral shape) random."""
+    p = rng.integers(0, 2, size=PARAM_BITS[codec], dtype=np.uint8)
+    _set_field(p, _B0_BITS[codec], b0)
+    if codec == IMBE7200:
+        L = pitch_table(codec)[b0][1]
+        K = 12 if L >= 37 else int(np.float32(L + 2) / np.float32(3))
+        p[48:48 + K] = 1 if voiced else 0          # the V/UV decisions of the K bands
+    else:
+        _set_field(p, _A2450_VUV_BITS, 0 if voiced else 16)   # V/UV codebook entries 0 (all voiced) and 16 (none)
+    return p
+
+
+def _ambe_special(kind, rng):
+    """AMBE+2 parameter bits of a tone frame (kind "tone": a valid single-frequency tone id) or a silence frame."""
+    p = rng.integers(0, 2, size=49, dtype=np.uint8)
+    if kind == "tone":
+        p[0:6] = 1
+        p[45:49] = 0
+        _set_field(p, _A2450_TONE_ID_BITS, int(rng.integers(8, 120)))
+    else:
+        _set_field(p, _B0_BITS[AMBE2450], 124)
+        _set_field(p, _A2450_VUV_BITS, 16)         # (bit 5 = 0: not a tone signature)
+    return p
+
+
+class _Pool:
+    """Distinct parameter vectors, each encoded once; a plan of pool indices [S][F] becomes the channel frames."""
+
+    def __init__(self, codec, rng):
+        self.codec, self.rng, self.params = codec, rng, []
+
+    def add(self, p):
+        self.params.append(p)
+        return len(self.params) - 1
+
+    def voice(self, b0, voiced=True, n=8):
+        return np.array([self.add(voice_params(self.codec, b0, voiced, self.rng)) for _ in range(n)])
+
+    def frames(self, plan):
+        enc = encode_imbe7200_frame if self.codec == IMBE7200 else encode_ambe_frame
+        tab = np.stack([enc(p).reshape(-1) for p in self.params])
+        return tab[plan]
+
+
+def _heavy_pitches(codec):
+    """(b0 of the largest L, b0s whose w0 is > 10 % away from it with the next largest L)."""
+    tab = pitch_table(codec)
+    hi = max(tab, key=lambda b: (tab[b][1], b))
+    lo = sorted((b for b in tab if _unstable(tab[b][0], tab[hi][0])), key=lambda b: -tab[b][1])[:3]
+    return hi, lo
+
+
+def _pair_for(codec, count):
+    """Two pitch indices, all bands voiced, whose alternation gives `count` slots per frame: L_a + L_b = count and w0
+    apart by more than 10 % (no interpolated harmonic)."""
+    tab = pitch_table(codec)
+    best = None
+    for a in tab:
+        for b in tab:
+            if tab[a][1] + tab[b][1] == count and tab[a][1] <= tab[b][1] and _unstable(tab[a][0], tab[b][0], 1.1):
+                key = tab[b][1] - tab[a][1]
+                if best is None or key < best[0]:
+                    best = (key, a, b)
+    assert best is not None, "no pitch pair for %d slots" % count
+    return best[1], best[2]
+
+
+def _quiet(pool, S, F, rng):
+    """Frames that run no oscillator slot once the stream is quiet: every band unvoiced; on AMBE+2 also tone and
+    silence frames."""
+    codec, tab = pool.codec, pitch_table(pool.codec)
+    uv = np.concatenate([pool.voice(b0, voiced=False, n=1) for b0 in list(tab)[::7]])
+    plan = uv[rng.integers(0, len(uv), size=(S, F))]
+    if codec == AMBE2450:
+        tone = np.array([pool.add(_ambe_special("tone", rng)) for _ in range(8)])
+        sil = np.array([pool.add(_ambe_special("silence", rng)) for _ in range(4)])
+        k = (np.arange(S)[:, None] + np.arange(F)[None, :]) % 4
+        plan = np.where(k == 1, tone[rng.integers(0, 8, size=(S, F))], plan)
+        plan = np.where(k == 3, sil[rng.integers(0, 4, size=(S, F))], plan)
+    return plan
+
+
+def shaped_frames(codec, mix, S=SHAPED_STREAMS, F=SHAPED_FRAMES, seed=0):
+    """Valid channel frames uint8 [S][F][FRAME_BITS] of one shaped mix (SHAPED_MIXES):
+    heavy       every band voiced, the largest L, the pitch jumping by more than 10 % on every frame: ~100-112 slots
+    boundaries  pitch pairs whose alternation gives 32, 64, 96, 33, 65 and 97 slots, in four-frame runs whose order
+                rotates from a per-stream offset
+    empty       streams (s // 74) % 40 < 4 heavy, the others quiet: a warp that walks frame f of every 74th stream (W =
+                4736 warps, 64 frames) meets four heavy frames, then 36 without a slot
+    interp      steady voice, mostly high pitch (few bands), the pitch index stepping by 1-2 every frame: interpolated
+                harmonics with a non-zero w0 change, several frames per pass
+    quiet       nothing but frames without slots (the first frame of a stream may fade out the initial model)"""
+    rng = np.random.default_rng((seed, codec, SHAPED_MIXES.index(mix)))
+    pool = _Pool(codec, rng)
+    tab = pitch_table(codec)
+    ss = np.arange(S)[:, None]
+    ff = np.arange(F)[None, :]
+
+    def heavy_plan():
+        hi, lo = _heavy_pitches(codec)
+        vh = pool.voice(hi)
+        vl = np.concatenate([pool.voice(b) for b in lo])
+        return np.where((ss + ff) % 2 == 0, vh[rng.integers(0, len(vh), size=(S, F))],
+                        vl[rng.integers(0, len(vl), size=(S, F))])
+
+    if mix == "heavy":
+        plan = heavy_plan()
+    elif mix == "boundaries":
+        pairs = [_pair_for(codec, c) for c in BOUNDARY_COUNTS]
+        va = np.stack([pool.voice(a, n=4) for a, _ in pairs])     # [pair][variant]
+        vb = np.stack([pool.voice(b, n=4) for _, b in pairs])
+        t = (rng.integers(0, len(pairs), size=(S, 1)) + ff // 4) % len(pairs)
+        var = rng.integers(0, 4, size=(S, F))
+        plan = np.where(ff % 2 == 0, va[t, var], vb[t, var])
+    elif mix == "empty":
+        heavy = (ss // 74) % 40 < 4
+        plan = np.where(heavy, heavy_plan(), _quiet(pool, S, F, rng))
+    elif mix == "interp":
+        b0s = sorted(tab)
+        lo_b0 = [b for b in b0s if tab[b][1] <= 16]
+        mid_b0 = [b for b in b0s if 20 <= tab[b][1] <= 40]
+        start = np.where(rng.random(S) < 0.8, rng.choice(lo_b0, size=S), rng.choice(mid_b0, size=S))
+        steps = rng.choice(np.array([-2, -1, 1, 2]), size=(S, F))
+        walk = np.clip(start[:, None] + np.cumsum(steps, axis=1), b0s[0], b0s[-1])
+        ids = {b: pool.voice(b, n=2) for b in np.unique(walk)}
+        plan = np.empty((S, F), np.int64)
+        for b, v in ids.items():
+            m = walk == b
+            plan[m] = v[rng.integers(0, len(v), size=int(m.sum()))]
+    elif mix == "quiet":
+        plan = _quiet(pool, S, F, rng)
+    else:
+        raise ValueError(mix)
+    return pool.frames(plan)
+
+
+def bank_walk(n_items, n_warps):
+    """[warp][visit] item indices of the bank kernel's grid-stride walk, item = gw + v * W (-1 past the end)."""
+    v = np.arange((n_items + n_warps - 1) // n_warps)
+    it = np.arange(n_warps)[:, None] + v[None, :] * n_warps
+    return np.where(it < n_items, it, -1)

@@ -2,8 +2,6 @@
 to the first three).  The kernel streams the oscillator slots of the frames a warp visits through 32-slot passes across
 frame boundaries (DESIGN 4.5), so on a launch with many frames per warp nearly every lane of every pass holds a slot; the
 fused kernel counts nothing."""
-import ctypes
-
 import pytest
 import torch
 
@@ -11,14 +9,6 @@ import mbe_testlib as T
 from __graft_entry__ import load_package
 
 pytestmark = pytest.mark.gpu
-
-
-def counters(dec):
-    ms = (ctypes.c_double * 3)()
-    n = (ctypes.c_longlong * 3)()
-    cnt = (ctypes.c_ulonglong * 4)()
-    assert dec.lib.mbe_b200_kernel_timing(dec.h, ms, n, cnt) == 0
-    return list(cnt)
 
 
 def test_bank_passes_and_lane_fill():
@@ -39,7 +29,7 @@ def test_bank_passes_and_lane_fill():
         dec.set_kernel_timing(True)
         dec.process_frames_dev(codec, 0, 0, S, F, frames.data_ptr(), pcm.data_ptr(), 0, res.data_ptr(), 0, st.cuda_stream)
         st.synchronize()
-        slots, interp, synth, passes = counters(dec)
+        (slots, interp, synth, passes), _ = T.counters(dec)
         dec.set_kernel_timing(False)
         if path == 1:
             assert 0 < synth <= S * F

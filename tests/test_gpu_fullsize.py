@@ -1,8 +1,8 @@
 """Parity at BASELINE.json's full batch sizes through size-independent properties.
 
 A full-size batch cannot be pushed through the CPU oracle in a test, so it is built from 512 distinct
-(stream seed, frame sequence) pairs replicated across the batch: every replica must give byte-identical PCM,
-results and parameter bits wherever it sits in the grid (block position, ragged tail, pipeline chunk), and the
+(stream seed, frame sequence) pairs replicated across the batch: every replica must give byte-identical int16 and float
+PCM, results and parameter bits wherever it sits in the grid (block position, ragged tail, pipeline chunk), and the
 512 distinct streams are checked against the oracle.  Device buffers via torch (plumbing only)."""
 import numpy as np
 import pytest
@@ -32,16 +32,18 @@ def _run_fullsize(codec, n_streams, n_frames, seed, base_frames=None, soft=0):
         d_base = torch.from_numpy(base_frames.reshape(BASE_N, n_frames, -1)).to(dev)
         d_frames = d_base.unsqueeze(0).expand(reps, -1, -1, -1).reshape(n_streams, n_frames, -1).contiguous()
         d_pcm = torch.empty((n_streams, n_frames, 160), dtype=torch.int16, device=dev)
+        d_pcmf = torch.empty((n_streams, n_frames, 160), dtype=torch.float32, device=dev)
         d_res = torch.empty((n_streams, n_frames, 6), dtype=torch.int32, device=dev)
         d_bits = torch.empty((n_streams, n_frames, pkg.PARAM_BITS[codec]), dtype=torch.uint8, device=dev)
         # cuda_stream = 0 selects the context's own NON-BLOCKING stream, which does not wait for torch's legacy
         # default stream: finish the replication copy before the launch
         torch.cuda.synchronize()
-        dec.process_frames_dev(codec, soft, 0, n_streams, n_frames, d_frames.data_ptr(), d_pcm.data_ptr(), 0,
+        dec.process_frames_dev(codec, soft, 0, n_streams, n_frames, d_frames.data_ptr(), d_pcm.data_ptr(), d_pcmf.data_ptr(),
                                d_res.data_ptr(), d_bits.data_ptr())
         torch.cuda.synchronize()
         # every replica equals replica 0
-        for name, t in (("pcm", d_pcm), ("results", d_res), ("bits", d_bits)):
+        # (float PCM bit for bit: rounding to int16 would hide last-bit differences in the bank kernel's sums)
+        for name, t in (("pcm", d_pcm), ("pcmf", d_pcmf.view(torch.int32)), ("results", d_res), ("bits", d_bits)):
             v = t.view(reps, BASE_N, -1)
             bad = (v != v[0:1]).any(dim=2)          # [replica][base stream]
             if bool(bad.any()):
@@ -52,6 +54,7 @@ def _run_fullsize(codec, n_streams, n_frames, seed, base_frames=None, soft=0):
         for r in (0, reps - 1):
             sl = slice(r * BASE_N, (r + 1) * BASE_N)
             assert np.array_equal(d_pcm[sl].cpu().numpy(), want["pcm"])
+            assert np.array_equal(d_pcmf[sl].cpu().numpy().view(np.uint32), want["pcmf"].view(np.uint32))
             assert np.array_equal(d_bits[sl].cpu().numpy(), want["bits"])
             assert np.array_equal(d_res[sl, :, 4].cpu().numpy(), want["results"][..., 4])
         # final state of the last replica equals the first replica's, byte for byte
@@ -68,7 +71,8 @@ def test_config2_ambe2450_65536_streams_x_50_frames():
 
 
 def test_config3_imbe7200_1m_streams_x_50_frames():
-    """BASELINE.json configs[2] at its single-GPU size: IMBE 7200x4400, 1,048,576 streams x 50 frames (37 GB of HBM)."""
+    """BASELINE.json configs[2] at its single-GPU size: IMBE 7200x4400, 1,048,576 streams x 50 frames (about 71 GB of HBM with
+    float PCM)."""
     _run_fullsize(0, 1048576, 50, 0x7200)
 
 

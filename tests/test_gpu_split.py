@@ -101,18 +101,29 @@ def test_kernel_timing_and_bank_counters(pkg):
     dec.close()
 
 
-@pytest.mark.parametrize("soft", [0, 1], ids=["hard", "soft"])
-@pytest.mark.parametrize("codec", [0, 1, 2, 3])
-def test_state_machine_fuzz_against_the_oracle(pkg, codec, soft):
+# (codec, input): hard and soft input for every codec through the host pipeline, and hard input through one device-resident
+# call large enough that every bank warp walks at least 64 frames (its 32-frame window fills and moves, DESIGN 4.5)
+FUZZ_CASES = [pytest.param(c, s, id="%d-%s" % (c, s)) for s in ("hard", "soft") for c in (0, 1, 2, 3)] + \
+             [pytest.param(c, "dev", id="%d-dev" % c) for c in (0, 3)]
+
+
+@pytest.mark.parametrize("codec,mode", FUZZ_CASES)
+def test_state_machine_fuzz_against_the_oracle(pkg, codec, mode):
     """Differential fuzz of the frame state machines on the default (multi-kernel) path: 4096 streams x 24 frames per codec,
     every frame drawn at random from {random bits, a fresh valid frame, the previous valid frame held, a valid frame with
     1-8 % flipped bits, an AMBE tone / erasure signature, a frame with a non-binary bit}, so that repeats, headroom resets,
     mutes, re-initialisation, erasures, replays and tones follow each other in every order - which is what the descriptor's
     previousUw op codes have to replay exactly.  Everything against the oracle: bits, results, int16 / float PCM, final
     triplets.  Soft-decision input: the same mixture with seeded flips and reliabilities (fewer streams: the oracle's
-    exhaustive soft decoders are slow), decoded in three launches of different lengths."""
-    rng = np.random.default_rng(0xF022 + codec + 16 * soft)
-    S, F = (4096, 24) if not soft else (384, 18)
+    exhaustive soft decoders are slow), decoded in three launches of different lengths.  Device-resident: hard input, as
+    many streams as give 64 frames to each warp of the resident bank grid, in one process_frames_dev call."""
+    soft = int(mode == "soft")
+    rng = np.random.default_rng(0xF022 + codec + 16 * soft + 32 * (mode == "dev"))
+    S, F = (4096, 24) if mode == "hard" else (384, 18) if soft else (0, 24)
+    if mode == "dev":
+        import torch
+        bank_warps = torch.cuda.get_device_properties(0).multi_processor_count * T.BANK_WARPS_PER_SM
+        S = -(-64 * bank_warps // F // 64) * 64
     fb, pb = T.FRAME_BITS[codec], T.PARAM_BITS[codec]
     enc = {0: T.encode_imbe7200_frame, 1: T.encode_imbe7100_frame}.get(codec, T.encode_ambe_frame)
     P = 96
@@ -155,6 +166,22 @@ def test_state_machine_fuzz_against_the_oracle(pkg, codec, soft):
         parts = [dec.process_frames(codec, np.ascontiguousarray(frames[:, a:b]), soft=True, want_float=True)
                  for a, b in ((0, 1), (1, 7), (7, F))]
         got = {k: np.concatenate([p[k] for p in parts], axis=1) for k in ("bits", "results", "pcm", "pcmf")}
+    elif mode == "dev":
+        d_frames = torch.from_numpy(frames).to("cuda:0")
+        d = dict(pcm=torch.empty((S, F, 160), dtype=torch.int16, device="cuda:0"),
+                 pcmf=torch.empty((S, F, 160), dtype=torch.float32, device="cuda:0"),
+                 results=torch.empty((S, F, 6), dtype=torch.int32, device="cuda:0"),
+                 bits=torch.empty((S, F, pb), dtype=torch.uint8, device="cuda:0"))
+        torch.cuda.synchronize()
+        dec.set_kernel_timing(True)
+        dec.process_frames_dev(codec, 0, 0, S, F, d_frames.data_ptr(), d["pcm"].data_ptr(), d["pcmf"].data_ptr(),
+                               d["results"].data_ptr(), d["bits"].data_ptr())
+        torch.cuda.synchronize()
+        _, launches = T.counters(dec)
+        dec.set_kernel_timing(False)
+        assert launches[1] == 1 and S * F >= 64 * bank_warps
+        got = {k: v.cpu().numpy() for k, v in d.items()}
+        got["results"] = got["results"].view(pkg.RESULT_DTYPE)[..., 0]
     else:
         got = dec.process_frames(codec, frames, want_float=True)
     res = got["results"]
