@@ -111,6 +111,9 @@ MBE_B200_API int mbe_b200_kernel_path(const mbe_b200_ctx* ctx);
  * kernel counts nothing. */
 MBE_B200_API int mbe_b200_set_kernel_timing(mbe_b200_ctx* ctx, int enable);
 MBE_B200_API int mbe_b200_kernel_timing(mbe_b200_ctx* ctx, double ms[3], long long launches[3], unsigned long long counters[4]);
+/* The unvoiced kernel's counters over the same timing session: [0] frames whose noise spectrum came from the context's
+ * noise table, [1] frames that computed their own (cold starts, imported states, MBE_B200_NOISE_TABLE=0).  Synchronises. */
+MBE_B200_API int mbe_b200_noise_table_counters(mbe_b200_ctx* ctx, unsigned long long counters[2]);
 
 /* ---- stream state ---------------------------------------------------------------------------
  * init_streams == per stream: mbe_setThreadRngSeed(seed) (mbelib.h:596; seeds==NULL: fresh-thread

@@ -41,6 +41,7 @@ _EXPORTS = ["mbe_b200_create", "mbe_b200_destroy", "mbe_b200_last_error", "mbe_b
             "mbe_b200_pool_shards", "mbe_b200_pool_shard", "mbe_b200_pool_init_streams", "mbe_b200_pool_export_state",
             "mbe_b200_pool_import_state", "mbe_b200_pool_process_frames", "mbe_b200_pool_process_frames_packed",
             "mbe_b200_set_kernel_path", "mbe_b200_kernel_path", "mbe_b200_set_kernel_timing", "mbe_b200_kernel_timing",
+            "mbe_b200_noise_table_counters",
             "mbe_b200_host_alloc", "mbe_b200_host_free", "mbe_b200_host_register", "mbe_b200_host_unregister",
             "mbe_b200_single_frame", "mbe_b200_process_indexed_dev", "mbe_b200_process_indexed", "mbe_b200_submit_indexed",
             "mbe_b200_init_streams_indexed", "mbe_b200_export_state_indexed", "mbe_b200_import_state_indexed",
@@ -97,6 +98,7 @@ def load_library():
         lib.mbe_b200_host_register.argtypes = [vp, ctypes.c_size_t]
         lib.mbe_b200_host_unregister.argtypes = [vp]
         lib.mbe_b200_kernel_timing.argtypes = [vp, vp, vp, vp]
+        lib.mbe_b200_noise_table_counters.argtypes = [vp, vp]
         lib.mbe_b200_packed_frame_bytes.argtypes = [ci]
         lib.mbe_b200_pipeline_plan.argtypes = [ci, ctypes.POINTER(ci), ci]
         lib.mbe_b200_process_frames_packed_dev.argtypes = [vp, ci, ci, ci, ci, vp, vp, vp, vp, vp, vp]
@@ -544,6 +546,12 @@ class Decoder:
         names = ("parameter", "bank", "unvoiced")
         return ({names[i]: (float(ms[i]), int(n[i])) for i in range(3)},
                 dict(slots=int(cnt[0]), interpolated=int(cnt[1]), frames=int(cnt[2])))
+
+    def noise_table_counters(self):
+        """Unvoiced-kernel frames since set_kernel_timing(True): (noise spectra read from the table, computed in the kernel)."""
+        cnt = np.zeros(2, np.uint64)
+        self._check(self.lib.mbe_b200_noise_table_counters(self.h, _p(cnt)), "noise_table_counters")
+        return int(cnt[0]), int(cnt[1])
 
     def set_normalized_float(self, enable):
         self._check(self.lib.mbe_b200_set_normalized_float(self.h, int(bool(enable))), "set_normalized_float")

@@ -1387,7 +1387,10 @@ struct mbe_b200_ctx {
     int kt_on, kt_n;
     cudaEvent_t* kt_ev;               // [2 * KT_MAX]
     unsigned char* kt_kind;           // [KT_MAX]: 0 parameter (or fused) kernel, 1 bank kernel, 2 unvoiced kernel
-    unsigned long long* d_cnt;        // [4] device counters of the bank kernel
+    unsigned long long* d_cnt;        // [6] device counters of the bank kernel ([0..3]) and the unvoiced kernel ([4..5])
+    // noise spectrum table of the unvoiced kernel (mbe_noise_table_kernel): built on the first multi-kernel launch
+    float* d_noise_tab;
+    cudaEvent_t ev_noise_tab;         // the build is done (launches on the pipeline's compute streams wait for it)
     // indexed calls: the claim tag of every slot (mbe_claim_kernel), the epoch of the latest call, and the device copy of a
     // host slot list (reused like d_in: host-pointer calls are synchronous or pending until mbe_b200_wait)
     unsigned long long* d_claim;      // [max_streams]
@@ -1509,6 +1512,17 @@ static void build_tables(DevTables* t) {
         for (int k = 0; k <= 160; ++k) {
             t->uvA[k] = (unsigned)a;
             t->uvC[k] = (unsigned)c;
+            c = (171ull * c + 11213ull) % 53125ull;
+            a = (171ull * a) % 53125ull;
+        }
+    }
+    {
+        unsigned long long a = 1, c = 0;
+        for (int k = 0; k < NOISE_ROWS; ++k) {
+            if (k >= NOISE_ROWS - 96) {
+                t->uvBA[k - (NOISE_ROWS - 96)] = (unsigned)a;
+                t->uvBC[k - (NOISE_ROWS - 96)] = (unsigned)c;
+            }
             c = (171ull * c + 11213ull) % 53125ull;
             a = (171ull * a) % 53125ull;
         }
@@ -1636,6 +1650,7 @@ struct Knobs {
     long desc_mb;     // MBE_B200_DESC_MB: descriptor buffer budget per launch, MiB
     int skip_kernels; // MBE_B200_SKIP_KERNELS (timing experiments only, results are wrong): 1 parameter (after the first use of
                       // a descriptor buffer), 2 bank, 4 unvoiced kernel launches are skipped
+    int noise_table;  // MBE_B200_NOISE_TABLE: 0 = the unvoiced kernel computes every noise spectrum (no 54 MB table per context)
 };
 static Knobs g_knobs;
 static std::once_flag g_knobs_once;
@@ -1656,6 +1671,8 @@ static const Knobs& knobs() {
         g_knobs.split = e ? atoi(e) : MBE_SPLIT_DEFAULT;
         e = getenv("MBE_B200_SKIP_KERNELS");
         g_knobs.skip_kernels = e ? atoi(e) : 0;
+        e = getenv("MBE_B200_NOISE_TABLE");
+        g_knobs.noise_table = e ? atoi(e) : 1;
         e = getenv("MBE_B200_DESC_MB");
         g_knobs.desc_mb = e ? atol(e) : 2048;
         if (g_knobs.desc_mb < 1) {
@@ -1717,7 +1734,8 @@ static StreamKernelFn pick_stream_kernel(int codec, int soft, int mode, bool spl
 }
 
 static size_t bank_kernel_smem(void) { return BANK_TAB_FLOATS * sizeof(float) + (size_t)B_WARPS * sizeof(BankWS); }
-static size_t unvoiced_kernel_smem(void) { return sizeof(BlockTables) + (size_t)U_WARPS * sizeof(UnvWS); }
+static size_t unvoiced_kernel_smem(void) { return sizeof(BlockTables) + 96 * sizeof(uint2) + (size_t)U_WARPS * sizeof(UnvWS); }
+static size_t noise_table_smem(void) { return sizeof(BlockTables) + (size_t)NOISE_TAB_WARPS * sizeof(UnvWS); }
 
 typedef void (*DecodeKernelFn)(int, const uint8_t*, uint8_t*, mbe_b200_result*, const DevTables*);
 static DecodeKernelFn pick_decode_kernel(int codec, int soft) {
@@ -1891,6 +1909,7 @@ int mbe_b200_create(mbe_b200_ctx** out, int device_ordinal, int max_streams) {
     CUC(cudaFuncSetAttribute(mbe_split_bank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bank_kernel_smem()));
     CUC(cudaFuncSetAttribute(mbe_split_unvoiced_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)unvoiced_kernel_smem()));
+    CUC(cudaFuncSetAttribute(mbe_noise_table_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)noise_table_smem()));
     for (int i = 0; i < DESC_SLOTS; ++i) {
         CUC(cudaEventCreateWithFlags(&ctx->ev_desc[i], cudaEventDisableTiming));
     }
@@ -1899,6 +1918,7 @@ int mbe_b200_create(mbe_b200_ctx** out, int device_ordinal, int max_streams) {
         CUC(cudaEventCreateWithFlags(&ctx->ev_join[i], cudaEventDisableTiming));
     }
     CUC(cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
+    CUC(cudaEventCreateWithFlags(&ctx->ev_noise_tab, cudaEventDisableTiming));
     ctx->split = knobs().split ? 1 : 0;
     CUC(cudaFuncSetAttribute(mbe_stage_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)stream_kernel_smem()));
 #undef CUC
@@ -1956,6 +1976,10 @@ void mbe_b200_destroy(mbe_b200_ctx* ctx) {
     if (ctx->ev_fork) {
         cudaEventDestroy(ctx->ev_fork);
     }
+    if (ctx->ev_noise_tab) {
+        cudaEventDestroy(ctx->ev_noise_tab);
+    }
+    cudaFree(ctx->d_noise_tab);
     for (int i = 0; i < DESC_SLOTS; ++i) {
         if (ctx->ev_desc[i]) {
             cudaEventDestroy(ctx->ev_desc[i]);
@@ -2265,6 +2289,27 @@ static int launch_stream_kernel(mbe_b200_ctx* ctx, const LaunchArgs& a_in, cudaS
     }
     const bool fork = (kslot < 0);
     int rc;
+    if (knobs().noise_table && !ctx->d_noise_tab) {
+        // published to the context only once the build is enqueued: a context never holds an unfilled table
+        float* tab = nullptr;
+        CU(cudaMalloc(&tab, (size_t)NOISE_ROWS * NFFT * sizeof(float)));
+        mbe_noise_table_kernel<<<(NOISE_ROWS + NOISE_TAB_WARPS - 1) / NOISE_TAB_WARPS, NOISE_TAB_WARPS * 32, noise_table_smem(),
+                                 st>>>(ctx->d_tab, tab);
+        cudaError_t e = cudaGetLastError();
+        if (e == cudaSuccess) {
+            e = cudaEventRecord(ctx->ev_noise_tab, st);
+        }
+        if (e != cudaSuccess) {
+            cudaFree(tab);
+            return fail(ctx, MBE_B200_E_CUDA, "noise table build", e);
+        }
+        ctx->d_noise_tab = tab;
+    }
+    if (ctx->d_noise_tab) {
+        // every launch, on whatever stream, is ordered after the build (which ran on the stream of the first launch); on a
+        // caller's stream before the fork, so that every internal stream inherits it
+        CU(cudaStreamWaitEvent(st, ctx->ev_noise_tab, 0));
+    }
     if (fork) {
         CU(cudaEventRecord(ctx->ev_fork, st));
         for (int i = 0; i < n_aux; ++i) {
@@ -2306,6 +2351,7 @@ static int launch_stream_kernel(mbe_b200_ctx* ctx, const LaunchArgs& a_in, cudaS
         sa.counters = ctx->kt_on ? ctx->d_cnt : nullptr;
         sa.slots = a.slots;
         sa.slot_base = a.slot_base;
+        sa.noise_tab = ctx->d_noise_tab;
         long long bank_blocks = ((long long)ns * a.n_frames + B_WARPS - 1) / B_WARPS;   // at least one frame per warp
         const long long resident = (long long)g_sm_count.load() * B_MINB;   // grid-stride warps: one resident wave is enough
         if (bank_blocks > resident) {
@@ -2362,11 +2408,11 @@ int mbe_b200_set_kernel_timing(mbe_b200_ctx* ctx, int enable) {
         for (int i = 0; i < 2 * KT_MAX; ++i) {
             CU(cudaEventCreate(&ctx->kt_ev[i]));
         }
-        CU(cudaMalloc(&ctx->d_cnt, 4 * sizeof(unsigned long long)));
+        CU(cudaMalloc(&ctx->d_cnt, 6 * sizeof(unsigned long long)));
     }
     if (enable) {
         CU(cudaDeviceSynchronize());
-        CU(cudaMemsetAsync(ctx->d_cnt, 0, 4 * sizeof(unsigned long long), ctx->stream));
+        CU(cudaMemsetAsync(ctx->d_cnt, 0, 6 * sizeof(unsigned long long), ctx->stream));
         CU(cudaStreamSynchronize(ctx->stream));
         ctx->kt_n = 0;
     }
@@ -2398,6 +2444,20 @@ int mbe_b200_kernel_timing(mbe_b200_ctx* ctx, double ms[3], long long launches[3
         launches[k]++;
     }
     CU(cudaMemcpy(counters, ctx->d_cnt, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+    return 0;
+}
+
+int mbe_b200_noise_table_counters(mbe_b200_ctx* ctx, unsigned long long counters[2]) {
+    if (!ctx || !counters) {
+        return MBE_B200_E_ARG;
+    }
+    counters[0] = counters[1] = 0;
+    if (!ctx->d_cnt) {
+        return 0;
+    }
+    CU(cudaSetDevice(ctx->device));
+    CU(cudaDeviceSynchronize());
+    CU(cudaMemcpy(counters, ctx->d_cnt + 4, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
     return 0;
 }
 

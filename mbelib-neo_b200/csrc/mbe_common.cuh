@@ -185,6 +185,7 @@ struct DevTables {
     // LCG jump-ahead tables: x_k = (A[k]*x_0 + C[k]) mod m
     unsigned short pnA[116], pnC[116];  // PN de-scrambler, mod 65536
     unsigned uvA[161], uvC[161];        // unvoiced noise, mod 53125
+    unsigned uvBA[96], uvBC[96];        // LCG^(53125 - 96 + k) = LCG^(k - 96) (full period): a frame's natural overlap word k
     unsigned long long cnA[161], cnC[161];  // comfort noise, mod 2^48
     // ECC
     unsigned short golay_par_hi[64], golay_par_lo[64];

@@ -232,9 +232,11 @@ struct SynthArgs {
     uint32_t* state;        // [max_streams][STATE_WORDS]: only the previousUw words are touched
     const DevTables* tab;
     unsigned long long* counters;   // profiling (may be null): [0] oscillator slots run, [1] of them interpolated harmonics,
-                                    // [2] frames synthesised, [3] 32-slot passes of the bank kernel
+                                    // [2] frames synthesised, [3] 32-slot passes of the bank kernel; unvoiced kernel:
+                                    // [4] noise spectra taken from the table, [5] noise spectra computed in the kernel
     const int32_t* slots;   // indexed calls: as LaunchArgs (slot_of)
     int slot_base;
+    const float* noise_tab; // [NOISE_ROWS][256] forward noise spectra (mbe_noise_table_kernel), null: every frame computes its own
 };
 
 // Oscillator tile of the bank kernel: 32 samples x 32 slots, rows padded to 36 words: phase A (lane = slot, one row per
@@ -465,10 +467,16 @@ __global__ void __launch_bounds__(B_WARPS * 32, B_MINB) mbe_split_bank_kernel(co
 }
 
 // ---- unvoiced kernel ---------------------------------------------------------------------------------------------------
+// Three transform buffers: a frame runs in two of them (A, B) while the third receives the next frame's noise spectrum from
+// the table; the next frame's A is that third buffer, its B the frame's A, and its prefetch target the frame's B.
+// With the table, a frame's header words 0..7 and overlap are staged into dstage two frames ahead: the check that picks the
+// next frame's table row, and the frame's own ops and noise buffer, wait for no global load.
+constexpr int DSTAGE_WORDS = 8 + 96;
 struct __align__(16) UnvWS {
-    float a[324];
-    float b[324];
-    float scale[132];
+    float buf[3][324];
+    uint32_t dstage[2][DSTAGE_WORDS];
+    float scale[130];
+    unsigned n_tab[2];   // frames of the launch whose noise spectrum came from the table / was computed (with A.counters)
 };
 
 __device__ __forceinline__ void uw_copy(uint32_t* dst, const uint32_t* src, int lane) {
@@ -484,9 +492,8 @@ __device__ __forceinline__ void uw_copy(uint32_t* dst, const uint32_t* src, int 
 }
 
 // band scales + backward transform for one frame (unvoiced_shape on descriptor data)
-__device__ __forceinline__ void split_unvoiced_shape(UnvWS& ws, const uint32_t* d, int L, float w0, unsigned cu_lo, unsigned cu_hi,
-                                                     const BlockTables* bt, int lane) {
-    float* A = ws.a;
+__device__ __forceinline__ void split_unvoiced_shape(UnvWS& ws, float* A, float* B, const uint32_t* d, int L, float w0,
+                                                     unsigned cu_lo, unsigned cu_hi, const BlockTables* bt, int lane) {
     float* scale = ws.scale;
     const float mult = (256.0f / (2.0f * 3.14159265358979323846f)) * w0;
     for (int l = 1 + lane; l <= L; l += 32) {
@@ -519,27 +526,14 @@ __device__ __forceinline__ void split_unvoiced_shape(UnvWS& ws, const uint32_t* 
         }
     }
     __syncwarp();
-    rfft256_backward(A, ws.b, bt->tw, scale, lane);
+    rfft256_backward(A, B, bt->tw, scale, lane);
 }
 
-// the frame's windowed noise buffer from the descriptor (make_noise's FFT input)
-__device__ __forceinline__ void split_noise(UnvWS& ws, const uint32_t* d, const BlockTables* bt, int lane) {
-    float* A = ws.a;
-    const float seed = __uint_as_float(d[D_SEED]);
-    if (seed < 0.0f) {
-        for (int i = lane; i < NFFT; i += 32) {
-            A[i] = 0.0f;
-        }
-        return;
-    }
+// make_noise's FFT input: the windowed 256-sample buffer of a frame whose generator starts at sc (sc < 53125) and whose
+// overlap word 32 r + lane is ov[r]
+__device__ __forceinline__ void noise_buffer(float* A, unsigned sc, const float ov[3], const BlockTables* bt, int lane) {
     constexpr unsigned A32 = lcg_pow_a(32), C32 = lcg_pow_c(32);
-    unsigned sc = ((unsigned)seed) % 53125u;
     const uint2 jl = bt->uv_jump[lane];
-    float ov[3];
-#pragma unroll
-    for (int r = 0; r < 3; ++r) {
-        ov[r] = __uint_as_float(d[D_OV + 32 * r + lane]);
-    }
 #pragma unroll
     for (int c = 0; c < 5; ++c) {
         const int i = 32 * c + lane;
@@ -554,11 +548,120 @@ __device__ __forceinline__ void split_noise(UnvWS& ws, const uint32_t* d, const 
     }
 }
 
+// the generator state a frame starts from: (unsigned)seed % 53125 for seed >= 0, as make_noise computes it
+__device__ __forceinline__ unsigned noise_start(float seed) { return ((unsigned)seed) % 53125u; }
+
+// the frame's windowed noise buffer from its descriptor's seed and overlap words ov[0..95]
+__device__ __forceinline__ void split_noise(float* A, float seed, const uint32_t* ov_words, const BlockTables* bt, int lane) {
+    if (seed < 0.0f) {
+        for (int i = lane; i < NFFT; i += 32) {
+            A[i] = 0.0f;
+        }
+        return;
+    }
+    float ov[3];
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        ov[r] = __uint_as_float(ov_words[32 * r + lane]);
+    }
+    noise_buffer(A, noise_start(seed), ov, bt, lane);
+}
+
+// ---- noise spectrum table ------------------------------------------------------------------------------------------
+// A frame whose overlap is the one its own generator state sc left behind - overlap word k = LCG^(k - 96)(sc), the 96 states
+// before sc, which make_noise_state always produces - has a noise buffer that depends on sc alone, and so has its forward
+// spectrum.  Row sc of the table is that spectrum, A[1..256] of the X4 layout, computed by the unvoiced kernel's own
+// noise_buffer and rfft256_forward.  A frame takes its row only after checking all 96 overlap words bit for bit
+// (noise_prefetch); any other frame (cold starts, imported states) computes its own.
+constexpr int NOISE_ROWS = 53125;
+constexpr int NOISE_TAB_WARPS = 8;
+
+// overlap word 32 r + lane of the natural overlap before generator state sc; bk[r] = (uvBA, uvBC)[32 r + lane]
+__device__ __forceinline__ unsigned noise_overlap_word(unsigned sc, uint2 bk) { return (bk.x * sc + bk.y) % 53125u; }
+
+__global__ void __launch_bounds__(NOISE_TAB_WARPS * 32) mbe_noise_table_kernel(const DevTables* __restrict__ T, float* tab) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    BlockTables* bt = reinterpret_cast<BlockTables*>(smem_raw);
+    UnvWS* wsa = reinterpret_cast<UnvWS*>(smem_raw + sizeof(BlockTables));
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) {
+        bt->tw[i] = T->tw[i];
+        bt->uvwin[i] = T->uvwin[i];
+    }
+    if (threadIdx.x < 32) {
+        bt->uv_jump[threadIdx.x] = make_uint2(T->uvA[threadIdx.x], T->uvC[threadIdx.x]);
+    }
+    __syncthreads();
+    const int warp = threadIdx.x >> 5;
+    const int lane = threadIdx.x & 31;
+    float* A = wsa[warp].buf[0];
+    float* B = wsa[warp].buf[1];
+#pragma unroll 1
+    for (int sc = blockIdx.x * NOISE_TAB_WARPS + warp; sc < NOISE_ROWS; sc += gridDim.x * NOISE_TAB_WARPS) {
+        float ov[3];
+#pragma unroll
+        for (int r = 0; r < 3; ++r) {
+            const int k = 32 * r + lane;
+            ov[r] = (float)noise_overlap_word((unsigned)sc, make_uint2(T->uvBA[k], T->uvBC[k]));
+        }
+        noise_buffer(A, (unsigned)sc, ov, bt, lane);
+        __syncwarp();
+        rfft256_forward(A, B, bt->tw, lane);
+        float* row = tab + (size_t)sc * NFFT;
+#pragma unroll
+        for (int q = 0; q < 8; ++q) {
+            row[32 * q + lane] = A[1 + 32 * q + lane];
+        }
+        __syncwarp();
+    }
+}
+
+// 4-byte asynchronous copies global -> shared (the spectrum sits at A + 1, which is 8-byte but not 16-byte aligned)
+__device__ __forceinline__ void cp_async4(float* dst, const float* src) {
+    const unsigned s = (unsigned)__cvta_generic_to_shared(dst);
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(s), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;\n" ::: "memory"); }
+
+// descriptor words 0..7 and the overlap of frame d into a staging buffer (16-byte copies: both runs are 16-byte aligned)
+static_assert(D_SEED < 8 && D_INFO < 8 && D_OV % 4 == 0, "staged descriptor words");
+__device__ __forceinline__ void stage_desc(uint32_t* st, const uint32_t* d, int lane) {
+    if (lane < DSTAGE_WORDS / 4) {
+        const int w = 4 * lane;
+        const uint32_t* src = d + (w < 8 ? w : D_OV + w - 8);
+        const unsigned s = (unsigned)__cvta_generic_to_shared(st + w);
+        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(s), "l"(src) : "memory");
+    }
+}
+
+// whether a frame's noise spectrum is row sc of the table (st = its staged descriptor words): the frame runs the synthesis,
+// seed >= 0, and its overlap is the natural one of sc, word for word (bk = the uvBA / uvBC pairs).  If so, the row is fetched
+// into A + 1 (asynchronously: cp_async_wait_all).
+__device__ __forceinline__ bool noise_prefetch(const uint32_t* st, const float* tab, const uint2* bk, float* A, int lane) {
+    const float seed = __uint_as_float(st[D_SEED]);
+    const bool cand = (st[D_INFO] & 1u) && seed >= 0.0f;
+    bool ok = cand;
+    const unsigned sc = cand ? noise_start(seed) : 0u;
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        ok = ok && st[8 + 32 * r + lane] == __float_as_uint((float)noise_overlap_word(sc, bk[32 * r + lane]));
+    }
+    if (__ballot_sync(FULL, ok) != FULL) {
+        return false;
+    }
+    const float* row = tab + (size_t)sc * NFFT;
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {
+        cp_async4(A + 1 + 32 * q + lane, row + 32 * q + lane);
+    }
+    return true;
+}
+
 // one warp = one stream, frames in order (the overlap-add needs the previous frame's block)
 __global__ void __launch_bounds__(U_WARPS * 32, U_MINB) mbe_split_unvoiced_kernel(const SynthArgs A) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     BlockTables* bt = reinterpret_cast<BlockTables*>(smem_raw);
-    UnvWS* wsa = reinterpret_cast<UnvWS*>(smem_raw + sizeof(BlockTables));
+    uint2* bk = reinterpret_cast<uint2*>(smem_raw + sizeof(BlockTables));   // [96] uvBA / uvBC
+    UnvWS* wsa = reinterpret_cast<UnvWS*>(smem_raw + sizeof(BlockTables) + 96 * sizeof(uint2));
     const DevTables* T = A.tab;
     {
         for (int i = threadIdx.x; i < 256; i += blockDim.x) {
@@ -573,6 +676,9 @@ __global__ void __launch_bounds__(U_WARPS * 32, U_MINB) mbe_split_unvoiced_kerne
         if (threadIdx.x < 32) {
             bt->uv_jump[threadIdx.x] = make_uint2(T->uvA[threadIdx.x], T->uvC[threadIdx.x]);
         }
+        for (int i = threadIdx.x; i < 96; i += blockDim.x) {
+            bk[i] = make_uint2(T->uvBA[i], T->uvBC[i]);
+        }
         __syncthreads();
     }
     const int warp = threadIdx.x >> 5;
@@ -586,6 +692,25 @@ __global__ void __launch_bounds__(U_WARPS * 32, U_MINB) mbe_split_unvoiced_kerne
     uint32_t* h_prev = gs + PARMS_WORDS;
     uint32_t* h_enh = gs + 2 * PARMS_WORDS;
     uint32_t* h_spill = gs + SPILL_WORD;
+    // bits 0..1: the buffer of the frame's A (see UnvWS); bit 2: its noise spectrum is on its way from the table.  At the top
+    // of frame f the warp waits for the copies it issued a frame earlier (frame f's row, frame f + 1's staged words) and
+    // issues frame f + 1's row; frame f + 2's words follow once frame f's own staged words have been read.
+    unsigned tb = 0u;
+    if (live && A.noise_tab) {
+        const uint32_t* d0 = A.desc + (size_t)s * A.n_frames * DESC_WORDS;
+        stage_desc(ws.dstage[0], d0, lane);
+        if (A.n_frames > 1) {
+            stage_desc(ws.dstage[1], d0 + DESC_WORDS, lane);
+        }
+        cp_async_wait_all();
+        __syncwarp();
+        if (noise_prefetch(ws.dstage[0], A.noise_tab, bk, ws.buf[0], lane)) {
+            tb = 4u;
+        }
+    }
+    if (lane == 0) {
+        ws.n_tab[0] = ws.n_tab[1] = 0u;
+    }
 #pragma unroll 1
     for (int f = 0; f < A.n_frames; ++f) {
 #if MBE_U_LOCKSTEP
@@ -596,7 +721,43 @@ __global__ void __launch_bounds__(U_WARPS * 32, U_MINB) mbe_split_unvoiced_kerne
         }
         const size_t idx = (size_t)(A.io_base + s) * A.n_frames + f;
         const uint32_t* d = A.desc + ((size_t)s * A.n_frames + f) * DESC_WORDS;
-        unsigned ops = d[D_OPS];
+        const unsigned ia = tb & 3u;
+        const bool hit = (tb & 4u) != 0u;
+        tb = (ia == 0u) ? 2u : ia - 1u;
+        const uint32_t* dw = d;   // frame f's words 0..7 and, at dw + dov, its overlap
+        int dov = D_OV;
+        if (A.noise_tab) {
+            cp_async_wait_all();
+            __syncwarp();
+            if (f + 1 < A.n_frames && noise_prefetch(ws.dstage[(f + 1) & 1], A.noise_tab, bk, ws.buf[tb], lane)) {
+                tb |= 4u;
+            }
+            dw = ws.dstage[f & 1];
+            dov = 8;
+        }
+        float* Af = ws.buf[ia];
+        float* Bf = ws.buf[ia == 2u ? 0u : ia + 1u];
+        unsigned ops = dw[D_OPS];
+        // the noise spectrum depends on the descriptor alone, not on the previousUw ops: it is ready before they run
+        if (dw[D_INFO] & 1u) {
+            for (int i = lane; i < 129; i += 32) {
+                ws.scale[i] = 0.0f;
+            }
+            if (A.counters && lane == 0) {
+                ++ws.n_tab[hit ? 0 : 1];
+            }
+            if (!hit) {
+                split_noise(Af, __uint_as_float(dw[D_SEED]), dw + dov, bt, lane);
+                __syncwarp();
+                rfft256_forward_inl(Af, Bf, bt->tw, lane);
+            } else {
+                __syncwarp();
+            }
+        }
+        if (A.noise_tab && f + 2 < A.n_frames) {
+            __syncwarp();   // (every lane has read frame f's staged words)
+            stage_desc(ws.dstage[f & 1], d + 2 * DESC_WORDS, lane);
+        }
 #pragma unroll 1
         while (ops) {
             const unsigned op = ops & 15u;
@@ -613,14 +774,8 @@ __global__ void __launch_bounds__(U_WARPS * 32, U_MINB) mbe_split_unvoiced_kerne
                 for (int q = 0; q < 5; ++q) {
                     voiced[q] = __uint_as_float(d[D_VOICED + 32 * q + lane]);
                 }
-                split_noise(ws, d, bt, lane);
-                for (int i = lane; i < 129; i += 32) {
-                    ws.scale[i] = 0.0f;
-                }
-                __syncwarp();
-                rfft256_forward(ws.a, ws.b, bt->tw, lane);
-                split_unvoiced_shape(ws, d, L, __uint_as_float(d[D_CW0]), d[D_CU], d[D_CU + 1], bt, lane);
-                const float* Ab = ws.a;
+                split_unvoiced_shape(ws, Af, Bf, d, L, __uint_as_float(d[D_CW0]), d[D_CU], d[D_CU + 1], bt, lane);
+                const float* Ab = Af;
                 const float inv = 1.0f / (float)NFFT;
 #pragma unroll
                 for (int cc = 0; cc < 5; ++cc) {
@@ -671,6 +826,11 @@ __global__ void __launch_bounds__(U_WARPS * 32, U_MINB) mbe_split_unvoiced_kerne
                 }
             }
         }
+    }
+    cp_async_wait_all();
+    if (A.counters && live && lane == 0) {
+        atomicAdd(&A.counters[4], (unsigned long long)ws.n_tab[0]);
+        atomicAdd(&A.counters[5], (unsigned long long)ws.n_tab[1]);
     }
 }
 

@@ -772,8 +772,8 @@ __device__ __forceinline__ void radb4_last(float c, float a, float d, float b, f
 
 // forward transform: A = X0 on entry, A = X4 on exit (B scratch).  tw = FFTPACK twiddle table:
 // ido=64 rows at 0/64/128, ido=16 rows at 192/208/224, ido=4 rows at 240/244/248.
-__device__ __noinline__ void rfft256_forward(float* __restrict__ A, float* __restrict__ B, const float* __restrict__ tw,
-                                             int lane) {
+__device__ __forceinline__ void rfft256_forward_inl(float* __restrict__ A, float* __restrict__ B, const float* __restrict__ tw,
+                                                    int lane) {
     // ---- ido = 1, l1 = 64: X0 -> X1
 #pragma unroll
     for (int h = 0; h < 2; ++h) {
@@ -850,6 +850,10 @@ __device__ __noinline__ void rfft256_forward(float* __restrict__ A, float* __res
         A[256] = oL3;
     }
     __syncwarp();
+}
+__device__ __noinline__ void rfft256_forward(float* __restrict__ A, float* __restrict__ B, const float* __restrict__ tw,
+                                             int lane) {
+    rfft256_forward_inl(A, B, tw, lane);
 }
 
 // backward transform: A = X4 on entry (unscaled spectrum; every bin is multiplied by scale[bin] as it is
